@@ -6,7 +6,7 @@ kdFindWithinRange queries at the RRTx shrinking-ball radius, neighbour indices A
 distance keys produced), plus edge collision checks/s for the obstacle-add sweep
 (config C3) as an extra object on the same JSON line.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 One process per GPU (torchrun for N > 1): the tree is replicated, every rank owns its
 own batch of queries (weak scaling, no data-path collective; per-query counts are
@@ -200,6 +200,55 @@ def run_reference(args, rank, world):
             "e2e": {"value": value, "unit": "queries/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
             "gpu_launches": 0}
     print(json.dumps(line), flush=True)
+
+
+def tensor_from_ptr(torch_mod, p, n, dtype):
+    # zero-copy view of library-owned device memory through the CUDA array interface
+    class _Holder:
+        pass
+    h = _Holder()
+    typestr = {torch_mod.int32: "<i4", torch_mod.float64: "<f8"}[dtype]
+    h.__cuda_array_interface__ = {"shape": (n,), "typestr": typestr, "data": (int(p), False), "version": 3}
+    return torch_mod.as_tensor(h, device="cuda")
+
+
+DUMP_MAX_BYTES = 64 << 20
+DUMP_COUNT_QUERIES = 1 << 20     # counts of all queries at the default size
+DUMP_LIST_QUERIES = 4096         # ~1.8M neighbours at the default radius
+DUMP_SEED = 77
+
+
+def dump_range_outputs(out_dir, res, n_queries):
+    """--dump-outputs: what the caller of the timed C2 step receives, from the result of the LAST timed step, as
+    float64 .npy files under out_dir (at most DUMP_MAX_BYTES).  Queries are sampled with a fixed splitmix64 seed:
+      query_index.npy        ascending indices of up to DUMP_COUNT_QUERIES queries (all of them at the default size)
+      counts.npy             their neighbour counts
+      list_query_index.npy   ascending indices of up to DUMP_LIST_QUERIES of those queries (fewer if the lists would
+                             exceed the size limit)
+      neighbour_idx.npy      their neighbour lists, concatenated in that order, each list in ascending node index
+      neighbour_dist.npy     the distance key of each of those neighbours
+    A list is a set (include/rrtqx_b200.h): its order on the device and the offsets that place it in memory are not
+    part of the result, so they are not written and two builds compare file for file."""
+    import torch
+    counts, offsets = res.layout()
+    order = np.argsort(W.splitmix64(DUMP_SEED, 0, n_queries), kind="stable")
+    sel = np.sort(order[:min(n_queries, DUMP_COUNT_QUERIES)])
+    take = order[:min(n_queries, DUMP_LIST_QUERIES)]
+    room = DUMP_MAX_BYTES - 16 * len(sel) - 4096          # 4096: the five .npy headers
+    take = np.sort(take[:np.searchsorted(np.cumsum(16 * counts[take].astype(np.int64) + 8), room, side="right")])
+    n = counts[take].astype(np.int64)
+    owner = np.repeat(np.arange(len(take)), n)
+    pos = offsets[take][owner] + (np.arange(int(n.sum())) - np.repeat(np.cumsum(n) - n, n))
+    _, _, idx_p, dist_p = res.device_pointers()
+    total = res.sizes()[1]
+    pos_d = torch.from_numpy(pos).cuda()
+    idx = tensor_from_ptr(torch, idx_p, total, torch.int32)[pos_d].cpu().numpy()
+    dist = tensor_from_ptr(torch, dist_p, total, torch.float64)[pos_d].cpu().numpy()
+    by_node = np.lexsort((idx, owner))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("query_index", sel), ("counts", counts[sel]), ("list_query_index", take),
+                    ("neighbour_idx", idx[by_node]), ("neighbour_dist", dist[by_node])):
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 _C3_CACHE = {}
@@ -485,7 +534,13 @@ def main():
     ap.add_argument("--no-c5", action="store_true")
     ap.add_argument("--c5-instances", type=int, default=64)
     ap.add_argument("--c5-iterations", type=int, default=1000)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed C2 step computed to DIR/<name>.npy (see dump_range_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -538,14 +593,6 @@ def main():
             comm.allgather([res.device_pointers()[0]], [gathered.data_ptr()], args.queries * 4, side_stream=True)
         return total
 
-    def tensor_from_ptr(torch_mod, p, n, dtype):
-        # zero-copy view of library-owned device memory through the CUDA array interface
-        class _Holder:
-            pass
-        h = _Holder()
-        h.__cuda_array_interface__ = {"shape": (n,), "typestr": "<i4", "data": (int(p), False), "version": 3}
-        return torch_mod.as_tensor(h, device="cuda")
-
     sampler = ClockSampler(local_rank)
     sampler.start()
     for _ in range(args.warmup):
@@ -595,6 +642,8 @@ def main():
     else:
         ms, total_all = ms_local, total
     value = world * args.queries / (ms / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_range_outputs(args.dump_outputs, res, args.queries)
 
     # roofline of the step: compulsory bytes (SURVEY 8d): N*24 + Q*24 + (Q+1)*8 + K*(4+8)
     K = total

@@ -10,6 +10,7 @@ and, with -m gpu, through the same three routes of the CUDA library.  Twelve val
 Julia script of tests/test_reference_vectors.py does that), but they are the reference's own output, not ours."""
 import ctypes as C
 import json
+import math
 import os
 
 import numpy as np
@@ -29,16 +30,18 @@ def _load():
 
 
 def test_fixture_is_the_reference_output():
+    """The stored rows are bit patterns copied from the reference's files (make_reference_outputs.py).  What ties them
+    to the stored obstacles is what identified the obstacle file: findClosestObs in plain IEEE double arithmetic (first
+    minimum wins) reproduces every recorded distance and argmin from the stored spheres, bit for bit."""
     S, rows, arg = _load()
     assert S.shape == (15, 4) and rows.shape == (12, 4)
-    ref = "/root/reference/code_RRTQx_3D/BVPData"
-    if os.path.isdir(ref):   # in the authoring container: the fixture equals the reference's files
-        got = []
-        for k in range(1, 5):
-            for line in open(os.path.join(ref, f"BVPDistFromStaticObs_{k}.txt")):
-                if line.strip():
-                    got.append([float(t) for t in line.split(",")])
-        assert np.array_equal(np.array(got).view(np.uint64), rows.view(np.uint64))
+    for (x, y, z, want), a in zip(rows, arg):
+        best, rad, j_best = -1.0, 0.0, -1
+        for j, (cx, cy, cz, r) in enumerate(S.tolist()):
+            d = math.sqrt((x - cx) ** 2 + (y - cy) ** 2 + (z - cz) ** 2)
+            if d < best or best == -1.0:
+                best, rad, j_best = d, r, j
+        assert j_best == a and (best - rad).hex() == float(want).hex()
 
 
 def test_oracle_reproduces_the_reference_distances_bit_for_bit():
