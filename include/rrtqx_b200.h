@@ -286,7 +286,10 @@ RRTQX_API rrtqx_status rrtqx_node_check_batch(rrtqx_ctx *ctx,
  * full count (if it exceeds capacity only the first `capacity` are written).
  * At most 768 ACTIVE obstacles (inactive entries of an ever-growing list are
  * compacted away, once per obstacle-set change); d == 3 for the edge checks
- * (other d: flags are 0).
+ * (other d: flags are 0).  Trees with wrap-around dimensions are refused with
+ * RRTQX_ERR_UNSUPPORTED: the launch searches the real point only, without the
+ * ghost identities of kdFindNearest / kdFindWithinRange; use
+ * rrtqx_nearest_batch and rrtqx_range_query_batch there.
  * Results arrive through mapped pinned memory: one launch, one synchronise. */
 RRTQX_API rrtqx_status rrtqx_extend_query(
     rrtqx_tree *tree, const rrtqx_spheres *spheres, const double *point,
@@ -312,7 +315,8 @@ RRTQX_API rrtqx_status rrtqx_edges_upload(rrtqx_edges *e, const int32_t *src,
  * (makeNeighborOf / makeInitialOutNeighborOf, DRRT_Q.jl:2589-2593); endpoints may be nodes inserted into the
  * tree since the upload.  rrtqx_edges_set_parents re-points parent edges (makeParentOf, DRRT_Q.jl:1841-1856):
  * parent_ids[i] becomes the parent of node_ids[i], -1 = rrtParentUsed false; nodes never mentioned have no
- * parent edge.  Neither call re-uploads the graph; the device CSR is rebuilt before the next sweep.  Edges
+ * parent edge (which of these calls need new Dubins trajectories: rrtqx_edges_solve_trajectories).
+ * Neither call re-uploads the graph; the device CSR is rebuilt before the next sweep.  Edges
  * are never deleted: results for edges the planner has culled are ignored by the caller. */
 RRTQX_API rrtqx_status rrtqx_edges_append(rrtqx_edges *e, const int32_t *src,
                                           const int32_t *dst, int64_t n_new);
@@ -445,7 +449,12 @@ RRTQX_API rrtqx_status rrtqx_edges_set_trajectories(rrtqx_edges *e,
 /* ... or have the device solve every item with calculateTrajectory
  * (DRRT_DubinsEdge_functions.jl:329-709; d == 4): start / end poses are the
  * resident node positions.  *n_rows_out = total trajectory rows.  Both calls
- * must be repeated after the edge set, the parents or the tree size change. */
+ * must be repeated after the edge set or the tree size change, and after a
+ * rrtqx_edges_set_parents call that gives some node a parent (>= 0) other than
+ * its current one, the first parents of an edge set uploaded without them
+ * included; until then the sweeps fail with RRTQX_ERR_STATE.  Setting parents
+ * to -1 keeps the trajectories valid: the item of a node without a parent edge
+ * is never read. */
 RRTQX_API rrtqx_status rrtqx_edges_solve_trajectories(rrtqx_edges *e,
                                                       double min_turn_radius,
                                                       int64_t *n_rows_out);

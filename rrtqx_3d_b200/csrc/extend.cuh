@@ -286,6 +286,10 @@ void extend_query(rrtqx_tree *t, const rrtqx_spheres *S, const double *point, do
   cudaStream_t st = ctx->stream;
   RQ_REQUIRE(point != nullptr && !is_device_ptr(point), "point must be a host array");
   RQ_REQUIRE(capacity >= 0, "capacity is negative");
+  // the kernel searches the real query point only: on a wrap-around tree its nearest node and neighbour list would
+  // miss the ghost identities that kdFindNearest / kdFindWithinRange visit (ghostPoint.jl:60-111)
+  if (t->wrap.num_wraps > 0)
+    throw Error(RRTQX_ERR_UNSUPPORTED, "extend query on a wrap-around tree (use the batched nearest / range calls)");
   if (t->n == 0) throw Error(RRTQX_ERR_EMPTY_TREE, "extend query on an empty tree");
   tree_prepare_query(t);
   ExtendState *es = &extend_state(t);

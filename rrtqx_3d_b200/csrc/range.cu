@@ -295,7 +295,9 @@ range_query_kernel(GridView g, WrapInfo wrap, const double *__restrict__ queries
         }
         emit(hit, j, s);
       }
-      if (WRAP) {
+      // qprev holds 2^MAX_WRAPS - 1 identities: the last one is never needed (nothing is searched after it), and
+      // storing it would write past the array with MAX_WRAPS wrap dimensions
+      if (WRAP && ident + 1 < n_ident) {
 #pragma unroll
         for (int k = 0; k < D; ++k) qprev[n_prev][k] = q[k];
         n_prev++;
@@ -516,6 +518,13 @@ nearest_kernel(GridView g, WrapInfo wrap, const double *__restrict__ queries, co
         best_dist = dd;
         best_node = bn;
       }
+    }
+    if (best_node < 0) {
+      // no radicand compared below +inf (NaN or infinite query coordinates): the reference keeps its first
+      // candidate, the root, with its distance (kdTree_general.jl:359-361)
+      const double4 p0 = g.pos[0];
+      best_node = 0;
+      best_dist = __dsqrt_rn(sqdist<D>(q0, p0.x, p0.y, p0.z, p0.w));
     }
     if (lane == 0) {
       out_idx[qid] = best_node;

@@ -182,12 +182,14 @@ void edges_append(rrtqx_edges *E, const int32_t *src, const int32_t *dst, int64_
   RQ_CUDA(cudaStreamSynchronize(st));  // the caller's arrays may be reused on return
 }
 
+// flags[0]: entries out of range; flags[1]: some node got a parent edge (p >= 0) other than the one it had
 __global__ void parent_scatter_kernel(const int32_t *__restrict__ nodes, const int32_t *__restrict__ parents, int64_t n,
-                                      int64_t n_nodes, int32_t *__restrict__ parent, int32_t *__restrict__ bad) {
+                                      int64_t n_nodes, int32_t *__restrict__ parent, int32_t *__restrict__ flags) {
   int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   const int v = nodes[i], p = parents[i];
-  if (v < 0 || v >= n_nodes || p < -1 || p >= n_nodes) { atomicAdd(bad, 1); return; }
+  if (v < 0 || v >= n_nodes || p < -1 || p >= n_nodes) { atomicAdd(&flags[0], 1); return; }
+  if (p >= 0 && parent[v] != p) flags[1] = 1;
   parent[v] = p;  // -1: rrtParentUsed = false
 }
 
@@ -211,14 +213,17 @@ void edges_set_parents(rrtqx_edges *E, const int32_t *nodes, const int32_t *pare
   const int32_t *dn = to_device(ctx, nodes, (size_t)n, ctx->stage_i32a);
   const int32_t *dp = to_device(ctx, parents, (size_t)n, ctx->stage_i32b);
   t->flagbuf.ensure(8, st);
-  RQ_CUDA(cudaMemsetAsync(t->flagbuf.p, 0, sizeof(int32_t), st));
+  RQ_CUDA(cudaMemsetAsync(t->flagbuf.p, 0, 2 * sizeof(int32_t), st));
   parent_scatter_kernel<<<div_up(n, 256), 256, 0, st>>>(dn, dp, n, nn, E->parent.p, t->flagbuf.p);
   post_launch(ctx);
-  int32_t bad = 0;
-  RQ_CUDA(cudaMemcpyAsync(&bad, t->flagbuf.p, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  int32_t flags[2] = {0, 0};
+  RQ_CUDA(cudaMemcpyAsync(flags, t->flagbuf.p, sizeof(flags), cudaMemcpyDeviceToHost, st));
   RQ_CUDA(cudaStreamSynchronize(st));
   E->dirty = true;
-  RQ_REQUIRE(bad == 0, "node / parent index out of range");
+  // a parent edge now runs to another node: its resident trajectory (item n_edges + v) is the old edge's.  Clearing
+  // parents keeps them valid, since the sweeps never read the item of a node without a parent edge.
+  if (flags[1]) E->traj_items = -1;
+  RQ_REQUIRE(flags[0] == 0, "node / parent index out of range");
 }
 
 // ------------------------------------------------------ sweep obstacle table

@@ -265,8 +265,9 @@ static void sweep2d_prepare(rrtqx_edges *E, const rrtqx_polygons *Pg, const int3
   RQ_REQUIRE(t->d == 2 || t->d == 4, "the Otte / Dubins sweeps need a 2-D ([x y]) or a Dubins ([x y t theta]) tree");
   RQ_REQUIRE(t->wrap.num_wraps <= 1, "at most one wrap-around dimension (the Dubins heading)");
   const int64_t items = sweep2d_items(E);
-  RQ_REQUIRE(E->traj_items == items, "trajectories are not resident for the current edge set "
-                                     "(rrtqx_edges_set_trajectories / rrtqx_edges_solve_trajectories after the last change)");
+  if (E->traj_items != items)
+    throw Error(RRTQX_ERR_STATE, "trajectories are not resident for the current edge set "
+                                 "(rrtqx_edges_set_trajectories / rrtqx_edges_solve_trajectories after the last change)");
   for (int64_t i = 0; i < n_ids; ++i) RQ_REQUIRE(ids_host[i] >= 0 && ids_host[i] < Pg->n, "obstacle id out of range");
   R->ids_stage2.ensure((size_t)n_ids + 1, st);
   R->filt2d.ensure((size_t)n_ids * sizeof(Sweep2dFilter) + 16, st);
