@@ -290,6 +290,10 @@ RRTQX_API rrtqx_status rrtqx_node_check_batch(rrtqx_ctx *ctx,
  * RRTQX_ERR_UNSUPPORTED: the launch searches the real point only, without the
  * ghost identities of kdFindNearest / kdFindWithinRange; use
  * rrtqx_nearest_batch and rrtqx_range_query_batch there.
+ * Non-finite input, as in kdFindNearest, which starts from the root: a sample
+ * whose every radicand is NaN or +inf (a NaN coordinate, 1e200) and any sample
+ * whose radicand to the root is NaN get nearest_idx = 0 with the root's
+ * distance (never -1).  Nearest ties go to the smallest node index.
  * Results arrive through mapped pinned memory: one launch, one synchronise. */
 RRTQX_API rrtqx_status rrtqx_extend_query(
     rrtqx_tree *tree, const rrtqx_spheres *spheres, const double *point,

@@ -183,10 +183,13 @@ extend_query_kernel(GridView g, const ExtendParams prm, const double4 *__restric
     hit = __any_sync(FULL, hit);
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) cert = fmin(cert, __shfl_xor_sync(FULL, cert, o));
+    // kdFindNearest keeps its first candidate, the root, when no radicand compares below +inf (NaN or huge sample
+    // coordinates) and when the root's radicand is NaN (nothing compares below it): kdTree_general.jl:359-379
+    if (bn == 0x7fffffff || s0 != s0) { bn = 0; bs = s0; }
     if (lane == 0) {
       ExtendHeader h;
       h.count = count;
-      h.nearest_idx = bn == 0x7fffffff ? -1 : bn;
+      h.nearest_idx = bn;
       h.nearest_dist = __dsqrt_rn(bs);
       h.point_collides = hit ? 1 : 0;
       h.overflow = count > prm.capacity ? 1 : 0;

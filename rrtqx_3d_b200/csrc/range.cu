@@ -491,18 +491,21 @@ nearest_kernel(GridView g, WrapInfo wrap, const double *__restrict__ queries, co
           // lower bound on the distance of any point outside the scanned cube
           // (faces at the grid boundary do not count: nothing lies beyond).
           double bound = INFINITY;
+          bool unseen = false;  // cells left outside the cube (their bound may be +inf for an infinite query)
           {
             double f;
-            if (cx - rho > 0)          { f = q[0] - (g.lo[0] + (cx - rho) * g.cell[0]); bound = fmin(bound, f); }
-            if (cx + rho < g.nx - 1)   { f = (g.lo[0] + (cx + rho + 1) * g.cell[0]) - q[0]; bound = fmin(bound, f); }
-            if (cy - rho > 0)          { f = q[1] - (g.lo[1] + (cy - rho) * g.cell[1]); bound = fmin(bound, f); }
-            if (cy + rho < g.ny - 1)   { f = (g.lo[1] + (cy + rho + 1) * g.cell[1]) - q[1]; bound = fmin(bound, f); }
+            if (cx - rho > 0)          { f = q[0] - (g.lo[0] + (cx - rho) * g.cell[0]); bound = fmin(bound, f); unseen = true; }
+            if (cx + rho < g.nx - 1)   { f = (g.lo[0] + (cx + rho + 1) * g.cell[0]) - q[0]; bound = fmin(bound, f); unseen = true; }
+            if (cy - rho > 0)          { f = q[1] - (g.lo[1] + (cy - rho) * g.cell[1]); bound = fmin(bound, f); unseen = true; }
+            if (cy + rho < g.ny - 1)   { f = (g.lo[1] + (cy + rho + 1) * g.cell[1]) - q[1]; bound = fmin(bound, f); unseen = true; }
             if (D >= 3) {
-              if (cz - rho > 0)        { f = q[2] - (g.lo[2] + (cz - rho) * g.cell[2]); bound = fmin(bound, f); }
-              if (cz + rho < g.nz - 1) { f = (g.lo[2] + (cz + rho + 1) * g.cell[2]) - q[2]; bound = fmin(bound, f); }
+              if (cz - rho > 0)        { f = q[2] - (g.lo[2] + (cz - rho) * g.cell[2]); bound = fmin(bound, f); unseen = true; }
+              if (cz + rho < g.nz - 1) { f = (g.lo[2] + (cz + rho + 1) * g.cell[2]) - q[2]; bound = fmin(bound, f); unseen = true; }
             }
           }
-          if (isinf(bound) && bound > 0) break;  // whole grid scanned
+          // whole grid scanned.  An infinite bound alone does not end the search: a query with an infinite
+          // coordinate has radicand +inf to every node, and the tie rule needs the smallest index among them all
+          if (!unseen) break;
           // conservative: shrink the bound by the cell-geometry slack
           double slack = 1e-9 * fmax(g.cell[0], fmax(g.cell[1], g.cell[2])) +
                          1e-12 * (fabs(q[0]) + fabs(q[1]) + (D >= 3 ? fabs(q[2]) : 0.0));
@@ -519,12 +522,16 @@ nearest_kernel(GridView g, WrapInfo wrap, const double *__restrict__ queries, co
         best_node = bn;
       }
     }
-    if (best_node < 0) {
-      // no radicand compared below +inf (NaN or infinite query coordinates): the reference keeps its first
-      // candidate, the root, with its distance (kdTree_general.jl:359-361)
+    {
+      // the reference seeds its best distance with the root's (kdTree_general.jl:359-361) and replaces it only by
+      // a strictly smaller one: it keeps the root when no radicand compared below +inf (NaN or infinite query
+      // coordinates) and when the root's radicand is NaN (then nothing compares below it, ghosts included)
       const double4 p0 = g.pos[0];
-      best_node = 0;
-      best_dist = __dsqrt_rn(sqdist<D>(q0, p0.x, p0.y, p0.z, p0.w));
+      const double s0 = sqdist<D>(q0, p0.x, p0.y, p0.z, p0.w);
+      if (best_node < 0 || s0 != s0) {
+        best_node = 0;
+        best_dist = __dsqrt_rn(s0);
+      }
     }
     if (lane == 0) {
       out_idx[qid] = best_node;
@@ -540,7 +547,8 @@ nearest_kernel(GridView g, WrapInfo wrap, const double *__restrict__ queries, co
 // the best radicand; the box of cells within that distance is then scanned, each cell skipped when a
 // conservative lower bound of its distance exceeds the best radicand.  Queries whose box is wider than
 // 2*NN_RHO_MAX+1 cells (far outside the grid, empty regions) are handed to the warp-per-query kernel.
-// Result semantics identical to nearest_kernel: minimum radicand, ties to the smallest node index.
+// Result semantics identical to nearest_kernel: minimum radicand, ties to the smallest node index; a NaN radicand
+// to the root answers (root, NaN).
 constexpr int NN_RHO_MAX = 3;
 
 template <int D>
@@ -554,6 +562,16 @@ nearest_tpq_kernel(GridView g, const double *__restrict__ queries, const int32_t
   double q[D];
 #pragma unroll
   for (int k = 0; k < D; ++k) q[k] = queries[(int64_t)qid * D + k];
+  {
+    // NaN radicand to the root: the reference's best distance starts as NaN and nothing compares below it
+    const double4 p0 = g.pos[0];
+    const double s0 = sqdist<D>(q, p0.x, p0.y, p0.z, p0.w);
+    if (s0 != s0) {
+      out_idx[qid] = 0;
+      if (out_dist) out_dist[qid] = s0;
+      return;
+    }
+  }
   double bs = INFINITY;
   int bn = 0x7fffffff;
   const int cx = cell_of(q[0], g.lo[0], g.inv[0], g.nx);
@@ -561,13 +579,17 @@ nearest_tpq_kernel(GridView g, const double *__restrict__ queries, const int32_t
   const int cz = D >= 3 ? cell_of(q[2], g.lo[2], g.inv[2], g.nz) : 0;
   const double slack = 1e-9 * fmax(g.cell[0], fmax(g.cell[1], g.cell[2])) +
                        1e-12 * (fabs(q[0]) + fabs(q[1]) + (D >= 3 ? fabs(q[2]) : 0.0));
-  // conservative lower bound of |p_c - q_c| for a point stored in cell k of axis c
-  auto gap = [&](int c, int k) {
+  // conservative lower bound of |p_c - q_c| for a point stored in cell k of axis c (n cells).  Boundary cells are
+  // open on their outer side: cell_of clamps into them whatever lies beyond the grid, and an axis whose bbox is not
+  // finite (a +-inf node, an overflowing extent) is one cell [lo, lo + 1] that holds every point
+  auto gap = [&](int c, int k, int n) {
     const double lo_k = g.lo[c] + k * g.cell[c], hi_k = lo_k + g.cell[c];
-    return fmax(0.0, fmax(lo_k - q[c], q[c] - hi_k) - slack);
+    const double a = (k == 0) ? -INFINITY : lo_k - q[c];
+    const double b = (k == n - 1) ? -INFINITY : q[c] - hi_k;
+    return fmax(0.0, fmax(a, b) - slack);
   };
   auto scan_cell = [&](int x, int y, int z) {
-    const double gx = gap(0, x), gy = gap(1, y), gz = D >= 3 ? gap(2, z) : 0.0;
+    const double gx = gap(0, x, g.nx), gy = gap(1, y, g.ny), gz = D >= 3 ? gap(2, z, g.nz) : 0.0;
     if ((gx * gx + gy * gy + gz * gz) * (1.0 - 1e-9) > bs) return;  // cannot beat (or tie) the best
     const int c = (z * g.ny + y) * g.nx + x;
     const int a = g.cell_start[c], b = g.cell_start[c + 1];
