@@ -62,6 +62,7 @@ typedef struct rrtqx_polygons rrtqx_polygons;
 typedef struct rrtqx_edges rrtqx_edges;
 typedef struct rrtqx_range_result rrtqx_range_result;
 typedef struct rrtqx_sweep_result rrtqx_sweep_result;
+typedef struct rrtqx_dubins_result rrtqx_dubins_result;
 
 /* ---------------------------------------------------------------- context */
 
@@ -289,7 +290,8 @@ RRTQX_API rrtqx_status rrtqx_node_check_batch(rrtqx_ctx *ctx,
  * (other d: flags are 0).  Trees with wrap-around dimensions are refused with
  * RRTQX_ERR_UNSUPPORTED: the launch searches the real point only, without the
  * ghost identities of kdFindNearest / kdFindWithinRange; use
- * rrtqx_nearest_batch and rrtqx_range_query_batch there.
+ * rrtqx_nearest_batch and rrtqx_range_query_batch there, or, on the
+ * DubinsEdge tree [x y t theta], rrtqx_extend_query_dubins below.
  * Non-finite input, as in kdFindNearest, which starts from the root: a sample
  * whose every radicand is NaN or +inf (a NaN coordinate, 1e200) and any sample
  * whose radicand to the root is NaN get nearest_idx = 0 with the root's
@@ -301,6 +303,40 @@ RRTQX_API rrtqx_status rrtqx_extend_query(
     int32_t *nearest_idx, double *nearest_dist, uint8_t *point_collides,
     double *point_cert, int32_t *n_neighbors, int32_t *nbr_idx,
     double *nbr_dist, uint8_t *fwd_collide, uint8_t *rev_collide);
+
+/* The DubinsEdge counterpart (config C4: a 4-D tree [x y t theta] whose
+ * dimension 3 wraps with period 2 pi = 6.283185307179586; every other layout
+ * fails with RRTQX_ERR_UNSUPPORTED) for the new sample `point` (4 doubles,
+ * host), in the reference's order:
+ *   kdFindNearest(KD, point), ghost identity included -> nearest_idx /
+ *       nearest_dist (ties and non-finite input as rrtqx_nearest_batch)
+ *   with RRTQX_EXTEND_SATURATE: saturate(point, nearest, delta)
+ *       (DRRT_DubinsEdge_functions.jl:70-95), written back into `point`;
+ *       without it the point is used as given (delta unused)
+ *   kdFindWithinRange(KD, range, point), ghost identity included
+ *       -> *n_neighbors, nbr_idx[], nbr_dist[] (as rrtqx_range_query_batch)
+ *   for neighbour i: edge 2i = new -> nbr (findBestParent, DRRT_Q.jl:1949-1960)
+ *   and edge 2i+1 = nbr -> new (:2600-2603): calculateTrajectory -> edge_dist[]
+ *   and edge_type[] (codes of rrtqx_dubins_trajectory_batch), Dubins
+ *   explicitEdgeCheck OR-ed over the polygon set -> edge_collide[]
+ *   (as rrtqx_dubins_edge_check_batch; RRTQX_CHECK_IGNORE_ACTIVE honoured).
+ * `capacity` = length of nbr_idx / nbr_dist; the edge arrays hold 2*capacity.
+ * *n_neighbors is the full count; only the first `capacity` neighbours and
+ * their edges are produced.  Any output pointer may be NULL.  With
+ * trajectories != NULL the rows of the 2*min(count, capacity) edges are left,
+ * in edge order, in that rrtqx_dubins_result (created when *trajectories is
+ * NULL); read them with rrtqx_dubins_result_sizes / _fetch / _device.
+ * The polygon-world node check is not part of this call.
+ * Three launches and one host wait on mapped pinned memory; a call whose rows
+ * outgrow the grow-only scratch grows it and runs once more. */
+enum { RRTQX_EXTEND_SATURATE = 8u }; /* same flags word as the RRTQX_CHECK_* */
+RRTQX_API rrtqx_status rrtqx_extend_query_dubins(
+    rrtqx_tree *tree, const rrtqx_polygons *polygons, double *point,
+    double delta, double range, double robot_radius, double min_turn_radius,
+    uint32_t flags, int32_t capacity, int32_t *nearest_idx,
+    double *nearest_dist, int32_t *n_neighbors, int32_t *nbr_idx,
+    double *nbr_dist, double *edge_dist, int32_t *edge_type,
+    uint8_t *edge_collide, rrtqx_dubins_result **trajectories);
 
 /* ------------------------------------------------- resident edge set + sweeps */
 /* Device mirror of the planner's out-edge lists: for node v the reference
@@ -508,7 +544,6 @@ RRTQX_API rrtqx_status rrtqx_obstacle_remove_sweep_2d(
  * earlier call (its buffers are reused).  Parity with the reference is by
  * tolerance (1e-9 relative; Julia libm and twice-precision ranges, SURVEY.md
  * appendix A14). */
-typedef struct rrtqx_dubins_result rrtqx_dubins_result;
 RRTQX_API rrtqx_status rrtqx_dubins_trajectory_batch(
     rrtqx_ctx *ctx, const double *starts, const double *goals, int64_t n_edges,
     double min_turn_radius, rrtqx_dubins_result **result);

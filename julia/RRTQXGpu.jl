@@ -53,6 +53,7 @@ const RANGE_COUNT_ONLY = UInt32(2)
 const CHECK_FMA_DOT       = UInt32(1)
 const CHECK_IGNORE_ACTIVE = UInt32(2)
 const CHECK_QUICK_PASS    = UInt32(4)
+const EXTEND_SATURATE     = UInt32(8)
 const SWEEP_REMOVED_INACTIVE = UInt32(16)
 
 # ------------------------------------------------------------------ context
@@ -694,10 +695,74 @@ function calculateTrajectoryBatch(ctx::Context, S, edges::Vector)
       (Ptr{Cvoid}, Ptr{Float64}, Ptr{Int32}, Ptr{Int64}, Ptr{Float64}), res[], dist, typ, ptr, xy))
   ccall((:rrtqx_dubins_result_destroy, LIB), Int32, (Ptr{Cvoid},), res[])
   for (i, e) in enumerate(edges)
-    e.dubinsType = typ[i] < 0 ? "xxx" : DUBINS_TYPES[typ[i] + 1]
-    e.Wdist = dist[i]; e.dist = dist[i]; e.distOriginal = dist[i]
-    e.trajectory = permutedims(xy[:, ptr[i]+1:ptr[i+1]])          # rows x 2, as the reference builds it
+    setDubinsTrajectory!(e, dist[i], typ[i], xy, ptr[i], ptr[i+1])
   end
+end
+
+# What calculateTrajectory sets on a DubinsEdge, from a device solve: dist = distOriginal = Wdist, dubinsType and
+# trajectory = rows first+1:last of xy (2 x rows, 0-based CSR bounds), as the reference builds it (rows x 2)
+function setDubinsTrajectory!(e, dist::Float64, typ::Integer, xy::AbstractMatrix{Float64}, first::Integer, last::Integer)
+  e.dubinsType = typ < 0 ? "xxx" : DUBINS_TYPES[typ + 1]
+  e.Wdist = dist; e.dist = dist; e.distOriginal = dist
+  e.trajectory = permutedims(xy[:, first+1:last])
+end
+
+# The DubinsEdge iteration in one call (rrtqx_extend_query_dubins): kdFindNearest, saturate(point, nearest, S.delta)
+# when `saturate` (DRRT_DubinsEdge_functions.jl:70-95), kdFindWithinRange(range) with the theta ghost, and for every
+# neighbour calculateTrajectory + explicitEdgeCheck of edge(new -> n) (findBestParent, DRRT_Q.jl:1949-1960) and
+# edge(n -> new) (:2600-2603).  Returns (nearest node, its distance, the (saturated) point, neighbour ids (0-based)
+# and keys, per-edge dist / type codes / collision flags with edge 2i-1 = new -> n_i and 2i = n_i -> new).  Arrays
+# are pinned and reused; the views are valid until the next call on the same CSpace.  The rows stay on the device
+# until dubinsEdgesFromQuery! puts them onto edge objects.  Collision flags are false during warm-up.
+function extendQueryDubins(S, tree::GpuKDTree, point::Array{Float64}, range::Float64; saturate::Bool = false,
+                           capacity::Int = 8192)
+  W = world(S)
+  G = syncPolygons!(W.polygons, S)
+  if !haskey(W.pinned, :didx) || length(W.pinned[:didx]) < capacity
+    W.pinned[:didx] = pinnedVector(W.ctx, Int32, capacity); W.pinned[:ddist] = pinnedVector(W.ctx, Float64, capacity)
+    W.pinned[:dedist] = pinnedVector(W.ctx, Float64, 2 * capacity)
+    W.pinned[:detype] = pinnedVector(W.ctx, Int32, 2 * capacity)
+    W.pinned[:decol] = pinnedVector(W.ctx, UInt8, 2 * capacity)
+  end
+  if !haskey(W.pinned, :dres)
+    r = Ref{Ptr{Cvoid}}(C_NULL)
+    W.pinned[:dres] = r
+    finalizer(x -> x[] != C_NULL && ccall((:rrtqx_dubins_result_destroy, LIB), Int32, (Ptr{Cvoid},), x[]), r)
+  end
+  idx = W.pinned[:didx]::Vector{Int32}; dist = W.pinned[:ddist]::Vector{Float64}
+  edist = W.pinned[:dedist]::Vector{Float64}; etype = W.pinned[:detype]::Vector{Int32}
+  ecol = W.pinned[:decol]::Vector{UInt8}; res = W.pinned[:dres]::Base.RefValue{Ptr{Cvoid}}
+  nearestIdx = Ref{Int32}(0); nearestDist = Ref{Float64}(0.0); n = Ref{Int32}(0)
+  p = Vector{Float64}(vec(point)[1:4])
+  flags = saturate ? EXTEND_SATURATE : UInt32(0)
+  GC.@preserve p idx dist edist etype ecol check(tree.ctx, ccall((:rrtqx_extend_query_dubins, LIB), Int32,
+      (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Float64}, Float64, Float64, Float64, Float64, UInt32, Int32, Ref{Int32},
+       Ref{Float64}, Ref{Int32}, Ptr{Int32}, Ptr{Float64}, Ptr{Float64}, Ptr{Int32}, Ptr{UInt8}, Ref{Ptr{Cvoid}}),
+      tree.h, G.h, p, S.delta, range, S.robotRadius, S.minTurningRadius, flags, Int32(length(idx)), nearestIdx,
+      nearestDist, n, idx, dist, edist, etype, ecol, res))
+  n[] <= length(idx) || return extendQueryDubins(S, tree, point, range; saturate = saturate, capacity = 2 * Int(n[]))
+  k = min(Int(n[]), length(idx))            # never slice past the buffers
+  warm = S.inWarmupTime                     # obstacles are ignored during warm-up (DRRT.jl:1660-1678)
+  return (tree.nodes[nearestIdx[] + 1], nearestDist[], p, view(idx, 1:k), view(dist, 1:k), view(edist, 1:2k),
+          view(etype, 1:2k), warm ? falses(2k) : view(ecol, 1:2k) .!= 0)
+end
+
+# Puts the device solve of the last extendQueryDubins on S onto DubinsEdge objects: edges[e] receives edge e of
+# that call (edges[2i-1] = new -> n_i, edges[2i] = n_i -> new; `nothing` entries are skipped).
+function dubinsEdgesFromQuery!(S, edges::Vector)
+  W = world(S)
+  res = W.pinned[:dres]::Base.RefValue{Ptr{Cvoid}}
+  ne = Ref{Int64}(0); nr = Ref{Int64}(0)
+  check(W.ctx, ccall((:rrtqx_dubins_result_sizes, LIB), Int32, (Ptr{Cvoid}, Ref{Int64}, Ref{Int64}), res[], ne, nr))
+  length(edges) <= ne[] || error("the last extendQueryDubins produced $(ne[]) edges, not $(length(edges))")
+  dist = Vector{Float64}(undef, ne[]); typ = Vector{Int32}(undef, ne[]); ptr = Vector{Int64}(undef, ne[] + 1)
+  xy = Matrix{Float64}(undef, 2, nr[])
+  GC.@preserve dist typ ptr xy check(W.ctx, ccall((:rrtqx_dubins_result_fetch, LIB), Int32,
+      (Ptr{Cvoid}, Ptr{Float64}, Ptr{Int32}, Ptr{Int64}, Ptr{Float64}), res[], dist, typ, ptr, xy))
+  for (i, e) in enumerate(edges)
+    e === nothing || setDubinsTrajectory!(e, dist[i], typ[i], xy, ptr[i], ptr[i+1])
+  end
+  return edges
 end
 
 # Dubins explicitEdgeCheck OR-ed over the obstacle list of G for a batch (DRRT_DubinsEdge_functions.jl:750-774);

@@ -22,6 +22,7 @@ RANGE_WANT_DIST, RANGE_COUNT_ONLY = 1, 2
 CHECK_FMA_DOT, CHECK_IGNORE_ACTIVE, CHECK_QUICK_PASS = 1, 2, 4
 SWEEP_REMOVED_INACTIVE = 16
 SWEEP_STATS = 32
+EXTEND_SATURATE = 8
 
 vp = C.c_void_p
 i32, i64, u32, f64 = C.c_int32, C.c_int64, C.c_uint32, C.c_double
@@ -58,6 +59,8 @@ SIGNATURES = {
     "rrtqx_nearest_batch": (i32, [vp, vp, i64, vp, vp]),
     "rrtqx_extend_query": (i32, [vp, vp, vp, f64, f64, u32, i32, C.POINTER(i32), C.POINTER(f64), C.POINTER(C.c_uint8),
                                  C.POINTER(f64), C.POINTER(i32), vp, vp, vp, vp]),
+    "rrtqx_extend_query_dubins": (i32, [vp, vp, vp, f64, f64, f64, f64, u32, i32, C.POINTER(i32), C.POINTER(f64),
+                                        C.POINTER(i32), vp, vp, vp, vp, vp, C.POINTER(vp)]),
     "rrtqx_spheres_create": (i32, [vp, C.POINTER(vp)]),
     "rrtqx_spheres_destroy": (i32, [vp]),
     "rrtqx_spheres_upload": (i32, [vp, vp, vp, vp, i64]),

@@ -478,6 +478,22 @@ rrtqx_status rrtqx_extend_query(rrtqx_tree *tree, const rrtqx_spheres *spheres, 
   });
 }
 
+rrtqx_status rrtqx_extend_query_dubins(rrtqx_tree *tree, const rrtqx_polygons *polygons, double *point, double delta,
+                                       double range, double robot_radius, double min_turn_radius, uint32_t flags,
+                                       int32_t capacity, int32_t *nearest_idx, double *nearest_dist,
+                                       int32_t *n_neighbors, int32_t *nbr_idx, double *nbr_dist, double *edge_dist,
+                                       int32_t *edge_type, uint8_t *edge_collide,
+                                       rrtqx_dubins_result **trajectories) {
+  if (!tree || !polygons) return RRTQX_ERR_INVALID;
+  rrtqx_ctx *ctx = tree->ctx;
+  return guarded(ctx, [&] {
+    bind_device(ctx);
+    extend_query_dubins(tree, polygons, point, delta, range, robot_radius, min_turn_radius, flags, capacity,
+                        nearest_idx, nearest_dist, n_neighbors, nbr_idx, nbr_dist, edge_dist, edge_type, edge_collide,
+                        trajectories);
+  });
+}
+
 // ---------------------------------------------------------------- spheres
 rrtqx_status rrtqx_spheres_create(rrtqx_ctx *ctx, rrtqx_spheres **out) {
   if (!ctx) return RRTQX_ERR_INVALID;

@@ -1,177 +1,20 @@
 // dubins.cu -- batched Dubins calculateTrajectory on the device
-// (DRRT_DubinsEdge_functions.jl:329-709, space without time; rightTurnDist / leftTurnDist
-// DRRT_distance_functions.jl:62-80) and the DubinsEdge steering point (saturate, :70-95).
+// (DRRT_DubinsEdge_functions.jl:329-709, space without time) and the DubinsEdge steering point
+// (saturate, :70-95); the solver, the discretisation and saturate live in dubins.cuh.
 //
-// One thread solves one edge: the four turning circles, the six words tried in the reference's
-// order (rsl, rsr, rlr, lsr, lsl, lrl) with its strict `bestDist > length` replacement, then the
-// discretisation of the winning word: arcs sampled every 0.1 rad from the start angle
-// (collect(phi_start:+-0.1:phi_end)), a straight part as its two end points.  The solver runs twice
-// per batch: a sizing pass (distance, word, number of trajectory rows), an exclusive scan of the row
-// counts on the device, and an emission pass that writes edge.trajectory[:,1:2] rows into a CSR.
-//
-// Parity: the reference evaluates sin/cos/atan/acos with Julia's libm ports and builds the angle
-// ranges in twice-precision arithmetic; this file uses the CUDA double-precision library and
-// phi_start + i*0.1.  Results agree to a few ulp, so trajectories and lengths are compared at 1e-9
-// relative (SURVEY.md appendix A14); the collision booleans computed FROM a trajectory are bit-exact.
-// Library built with -fmad=false: no contraction changes the operation order below.
+// One thread solves one edge.  The solver runs twice per batch: a sizing pass (distance, word, number of
+// trajectory rows), an exclusive scan of the row counts on the device, and an emission pass that writes
+// edge.trajectory[:,1:2] rows into a CSR.
+// Library built with -fmad=false: no contraction changes the operation order.
 #include <cmath>
 
 #include "common.cuh"
+#include "dubins.cuh"
 #include "scan.cuh"
 
 namespace rrtqx {
 
 namespace {
-
-constexpr double DB_PI = 3.141592653589793;  // Julia's Float64(pi)
-constexpr double DB_DPHI = 0.1;              // delta_phi, :506
-
-struct P2 {
-  double x, y;
-};
-
-__device__ __forceinline__ double len2(P2 a, P2 b) {  // sqrt(sum((a - b).^2))
-  const double dx = a.x - b.x, dy = a.y - b.y;
-  return sqrt(dx * dx + dy * dy);
-}
-// arc length from a to b around c turning right / left (DRRT_distance_functions.jl:62-80)
-__device__ __forceinline__ double turn_right(P2 a, P2 b, P2 c, double r) {
-  double th = atan2(a.y - c.y, a.x - c.x) - atan2(b.y - c.y, b.x - c.x);
-  if (th < 0) th = th + 2 * DB_PI;
-  return th * r;
-}
-__device__ __forceinline__ double turn_left(P2 a, P2 b, P2 c, double r) {
-  double th = atan2(b.y - c.y, b.x - c.x) - atan2(a.y - c.y, a.x - c.x);
-  if (th < 0) th = th + 2 * DB_PI;
-  return th * r;
-}
-
-// The winning word in a form the emission can walk: three pieces, each either an arc (centre, from,
-// to, direction) or the straight segment between the two transition points.
-struct Word {
-  double dist;
-  int type;      // 0 rsl, 1 rsr, 2 rlr, 3 lsr, 4 lsl, 5 lrl, -1 none
-  P2 c1, cm, c3; // first / middle / last turning circle
-  P2 t1, t2;     // transition points (tangent points, or the circle contact points of a CCC word)
-};
-
-__device__ inline Word solve(const double *s4, const double *g4, double r) {
-  const P2 il = {s4[0], s4[1]}, gl = {g4[0], g4[1]};
-  const double ith = s4[3], gth = g4[3];
-  // :346-356  centres of the right / left turning circles at both ends
-  const P2 irc = {il.x + r * cos(ith - DB_PI / 2.0), il.y + r * sin(ith - DB_PI / 2.0)};
-  const P2 ilc = {il.x + r * cos(ith + DB_PI / 2.0), il.y + r * sin(ith + DB_PI / 2.0)};
-  const P2 grc = {gl.x + r * cos(gth - DB_PI / 2.0), gl.y + r * sin(gth - DB_PI / 2.0)};
-  const P2 glc = {gl.x + r * cos(gth + DB_PI / 2.0), gl.y + r * sin(gth + DB_PI / 2.0)};
-  Word w;
-  w.dist = INFINITY;
-  w.type = -1;
-  w.c1 = w.cm = w.c3 = w.t1 = w.t2 = P2{0.0, 0.0};
-  auto offer = [&](double length, int type, P2 c1, P2 cm, P2 c3, P2 t1, P2 t2) {
-    if (w.dist > length) {  // strict: the earlier word wins ties
-      w.dist = length; w.type = type; w.c1 = c1; w.cm = cm; w.c3 = c3; w.t1 = t1; w.t2 = t2;
-    }
-  };
-  // inner tangents between a first circle A and a last circle B (rsl: sign = -1, lsr: sign = +1)
-  auto inner = [&](P2 A, P2 B, double sign, P2 &ta, P2 &tb) -> bool {
-    const double D = len2(B, A);
-    const double vx = (B.x - A.x) / D, vy = (B.y - A.y) / D;
-    const double R = sign * 2.0 * r / D;
-    if (fabs(R) > 1.0) return false;
-    const double sq = sqrt(1.0 - R * R);
-    if (sign < 0) {  // :373-377
-      const double a = r * (R * vx + vy * sq), b = r * (R * vy - vx * sq);
-      ta = P2{A.x - a, A.y - b};
-      tb = P2{B.x + a, B.y + b};
-    } else {         // :443-447
-      const double a = R * vx + vy * sq, b = R * vy - vx * sq;
-      ta = P2{A.x + a * r, A.y + b * r};
-      tb = P2{B.x - a * r, B.y - b * r};
-    }
-    return true;
-  };
-  P2 ta, tb;
-  // r-s-l :365-388
-  if (inner(irc, glc, -1.0, ta, tb))
-    offer(turn_right(il, ta, irc, r) + len2(tb, ta) + turn_left(tb, gl, glc, r), 0, irc, irc, glc, ta, tb);
-  // r-s-r :394-409 and r-l-r :413-433 (same centre line)
-  {
-    const double D = len2(grc, irc);
-    const double vx = (grc.x - irc.x) / D, vy = (grc.y - irc.y) / D;
-    ta = P2{-r * vy + irc.x, r * vx + irc.y};
-    tb = P2{-r * vy + grc.x, r * vx + grc.y};
-    offer(turn_right(il, ta, irc, r) + len2(tb, ta) + turn_right(tb, gl, grc, r), 1, irc, irc, grc, ta, tb);
-    if (D < 4.0 * r) {
-      const double th = -acos(D / (4 * r)) + atan2(vy, vx);
-      const P2 cm = {irc.x + 2 * r * cos(th), irc.y + 2 * r * sin(th)};
-      ta = P2{(cm.x + irc.x) / 2.0, (cm.y + irc.y) / 2.0};
-      tb = P2{(cm.x + grc.x) / 2.0, (cm.y + grc.y) / 2.0};
-      offer(turn_right(il, ta, irc, r) + turn_left(ta, tb, cm, r) + turn_right(tb, gl, grc, r), 2, irc, cm, grc, ta, tb);
-    }
-  }
-  // l-s-r :436-460
-  if (inner(ilc, grc, 1.0, ta, tb))
-    offer(turn_left(il, ta, ilc, r) + len2(tb, ta) + turn_right(tb, gl, grc, r), 3, ilc, ilc, grc, ta, tb);
-  // l-s-l :463-478 and l-r-l :481-499
-  {
-    const double D = len2(glc, ilc);
-    const double vx = (glc.x - ilc.x) / D, vy = (glc.y - ilc.y) / D;
-    ta = P2{r * vy + ilc.x, -r * vx + ilc.y};
-    tb = P2{r * vy + glc.x, -r * vx + glc.y};
-    offer(turn_left(il, ta, ilc, r) + len2(tb, ta) + turn_left(tb, gl, glc, r), 4, ilc, ilc, glc, ta, tb);
-    if (D < 4.0 * r) {
-      const double th = acos(D / (4 * r)) + atan2(vy, vx);
-      const P2 cm = {ilc.x + 2.0 * r * cos(th), ilc.y + 2.0 * r * sin(th)};
-      ta = P2{(cm.x + ilc.x) / 2.0, (cm.y + ilc.y) / 2.0};
-      tb = P2{(cm.x + glc.x) / 2.0, (cm.y + glc.y) / 2.0};
-      offer(turn_left(il, ta, ilc, r) + turn_right(ta, tb, cm, r) + turn_left(tb, gl, glc, r), 5, ilc, cm, glc, ta, tb);
-    }
-  }
-  return w;
-}
-
-// one arc piece: rows centre + r [cos(phi) sin(phi)], phi = phi_start, phi_start +- 0.1, ... up to phi_end
-// (a single row when the two angles coincide).  EMIT = false only counts.
-template <bool EMIT>
-__device__ __forceinline__ int arc_rows(P2 c, double r, P2 from, P2 to, bool right, double2 *out, int n) {
-  const double ps = atan2(from.y - c.y, from.x - c.x);
-  double pe = atan2(to.y - c.y, to.x - c.x);
-  double step;
-  if (right) {
-    if (pe > ps) pe = pe - 2.0 * DB_PI;
-    step = -DB_DPHI;
-  } else {
-    if (pe < ps) pe = pe + 2.0 * DB_PI;
-    step = DB_DPHI;
-  }
-  int rows = 1;
-  if (pe != ps) {
-    const double q = (pe - ps) / step;
-    rows = q >= 0.0 ? (int)floor(q) + 1 : 0;
-  }
-  if (EMIT)
-    for (int i = 0; i < rows; ++i) {
-      const double phi = ps + (double)i * step;
-      out[n + i] = make_double2(c.x + r * cos(phi), c.y + r * sin(phi));
-    }
-  return n + rows;
-}
-
-template <bool EMIT>
-__device__ inline int word_rows(const Word &w, const double *s4, const double *g4, double r, double2 *out) {
-  if (w.type < 0) return 0;
-  const bool first_right = w.type <= 2;                       // r**: 0,1,2
-  const bool last_right = w.type == 1 || w.type == 2 || w.type == 3;  // **r: rsr, rlr, lsr
-  const P2 il = {s4[0], s4[1]}, gl = {g4[0], g4[1]};
-  int n = arc_rows<EMIT>(w.c1, r, il, w.t1, first_right, out, 0);       // :508-548
-  if (w.type == 2) n = arc_rows<EMIT>(w.cm, r, w.t1, w.t2, false, out, n);        // rlr: middle left turn
-  else if (w.type == 5) n = arc_rows<EMIT>(w.cm, r, w.t1, w.t2, true, out, n);    // lrl: middle right turn
-  else {                                                                          // straight part :552-570
-    if (EMIT) { out[n] = make_double2(w.t1.x, w.t1.y); out[n + 1] = make_double2(w.t2.x, w.t2.y); }
-    n += 2;
-  }
-  return arc_rows<EMIT>(w.c3, r, w.t2, gl, last_right, out, n);         // :606-655
-}
 
 __global__ void dubins_size_kernel(const double *__restrict__ starts, const double *__restrict__ goals, int64_t n, double r,
                                    double *__restrict__ dist, int32_t *__restrict__ type, int32_t *__restrict__ rows) {
@@ -191,44 +34,17 @@ __global__ void dubins_emit_kernel(const double *__restrict__ starts, const doub
   word_rows<true>(w, starts + 4 * e, goals + 4 * e, r, traj + ptr[e]);
 }
 
-// saturate, DubinsEdge version (DRRT_DubinsEdge_functions.jl:70-95): dist = R3SDist (:41 of the
-// distance functions).  In place on new_points (n x 4).
+// saturate, DubinsEdge version (DRRT_DubinsEdge_functions.jl:70-95), in place on new_points (n x 4)
 __global__ void dubins_saturate_kernel(double *__restrict__ pts, const double *__restrict__ closest, int64_t n, double delta) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  double *p = pts + 4 * i;
-  const double *c = closest + 4 * i;
-  // R3SDist: sqrt(sum((x[1:3]-y[1:3]).^2) + min(|x4-y4|, min(x4,y4) + 2pi - max(x4,y4))^2)
-  const double dx = __dsub_rn(p[0], c[0]), dy = __dsub_rn(p[1], c[1]), dz = __dsub_rn(p[2], c[2]);
-  const double a = __dadd_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)), __dmul_rn(dz, dz));
-  const double w = jl_min(fabs(__dsub_rn(p[3], c[3])),
-                          __dsub_rn(__dadd_rn(jl_min(p[3], c[3]), 6.283185307179586), jl_max(p[3], c[3])));
-  const double d = __dsqrt_rn(__dadd_rn(a, __dmul_rn(w, w)));
-  if (d > delta) {
-    for (int k = 0; k < 3; ++k) p[k] = __dadd_rn(c[k], __ddiv_rn(__dmul_rn(__dsub_rn(p[k], c[k]), delta), d));
-    if (fabs(__dsub_rn(p[3], c[3])) < DB_PI) {
-      p[3] = __dadd_rn(c[3], __ddiv_rn(__dmul_rn(__dsub_rn(p[3], c[3]), delta), d));
-    } else {
-      p[3] = p[3] < DB_PI ? __dadd_rn(p[3], 2 * DB_PI) : __dsub_rn(p[3], 2 * DB_PI);
-      p[3] = __dadd_rn(c[3], __ddiv_rn(__dmul_rn(__dsub_rn(p[3], c[3]), delta), d));
-      p[3] = jl_max(jl_min(p[3], 2 * DB_PI), 0.0);
-    }
-  }
+  dubins_saturate_point(pts + 4 * i, closest + 4 * i, delta);
 }
 
 }  // namespace
 }  // namespace rrtqx
 
 using namespace rrtqx;
-
-struct rrtqx_dubins_result {
-  rrtqx_ctx *ctx = nullptr;
-  int64_t n_edges = 0, n_rows = 0;
-  DevBuf<double> starts, goals, dist;
-  DevBuf<int32_t> type, rows, scan_tmp;
-  DevBuf<int64_t> ptr, scan_tmp64;
-  DevBuf<double2> traj;
-};
 
 namespace {
 template <typename F>

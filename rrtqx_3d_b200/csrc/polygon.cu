@@ -61,13 +61,6 @@ dubins_check_v1_kernel(PolyView P, int ignore_active, const double *__restrict__
 #endif  // RRTQX_LEGACY
 
 // Dubins explicitEdgeCheck OR-ed over ALL obstacles of the set: one warp per edge (dubins_collide_warp, polygon.cuh).
-struct AllObstacles {
-  int n;
-  __device__ __forceinline__ int count() const { return n; }
-  __device__ __forceinline__ int id(int k) const { return k; }
-  __device__ __forceinline__ bool admit(int) const { return true; }
-};
-
 #ifndef DUBINS_MINB
 #define DUBINS_MINB 6  // FP64 dependency chains: latency-bound, 48 warps per SM beat 16 although 40 registers spill (0.93 -> 0.60 ms on C4)
 #endif

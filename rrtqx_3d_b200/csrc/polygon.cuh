@@ -155,6 +155,14 @@ __device__ __forceinline__ bool dubins_collide_warp(const PolyView &P, bool igno
   return collide;
 }
 
+// selector of dubins_collide_warp: every obstacle of the set
+struct AllObstacles {
+  int n;
+  __device__ __forceinline__ int count() const { return n; }
+  __device__ __forceinline__ int id(int k) const { return k; }
+  __device__ __forceinline__ bool admit(int) const { return true; }
+};
+
 }  // namespace rrtqx
 
 struct rrtqx_polygons {

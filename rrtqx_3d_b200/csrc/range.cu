@@ -11,7 +11,9 @@
 #include <cmath>
 #include <cstdlib>
 
+#include "dubins.cuh"
 #include "objects.cuh"
+#include "polygon.cuh"
 #include "scan.cuh"
 
 namespace rrtqx {
@@ -407,20 +409,13 @@ void range_query(rrtqx_tree *t, const double *queries, int64_t nq, double r, con
 // ---------------------------------------------------------- nearest kernel
 // One warp per query; cube of cells of growing half-width rho around the
 // query's cell until no unseen cell can hold a closer point.
+// nearest_warp: kdFindNearest of one query q0 by one warp (all 32 lanes take part); the result is warp-uniform.
+// Shared by nearest_kernel and the fused Dubins extend query (extend_dubins.cuh).
 template <int D, bool WRAP>
-__global__ void __launch_bounds__(256)
-nearest_kernel(GridView g, WrapInfo wrap, const double *__restrict__ queries, const int32_t *__restrict__ qorder,
-               int64_t nq, int32_t *__restrict__ out_idx, double *__restrict__ out_dist) {
+__device__ inline void nearest_warp(const GridView &g, const WrapInfo &wrap, const double *q0, int &out_node,
+                                    double &out_dist) {
   const int lane = lane_id();
-  const int64_t warp0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
-
-  for (int64_t qi = warp0; qi < nq; qi += nwarps) {
-    const int qid = qorder[qi];
-    double q0[D];
-#pragma unroll
-    for (int k = 0; k < D; ++k) q0[k] = queries[(int64_t)qid * D + k];
-
+  {
     // best over all identities so far (distance = sqrt of radicand; strict <
     // replacement, kdTree_general.jl:375-379)
     double best_dist = INFINITY;
@@ -533,6 +528,27 @@ nearest_kernel(GridView g, WrapInfo wrap, const double *__restrict__ queries, co
         best_dist = __dsqrt_rn(s0);
       }
     }
+    out_node = best_node;
+    out_dist = best_dist;
+  }
+}
+
+template <int D, bool WRAP>
+__global__ void __launch_bounds__(256)
+nearest_kernel(GridView g, WrapInfo wrap, const double *__restrict__ queries, const int32_t *__restrict__ qorder,
+               int64_t nq, int32_t *__restrict__ out_idx, double *__restrict__ out_dist) {
+  const int lane = lane_id();
+  const int64_t warp0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+
+  for (int64_t qi = warp0; qi < nq; qi += nwarps) {
+    const int qid = qorder[qi];
+    double q0[D];
+#pragma unroll
+    for (int k = 0; k < D; ++k) q0[k] = queries[(int64_t)qid * D + k];
+    int best_node;
+    double best_dist;
+    nearest_warp<D, WRAP>(g, wrap, q0, best_node, best_dist);
     if (lane == 0) {
       out_idx[qid] = best_node;
       if (out_dist) out_dist[qid] = best_dist;
@@ -700,5 +716,7 @@ void nearest_query(rrtqx_tree *t, rrtqx_range_result *sortbuf, const double *que
     default: throw Error(RRTQX_ERR_UNSUPPORTED, "d must be 2, 3 or 4");
   }
 }
+
+#include "extend_dubins.cuh"
 
 }  // namespace rrtqx

@@ -624,6 +624,76 @@ def dubins_saturate_batch(ctx: Context, new_points, closest, delta):
     return pts
 
 
+class ExtendDubinsResult:
+    """Outputs of one rrtqx_extend_query_dubins call.  Edge 2i runs new -> idx[i], edge 2i+1 idx[i] -> new."""
+    __slots__ = ("point", "nearest_idx", "nearest_dist", "count", "idx", "dist", "edge_dist", "edge_type",
+                 "edge_collide", "trajectories")
+
+
+def extend_query_dubins(tree: DeviceTree, polys: PolygonSet, point, r, robot_radius, min_turn_radius, delta=0.0,
+                        flags=0, capacity=8192, trajectories: DubinsResult | bool | None = None):
+    """The DubinsEdge planner's per-iteration work in one call on the [x y t theta] tree with the theta wrap:
+    nearest, saturate (flags | EXTEND_SATURATE), the ball of radius r, and calculateTrajectory + explicitEdgeCheck
+    of both edges per neighbour.  trajectories: a DubinsResult to keep the rows in (True: a new one), or None."""
+    p = np.array(A.as_f64(point).reshape(-1), copy=True)
+    assert p.size == 4, "point must hold [x y t theta]"
+    idx, dist = np.empty(max(capacity, 1), dtype=np.int32), np.empty(max(capacity, 1))
+    edist, etype = np.empty(2 * max(capacity, 1)), np.empty(2 * max(capacity, 1), dtype=np.int32)
+    ecol = np.empty(2 * max(capacity, 1), dtype=np.uint8)
+    if trajectories is True:
+        trajectories = DubinsResult(tree.ctx)
+    ni, nd, cnt = A.i32(0), A.f64(0.0), A.i32(0)
+    A.check(tree.L.rrtqx_extend_query_dubins(tree.h, polys.h, A.ptr(p), float(delta), float(r), float(robot_radius),
+                                             float(min_turn_radius), int(flags), int(capacity), C.byref(ni),
+                                             C.byref(nd), C.byref(cnt), A.ptr(idx), A.ptr(dist), A.ptr(edist),
+                                             A.ptr(etype), A.ptr(ecol),
+                                             C.byref(trajectories.h) if trajectories is not None else None),
+            tree.ctx.h)
+    out = ExtendDubinsResult()
+    out.point, out.nearest_idx, out.nearest_dist, out.count = p, int(ni.value), float(nd.value), int(cnt.value)
+    m = min(out.count, capacity)
+    out.idx, out.dist = idx[:m], dist[:m]
+    out.edge_dist, out.edge_type, out.edge_collide = edist[:2 * m], etype[:2 * m], ecol[:2 * m]
+    out.trajectories = trajectories
+    return out
+
+
+def extend_query_dubins_composed(tree: DeviceTree, polys: PolygonSet, point, r, robot_radius, min_turn_radius,
+                                 node_positions, delta=0.0, flags=0, trajectories: DubinsResult | None = None,
+                                 range_result: RangeResult | None = None):
+    """The work of extend_query_dubins through the batch entry points, one blocking call each: nearest ->
+    saturate -> range query -> Dubins trajectories -> Dubins edge check (the rows stay on the device).
+    node_positions: the caller's host copy of the tree's n x 4 positions (the planner's node table)."""
+    p = np.array(A.as_f64(point, 4), copy=True)
+    ni, nd = tree.nearest(p)
+    if flags & A.EXTEND_SATURATE:
+        p = dubins_saturate_batch(tree.ctx, p, node_positions[int(ni[0])], delta)
+    res, total = tree.range_query(p, r, want_dist=True, result=range_result)
+    idx, dist = res.fetch()
+    nb = node_positions[idx]
+    starts, goals = np.empty((2 * total, 4)), np.empty((2 * total, 4))
+    starts[0::2], starts[1::2] = p, nb          # edge 2i: new -> nbr i, edge 2i+1: nbr i -> new
+    goals[0::2], goals[1::2] = nb, p
+    if trajectories is None:
+        trajectories = DubinsResult(tree.ctx)
+    out = ExtendDubinsResult()
+    out.point, out.nearest_idx, out.nearest_dist, out.count = p.reshape(-1), int(ni[0]), float(nd[0]), int(total)
+    out.idx, out.dist = idx, dist
+    out.edge_dist, out.edge_type = np.empty(2 * total), np.empty(2 * total, dtype=np.int32)
+    out.edge_collide = np.zeros(2 * total, dtype=np.uint8)
+    out.trajectories = trajectories
+    dubins_trajectory_batch(tree.ctx, starts, goals, min_turn_radius, result=trajectories)
+    if total:
+        A.check(tree.L.rrtqx_dubins_result_fetch(trajectories.h, A.ptr(out.edge_dist), A.ptr(out.edge_type), None,
+                                                 None), tree.ctx.h)
+        _, _, dptr, dxy = trajectories.device_pointers()
+        s2, g2 = np.ascontiguousarray(starts[:, :2]), np.ascontiguousarray(goals[:, :2])
+        A.check(polys.L.rrtqx_dubins_edge_check_batch(polys.h, A.ptr(s2), A.ptr(g2), dptr, dxy, 2 * total,
+                                                      float(robot_radius), float(min_turn_radius), int(flags),
+                                                      A.ptr(out.edge_collide)), polys.ctx.h)
+    return out
+
+
 class Comm:
     """rrtqx_comm: the ranks of a sharded job.  Comm.local(ctxs): ONE process driving one context per device (the
     reference's host is one process); Comm.rank(ctx, id, rank, n): one process per GPU (torchrun), `id` being the
