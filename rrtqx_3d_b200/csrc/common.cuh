@@ -7,6 +7,7 @@
 #include <cuda_runtime.h>
 
 #include <atomic>
+#include <cmath>
 #include <cstdint>
 #include <cstdio>
 #include <cstring>
@@ -108,12 +109,10 @@ inline bool is_device_ptr(const void *p) {
 // iteration.  None of the switches selects a CPU path.
 namespace rrtqx {
 struct Tuning {
-  bool edge_no_grid = false, edge_no_queue = false, dubins_check_v1 = false, range_two_pass = false,
-       nearest_warp = false, no_item_grid = false;
+  bool edge_no_grid = false, edge_no_queue = false, range_two_pass = false, nearest_warp = false, no_item_grid = false;
   int64_t cover_min_items = -1;  // < 0: the measured break-even defaults
   int fused_variant = -1;        // < 0: chosen from the expected neighbour count
-  int range_kernel = 5, v5_nw = 24, qsort_s = 2, qsort_f = 1;   // supercells of 2^3 cells with the 2:1 grid aspect (scripts/tune_v5.sh)
-  unsigned v5_unit = 0;          // 0: V5_UNIT
+  int qsort_s = 2, qsort_f = 1;  // supercells of 2^3 cells with the 2:1 grid aspect (scripts/tune_v5.sh)
   bool comm_no_ipc = false;      // one process per GPU: gathers through NCCL even where IPC windows are possible
   int comm_ipc_mb = 64;          // bytes per slot of the IPC result window (two slots per rank), MiB
   int nccl_max_ctas = 0;         // cap on the CTAs NCCL may use for this library's gathers (0: NCCL's default; caps of 1-4 measured slower on 8 B200s)
@@ -125,16 +124,11 @@ struct Tuning {
     auto getd = [](const char *n) { const char *e = getenv(n); return e ? atof(e) : 0.0; };
     edge_no_grid = on("RRTQX_EDGE_NO_GRID");
     edge_no_queue = on("RRTQX_EDGE_NO_QUEUE");
-    dubins_check_v1 = on("RRTQX_DUBINS_CHECK_V1");
     range_two_pass = on("RRTQX_RANGE_TWO_PASS");
     nearest_warp = on("RRTQX_NEAREST_WARP");
     no_item_grid = on("RRTQX_NO_ITEM_GRID");
     cover_min_items = geti("RRTQX_COVER_MIN_ITEMS", -1);
     fused_variant = (int)geti("RRTQX_FUSED_VARIANT", -1);
-    range_kernel = (int)geti("RRTQX_RANGE_KERNEL", 5);
-    v5_nw = (int)geti("RRTQX_V5_NW", 24);
-    const long long u = geti("RRTQX_V5_UNIT", 0);
-    v5_unit = (unsigned)(u > 0 ? u : 0);
     nccl_max_ctas = (int)geti("RRTQX_NCCL_MAX_CTAS", 0);
     comm_no_ipc = on("RRTQX_COMM_NO_IPC");
     { const long long mb = geti("RRTQX_COMM_IPC_MB", 64); comm_ipc_mb = (int)(mb < 1 ? 1 : (mb > 4096 ? 4096 : mb)); }
@@ -332,6 +326,21 @@ __device__ inline double sqrt_thresh_lt(double r) {
   }
   while (t > 0.0 && __dsqrt_rn(t) >= r) t = next_down(t);
   while (__dsqrt_rn(t) < r) t = next_up(t);
+  return t;
+}
+
+// Host twin of sqrt_thresh_lt (std::sqrt is correctly rounded, like __dsqrt_rn).
+inline double host_sqrt_thresh_lt(double r) {
+  if (r != r) return r;
+  if (r <= 0.0) return 0.0;
+  if (std::isinf(r)) return r;
+  double t = r * r;
+  if (std::isinf(t)) {
+    t = 1.7976931348623157e308;
+    if (std::sqrt(t) < r) return INFINITY;
+  }
+  while (t > 0.0 && std::sqrt(t) >= r) t = std::nextafter(t, -INFINITY);
+  while (std::sqrt(t) < r) t = std::nextafter(t, INFINITY);
   return t;
 }
 

@@ -13,6 +13,46 @@
 constexpr int EXT_WARPS = 16;
 constexpr int EXT_MAX_SPHERES = 768;
 
+struct FGrid {
+  float inv[3], cell[3];
+};
+
+__device__ __forceinline__ int clampi(float v, int n) {  // floor + clamp to [0, n-1]; NaN -> 0
+  return (int)fminf(fmaxf(floorf(v), 0.0f), (float)(n - 1));
+}
+
+// Conservative cell range [cxa, cxb] of row (cy,cz) that can hold a point within r of the query at
+// ff (cell units); false if the row is out of reach.
+template <int D>
+__device__ __forceinline__ bool row_cells(const GridView &g, const FGrid &fg, const float *ff, float r2f, int cy, int cz,
+                                          int &cxa, int &cxb) {
+  // lower bounds of |p.y - q.y|, |p.z - q.z| in cell units; boundary rows also
+  // hold the points clamped in from beyond the grid, so they give no bound on
+  // that side.  1e-3 cells of slack covers the FP32 error of ff (coordinates
+  // up to 1024 cells: ulp 6e-5) and the FP64 rounding of cell_of().
+  const float ninf = -INFINITY;
+  float dyc = fmaxf(cy == 0 ? ninf : (float)cy - ff[1], cy == g.ny - 1 ? ninf : ff[1] - (float)(cy + 1));
+  dyc = fmaxf(dyc - 1e-3f, 0.0f);
+  const float dy = dyc * fg.cell[1];
+  float rem = r2f - dy * dy;
+  if (D >= 3) {
+    float dzc = fmaxf(cz == 0 ? ninf : (float)cz - ff[2], cz == g.nz - 1 ? ninf : ff[2] - (float)(cz + 1));
+    dzc = fmaxf(dzc - 1e-3f, 0.0f);
+    const float dz = dzc * fg.cell[2];
+    rem -= dz * dz;
+  }
+  if (isinf(r2f)) {  // unbounded query: whole row
+    cxa = 0;
+    cxb = g.nx - 1;
+    return true;
+  }
+  if (!(rem >= 0.0f)) return false;
+  const float xc = sqrtf(rem) * (1.0f + 1e-5f) * fg.inv[0] + 1e-3f;
+  cxa = clampi(ff[0] - xc, g.nx);
+  cxb = clampi(ff[0] + xc, g.nx);
+  return true;
+}
+
 struct ExtendEntry {   // 16 bytes
   int32_t node;
   uint8_t fwd, rev;

@@ -135,7 +135,7 @@ extend_dubins_query_kernel(GridView g, WrapInfo wrap, const ExtendDubinsParams p
       const int wy = cy1 - cy0 + 1;
       const int nrows = wy * (cz1 - cz0 + 1);
       for (int row = warp; row < nrows; row += EXD_WARPS) {
-        const RowSpan sp = row_span<4>(g, q, r_infl, r2_infl, cy0 + row % wy, cz0 + row / wy);
+        const RowSpan sp = row_span<4>(g, q, r2_infl, cy0 + row % wy, cz0 + row / wy);
         for (int j0 = sp.start; j0 < sp.end; j0 += 32) {
           const int j = j0 + lane;
           bool hit = false;

@@ -348,14 +348,11 @@ ig_units_kernel(ItemGridView G0, ItemGridView G1, int n_upper, const double4 *__
 // obstacle: |c - mid| + len/2 <= thr, so the reference's D, a distance to a point ON the segment, is <= thr) / needs the
 // exact test; the last kind is compacted into a per-warp list.  Phase 2 runs the exact FP64 test
 // (distancePointToSegment, 2 sqrt + 1 div) on that list with every lane busy.
-#ifndef IG_TEST_BLOCKS
-#define IG_TEST_BLOCKS 4
-#endif
-#ifndef IG_TEST_WAVES
-#define IG_TEST_WAVES 1
-#endif
+// One wave of persistent blocks, 4 per SM at 64 registers (5 / 6 blocks per SM spill and are 10 / 23 % slower,
+// 3 blocks 4 % slower).
+constexpr int IG_BLOCKS_PER_SM = 4;
 template <bool FMA_DOT, class Sink>
-static __global__ void __launch_bounds__(256, IG_TEST_BLOCKS)
+static __global__ void __launch_bounds__(256, IG_BLOCKS_PER_SM)
 ig_test_kernel(ItemGridView G0, ItemGridView G1, const IgObstacle *__restrict__ obs, const uint2 *__restrict__ units_all,
                const unsigned long long *__restrict__ cursors, int64_t cap, const int32_t *__restrict__ overflow, Sink S) {
   // per warp: two TMA tiles of FP32 records (the unit being classified and the next one in flight), their mbarriers,
@@ -632,7 +629,7 @@ static inline const int32_t *item_grid_run(rrtqx_ctx *ctx, const ItemGridBufs &B
   const int64_t cap = IG_MAX_UNITS / 2;
   ig_units_kernel<<<(has1 ? 2 : 1) * n_upper, 256, 0, st>>>(G0, G1, n_upper, rec, thr, ext, n_live, obs, R.obs_f.p, R.obs_aux.p,
                                                           n_obs, R.cursor.p, R.units.p, cap, overflow);
-  ig_test_kernel<FMA_DOT, Sink><<<ctx->sm_count * IG_TEST_WAVES * IG_TEST_BLOCKS, 256, 0, st>>>(G0, G1, obs, R.units.p, R.cursor.p, cap, overflow, S);
+  ig_test_kernel<FMA_DOT, Sink><<<ctx->sm_count * IG_BLOCKS_PER_SM, 256, 0, st>>>(G0, G1, obs, R.units.p, R.cursor.p, cap, overflow, S);
   post_launch(ctx, 2);
   if (last->n_degenerate > 0) {
     const ItemGridView G = last->view();

@@ -24,47 +24,9 @@ segment_check_2d_kernel(PolyView P, int ignore_active, const double *__restrict_
   out[i] = hit ? 1 : 0;
 }
 
-#ifdef RRTQX_LEGACY
-// (legacy A/B build only, make EXTRA=-DRRTQX_LEGACY + RRTQX_DUBINS_CHECK_V1=1)
-// Dubins explicitEdgeCheck OR-ed over all obstacles: one warp per edge.  Lanes run the coarse
-// start->end test (radius rho + 2 r_turn) over 32 obstacles at a time; each surviving obstacle
-// is then tested against the trajectory segments, 32 segments per trip.
-__global__ void __launch_bounds__(256)
-dubins_check_v1_kernel(PolyView P, int ignore_active, const double *__restrict__ starts, const double *__restrict__ ends,
-                    const int64_t *__restrict__ tptr, const double *__restrict__ traj, int64_t n_edges, double rho,
-                    double rho_coarse, uint8_t *__restrict__ out) {
-  const int lane = lane_id();
-  const int64_t e = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  if (e >= n_edges) return;
-  const double sx = starts[2 * e], sy = starts[2 * e + 1], ex = ends[2 * e], ey = ends[2 * e + 1];
-  const int64_t t0 = tptr[e], t1 = tptr[e + 1];
-  bool collide = false;
-  for (int o0 = 0; o0 < P.n && !collide; o0 += 32) {
-    const int o = o0 + lane;
-    const bool coarse = o < P.n && edge_check_2d(P, o, ignore_active, sx, sy, ex, ey, rho_coarse);  // :757-760
-    unsigned m = __ballot_sync(FULL, coarse);
-    while (m && !collide) {
-      const int ob = o0 + __ffs(m) - 1;
-      m &= m - 1;
-      for (int64_t i0 = t0 + 1; i0 < t1 && !collide; i0 += 32) {  // for i = 2:size(trajectory,1)  :767-771
-        const int64_t i = i0 + lane;
-        bool hit = false;
-        if (i < t1)
-          hit = edge_check_2d(P, ob, ignore_active, traj[2 * (i - 1)], traj[2 * (i - 1) + 1], traj[2 * i],
-                              traj[2 * i + 1], rho);
-        collide = __any_sync(FULL, hit);
-      }
-    }
-  }
-  if (lane == 0) out[e] = collide ? 1 : 0;
-}
-#endif  // RRTQX_LEGACY
-
 // Dubins explicitEdgeCheck OR-ed over ALL obstacles of the set: one warp per edge (dubins_collide_warp, polygon.cuh).
-#ifndef DUBINS_MINB
-#define DUBINS_MINB 6  // FP64 dependency chains: latency-bound, 48 warps per SM beat 16 although 40 registers spill (0.93 -> 0.60 ms on C4)
-#endif
-__global__ void __launch_bounds__(256, DUBINS_MINB)
+constexpr int DUBINS_CHECK_BLOCKS_PER_SM = 6;  // FP64 dependency chains: latency-bound, 48 warps per SM beat 16 although 40 registers spill (0.93 -> 0.60 ms on C4)
+__global__ void __launch_bounds__(256, DUBINS_CHECK_BLOCKS_PER_SM)
 dubins_check_kernel(PolyView P, int ignore_active, const double *__restrict__ starts, const double *__restrict__ ends,
                     const int64_t *__restrict__ tptr, const double *__restrict__ traj, int64_t n_edges, double rho,
                     double rho_coarse, uint8_t *__restrict__ out) {
@@ -200,14 +162,8 @@ rrtqx_status rrtqx_dubins_edge_check_batch(rrtqx_polygons *p, const double *star
       PhaseScope ph(ctx, "dubins_check");
       // S.robotRadius + 2*S.minTurningRadius (DRRT_DubinsEdge_functions.jl:758)
       const double rho_coarse = robot_radius + 2 * min_turn_radius;
-#ifdef RRTQX_LEGACY
-      if (ctx->tune.dubins_check_v1)
-        dubins_check_v1_kernel<<<div_up(n_edges * 32, 256), 256, 0, st>>>(p->view(), (flags & RRTQX_CHECK_IGNORE_ACTIVE) ? 1 : 0,
-                                                                         ds, de, dp, dt, n_edges, robot_radius, rho_coarse, dout);
-      else
-#endif
-        dubins_check_kernel<<<div_up(n_edges * 32, 256), 256, 0, st>>>(p->view(), (flags & RRTQX_CHECK_IGNORE_ACTIVE) ? 1 : 0,
-                                                                      ds, de, dp, dt, n_edges, robot_radius, rho_coarse, dout);
+      dubins_check_kernel<<<div_up(n_edges * 32, 256), 256, 0, st>>>(p->view(), (flags & RRTQX_CHECK_IGNORE_ACTIVE) ? 1 : 0,
+                                                                    ds, de, dp, dt, n_edges, robot_radius, rho_coarse, dout);
       post_launch(ctx);
     }
     if (!od) from_device(ctx, collide_out, dout, (size_t)n_edges);

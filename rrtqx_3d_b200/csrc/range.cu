@@ -108,12 +108,6 @@ static void sort_queries(rrtqx_tree *t, rrtqx_range_result *r, const double *dq,
 // wraps dimension wraps[w-1-b]; a ghost is used iff
 // !(euclid(closestUnwrappedPoint, ghost) > bound) (:104).
 template <int D>
-struct Identities {
-  double q[1 << MAX_WRAPS][D];
-  int count;
-};
-
-template <int D>
 __device__ inline bool make_ghost(const WrapInfo &w, const double *q, int pattern, double bound, double *ghost) {
   double closest[D];
 #pragma unroll
@@ -138,8 +132,7 @@ struct RowSpan { int start, end; };
 
 // Conservative slice of row (cy,cz) that can contain points within r of q.
 template <int D>
-__device__ __forceinline__ RowSpan row_span(const GridView &g, const double *q, double r_infl, double r2_infl, int cy,
-                                           int cz) {
+__device__ __forceinline__ RowSpan row_span(const GridView &g, const double *q, double r2_infl, int cy, int cz) {
   // lower bounds of |p.y-q.y| and |p.z-q.z| for points stored in this row;
   // boundary rows extend to infinity (clamped cells hold everything beyond).
   double dy = 0.0, dz = 0.0;
@@ -159,7 +152,6 @@ __device__ __forceinline__ RowSpan row_span(const GridView &g, const double *q, 
   double rem = r2_infl - dy * dy - dz * dz;
   if (!(rem >= 0.0)) { s.start = 0; s.end = 0; return s; }
   double xr = isinf(rem) ? rem : sqrt(rem) * (1.0 + 1e-9) + 1e-12 * fabs(q[0]);
-  (void)r_infl;
   int cxa = cell_of(q[0] - xr, g.lo[0], g.inv[0], g.nx);
   int cxb = cell_of(q[0] + xr, g.lo[0], g.inv[0], g.nx);
   int base = (cz * g.ny + cy) * g.nx;
@@ -267,7 +259,7 @@ range_query_kernel(GridView g, WrapInfo wrap, const double *__restrict__ queries
         for (int rb = 0; rb < nrows; rb += 32) {
           RowSpan sp{0, 0};
           int row = rb + lane;
-          if (row < nrows) sp = row_span<D>(g, q, r_infl, r2_infl, cy0 + row % wy, cz0 + row / wy);
+          if (row < nrows) sp = row_span<D>(g, q, r2_infl, cy0 + row % wy, cz0 + row / wy);
           const int lim = min(32, nrows - rb);
           for (int t = 0; t < lim; ++t) {
             const int a = __shfl_sync(FULL, sp.start, t);
@@ -331,8 +323,7 @@ static void launch_range(rrtqx_tree *t, bool fill, const double *dq, const int32
   post_launch(ctx);
 }
 
-
-#include "range_fused.cuh"
+#include "range_v5.cuh"
 #include "extend.cuh"
 
 template <int D>

@@ -1,9 +1,12 @@
 // range_v5.cuh -- single-pass batched kdFindWithinRange, fifth generation (included by range.cu,
-// inside namespace rrtqx, after range_fused.cuh whose row_cells / octet-table ideas it keeps).
+// inside namespace rrtqx).
 //
-// What changed against range_fused_kernel (profiles/README.md, "what the range kernel is bound by"):
-// the v4 kernel was instruction-issue bound (2450 warp-instructions per query: 1160 in the candidate
-// tests, 620 in the flush, 670 in set-up), so v5 removes instructions, not bytes:
+// One warp per pair of consecutive (cell-sorted) queries: the candidate rows of the pair are flattened
+// into a shared-memory table of octets (start slot, 1..8 points), each 8-lane sub-group takes one octet
+// per trip, hits are buffered per query and flushed densely after one atomic reserves the pair's output.
+// The previous generation (v4) was instruction-issue bound (profiles/README.md, "what the range kernel is
+// bound by": 2450 warp-instructions per query: 1160 in the candidate tests, 620 in the flush, 670 in
+// set-up), so v5 removes instructions, not bytes:
 //   * the candidate scan runs on an FP32 *filter*: slot records float4((x,y,z) - grid origin, w) are
 //     fetched with ONE 128-bit load and both queries of the warp's pair are tested with packed
 //     f32x2 arithmetic (sm_100 FADD2/FFMA2: 6 instructions for 2 x 32 tests).  The filter computes
@@ -20,13 +23,25 @@
 //     routine, so they cost no registers in the hot path.
 
 constexpr int V5_TABPAD = 16;  // zero entries behind the last one (a trip group never tests bounds)
-constexpr int V5_UNIT = 128;    // pairs per dynamically scheduled unit of work (a block's warps share one unit; scripts/tune_v5b.sh: 48 / 64 / 96 / 128 / 160 / 256 -> 2.78 / 2.69 / 2.70 / 2.665 / 2.664 / 2.70 ms)
+constexpr int V5_UNIT = 128;    // pairs per dynamically scheduled unit of work (a block's warps share one unit; C2 kernel time at 48 / 64 / 96 / 128 / 160 / 256 pairs: 2.78 / 2.69 / 2.70 / 2.665 / 2.664 / 2.70 ms)
 constexpr int V5_RING = 64;     // published unit bases kept per block
-#ifndef V5_U_TRIPS
-#define V5_U_TRIPS 4
-#endif
-constexpr int V5_U = V5_U_TRIPS;   // trips per loop iteration (loads in flight before the first test)
+constexpr int V5_U = 4;         // trips per loop iteration (loads in flight before the first test)
 
+__device__ __forceinline__ void sts32(unsigned addr, int v) {
+  asm volatile("st.shared.b32 [%0], %1;" ::"r"(addr), "r"(v) : "memory");
+}
+__device__ __forceinline__ int lds32(unsigned addr) {
+  int v;
+  asm volatile("ld.shared.b32 %0, [%1];" : "=r"(v) : "r"(addr) : "memory");
+  return v;
+}
+// keeps a value in a register (stops the compiler from re-deriving it from
+// special registers inside the hot loop)
+__device__ __forceinline__ unsigned pin_reg(unsigned v) {
+  unsigned r;
+  asm volatile("mov.u32 %0, %1;" : "=r"(r) : "r"(v));
+  return r;
+}
 __device__ __forceinline__ unsigned long long pk2(float a, float b) {
   unsigned long long r;
   asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(a), "f"(b));
@@ -59,29 +74,11 @@ __device__ __forceinline__ double4 ldg256(const double4 *p) {
   return v;
 }
 
-// Result stores.  The lists are written once and never read by the kernel: streaming stores (evict-first) keep the
-// 5 GB of output from pushing the 64 MB of records / cell starts out of L2.
-#ifndef V5_STORE_MODE
-#define V5_STORE_MODE 0
-#endif
-__device__ __forceinline__ void v5_st(int32_t *p, int32_t v) {
-#if V5_STORE_MODE == 1
-  __stcs(p, v);
-#elif V5_STORE_MODE == 2
-  __stwt(p, v);
-#else
-  *p = v;
-#endif
-}
-__device__ __forceinline__ void v5_st(double *p, double v) {
-#if V5_STORE_MODE == 1
-  __stcs(p, v);
-#elif V5_STORE_MODE == 2
-  __stwt(p, v);
-#else
-  *p = v;
-#endif
-}
+// Result stores of the flush.  Kept as calls: the same stores written inline change how the compiler schedules and
+// spills range_v5_kernel (other spill counts and stack frames), and the code generated through these calls is the
+// one that was measured.
+__device__ __forceinline__ void v5_st(int32_t *p, int32_t v) { *p = v; }
+__device__ __forceinline__ void v5_st(double *p, double v) { *p = v; }
 
 // double -> float rounded up (host twin: nextafter of the nearest conversion when it fell below)
 __host__ __device__ __forceinline__ float f32_up(double x) {
@@ -153,7 +150,7 @@ __device__ __noinline__ int v5_exact_query(const GridView *gp, const double *qpt
     for (int rb = 0; rb < nrows; rb += 32) {
       RowSpan sp{0, 0};
       const int row = rb + lane;
-      if (row < nrows) sp = row_span<D>(g, q, r_infl, r2_infl, cy0 + row % wy, cz0 + row / wy);
+      if (row < nrows) sp = row_span<D>(g, q, r2_infl, cy0 + row % wy, cz0 + row / wy);
       const int lim = min(32, nrows - rb);
       for (int t = 0; t < lim; ++t) {
         const int a = __shfl_sync(FULL, sp.start, t);
@@ -188,10 +185,7 @@ __device__ __noinline__ int v5_exact_query(const GridView *gp, const double *qpt
 template <int D, bool TAIL>
 __device__ __forceinline__ void v5_flush(const GridView &g, const double *q, unsigned sbuf_k, unsigned stab, int n, int lane,
                                          int32_t *__restrict__ oi, double *__restrict__ od) {
-#ifndef V5_FLUSH_U
-#define V5_FLUSH_U 4
-#endif
-  constexpr int U = V5_FLUSH_U;  // rows of 32 hits in flight per flush step
+  constexpr int U = 4;  // rows of 32 hits in flight per flush step
   auto fetch = [&](unsigned h, int &node, double4 &p) {
     if (!TAIL || !(h & 0x8000u)) {
       const int ent = lds32(stab + 4u * (h >> 3));
@@ -236,7 +230,7 @@ __device__ __forceinline__ void v5_flush(const GridView &g, const double *q, uns
       }
   };
   const int rem = n - n_full;
-  if (U >= 4 && rem > 64) tail(std::integral_constant<int, (U >= 4 ? 4 : 1)>{});
+  if (rem > 64) tail(std::integral_constant<int, 4>{});
   else if (rem > 32) tail(std::integral_constant<int, 2>{});
   else if (rem > 0) tail(std::integral_constant<int, 1>{});
 }
@@ -739,7 +733,7 @@ static void launch_v5(rrtqx_ctx *ctx, const GridView &g, const double *dq, const
   P.RU = v5_radius(r, T, true);
   P.invx = (float)g.inv[0]; P.invy = (float)g.inv[1]; P.invz = (float)g.inv[2];
   P.celly = (float)g.cell[1]; P.cellz = (float)g.cell[2];
-  P.unit = ctx->tune.v5_unit ? ctx->tune.v5_unit : (unsigned)V5_UNIT;
+  P.unit = V5_UNIT;
   P.ghost_pairs = ghost_pairs;
   const int64_t n_units = ((nq + 1) / 2 + P.unit - 1) / P.unit;
   const int blocks = (int)std::max<int64_t>(1, std::min<int64_t>(n_units, (int64_t)ctx->sm_count));
@@ -750,4 +744,108 @@ static void launch_v5(rrtqx_ctx *ctx, const GridView &g, const double *dq, const
     range_v5_kernel<D, NW, CAP, TAB, true><<<blocks, NW * 32, smem, ctx->stream>>>(g, P, dq, dqs, qorder, nq, r, T, dr, dT, counts,
                                                                              offsets, idx, dist, cap, cursor, write_lists);
   post_launch(ctx);
+}
+
+__global__ void thresh_kernel(const double *__restrict__ ranges, int64_t n, double *__restrict__ Tq) {
+  int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) Tq[i] = sqrt_thresh_lt(ranges[i]);
+}
+
+template <int D>
+static void range_query_fused(rrtqx_tree *t, const double *dq, const double *dr, int64_t nq, double r, uint32_t flags,
+                              rrtqx_range_result *res) {
+  rrtqx_ctx *ctx = t->ctx;
+  cudaStream_t st = ctx->stream;
+  const bool count_only = flags & RRTQX_RANGE_COUNT_ONLY;
+  const bool want_dist = flags & RRTQX_RANGE_WANT_DIST;
+  res->cursor.ensure(4, st);
+  {
+    PhaseScope p2(ctx, "range_sort");
+    sort_queries<D>(t, res, dq, nq);
+  }
+  // wrap-around tree (one wrap dimension, r <= period / 2, checked by the caller): expand into (real, ghost) pairs
+  const bool ghost = t->wrap.num_wraps == 1;
+  const double *kq = dq, *kqs = res->qbins > 0 ? res->qsorted.p : nullptr;
+  const int32_t *korder = res->qorder.p;
+  int32_t *kcounts = res->counts.p;
+  int64_t *koffsets = res->offsets.p;
+  int64_t knq = nq;
+  if (ghost) {
+    res->vq.ensure((size_t)nq * 2 * D, st);
+    res->vorder.ensure((size_t)nq * 2, st);
+    res->vcounts.ensure((size_t)nq * 2 + 1, st);
+    res->voffsets.ensure((size_t)nq * 2 + 1, st);
+    ghost_expand_kernel<D><<<div_up(nq, 256), 256, 0, st>>>(t->wrap, dq, kqs, res->qorder.p, nq, r, res->vq.p, res->vorder.p);
+    post_launch(ctx);
+    kq = nullptr; kqs = res->vq.p; korder = res->vorder.p; kcounts = res->vcounts.p; koffsets = res->voffsets.p; knq = 2 * nq;
+  }
+  const double T = host_sqrt_thresh_lt(r);
+  const double *dT = nullptr;
+  if (dr) {
+    res->tq.ensure((size_t)nq, st);
+    thresh_kernel<<<div_up(nq, 256), 256, 0, st>>>(dr, nq, res->tq.p);
+    post_launch(ctx);
+    dT = res->tq.p;
+  }
+  // Output capacity: grow-only buffers sized by the previous results; if the
+  // lists do not fit, the pass still yields exact counts + total and is
+  // repeated once with the exact size (first call / growing workloads only).
+  size_t cap = count_only ? 0 : res->idx.cap;
+  if (!count_only && want_dist) cap = std::min(cap, res->dist.cap);
+  if (!count_only && cap == 0) {
+    cap = (size_t)nq * 64;
+    res->idx.ensure(cap, st, 0, 1.0);
+    if (want_dist) res->dist.ensure(cap, st, 0, 1.0);
+    cap = want_dist ? std::min(res->idx.cap, res->dist.cap) : res->idx.cap;
+  }
+  // Expected neighbours per query (only selects the kernel variant): the uniform-density estimate
+  // n * V_ball(r) / V_grid with a 15 % margin; per-query radii take the large-buffer variant.
+  double k_est = 1e9;
+  if (!dr && r > 0.0 && std::isfinite(r)) {
+    double vol = 1.0;
+    int dims = 0;
+    const int nd[3] = {t->nx, t->ny, t->nz};
+    for (int c = 0; c < 3; ++c)
+      if (nd[c] > 1) { vol *= nd[c] * t->cell[c]; dims++; }
+    const double ball = dims == 3 ? 4.18879 * r * r * r : (dims == 2 ? 3.14159 * r * r : 2.0 * r);
+    k_est = dims ? 1.15 * (double)t->n * ball / vol : (double)t->n;
+  } else if (!dr) {
+    k_est = 0.0;
+  }
+  int variant = k_est <= 576.0 ? 0 : (k_est <= 1280.0 ? 1 : (k_est <= 2048.0 ? 2 : 3));
+  if (ctx->tune.fused_variant >= 0) variant = ctx->tune.fused_variant;
+  unsigned long long total = 0;
+  for (int attempt = 0; attempt < 2; ++attempt) {
+    GridView g = t->view();
+    RQ_CUDA(cudaMemsetAsync(res->cursor.p, 0, 4 * sizeof(unsigned long long), st));
+    {
+      PhaseScope p2(ctx, "range_fill");
+#define RQ_V5(NW_, CAP_, TAB_)                                                                                       \
+  launch_v5<D, NW_, CAP_, TAB_>(ctx, g, kq, kqs, korder, knq, r, T, dr, dT, kcounts, koffsets, res->idx.p, \
+                                want_dist ? res->dist.p : nullptr, (unsigned long long)cap, res->cursor.p, count_only ? 0 : 1, ghost ? 1 : 0)
+      // hit buffers leave 32*V5_U entries of head-room; the octet table must hold a whole pair's region (else the
+      // pair takes the exact routine)
+      if (variant == 0) RQ_V5(24, 704, 256);          // 24 warps/SM (80 registers), 94 KB shared
+      else if (variant == 1) RQ_V5(24, 1408, 512);    // 186 KB
+      else if (variant == 2) RQ_V5(16, 2176, 1024);   // 205 KB
+      else RQ_V5(8, 4224, 2048);                      // 201 KB
+#undef RQ_V5
+    }
+    RQ_CUDA(cudaMemcpyAsync(&total, res->cursor.p, sizeof(total), cudaMemcpyDeviceToHost, st));
+    RQ_CUDA(cudaStreamSynchronize(st));
+    if (count_only || total <= cap) break;
+    RQ_REQUIRE(attempt == 0, "internal: range output did not fit after resizing");
+    cap = (size_t)total + (size_t)(total / 32) + 1024;
+    res->idx.ensure(cap, st, 0, 1.0);
+    if (want_dist) res->dist.ensure(cap, st, 0, 1.0);
+    cap = want_dist ? std::min(res->idx.cap, res->dist.cap) : res->idx.cap;
+  }
+  if (ghost) {
+    ghost_merge_kernel<<<div_up(nq, 256), 256, 0, st>>>(res->vcounts.p, res->voffsets.p, nq, res->counts.p, res->offsets.p);
+    post_launch(ctx);
+  }
+  res->n_queries = nq;
+  res->total = (int64_t)total;
+  res->has_lists = !count_only;
+  res->has_dist = !count_only && want_dist;
 }

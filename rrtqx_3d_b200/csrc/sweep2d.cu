@@ -83,9 +83,7 @@ struct ListedObstacles {  // the obstacles of the call, each with the start-node
   __device__ __forceinline__ bool admit(int k) const { return !filt || sweep2d_candidate<D>(filt[k], pv, v); }
 };
 
-#ifndef SWEEP2D_MINB
-#define SWEEP2D_MINB 6  // as DUBINS_MINB (polygon.cu): latency-bound FP64 chains, 48 warps per SM (16.7 -> 10.5 ms on the C4 graph)
-#endif
+constexpr int SWEEP2D_BLOCKS_PER_SM = 6;  // as DUBINS_CHECK_BLOCKS_PER_SM (polygon.cu): latency-bound FP64 chains, 48 warps per SM (16.7 -> 10.5 ms on the C4 graph)
 constexpr int SWEEP2D_SELECT_MAX_OBS = 8;  // more listed obstacles admit nearly every item: no list
 // Few listed obstacles (the planner's call: ONE): the start-node filter admits a few per cent of the items, so a
 // thread-per-item pass lists them first and the warp-per-item kernels below run over that list only (a device-side
@@ -122,7 +120,7 @@ sweep2d_select_kernel(const double4 *__restrict__ pos, int64_t n_nodes, const in
 // addNewObstacle: item i < n_edges is out-edge i (src[i] -> dst[i]); item n_edges + v is the parent edge of node v.
 // cand == nullptr: one warp per item of the graph; otherwise persistent warps over the listed items.
 template <int D>
-__global__ void __launch_bounds__(256, SWEEP2D_MINB)
+__global__ void __launch_bounds__(256, SWEEP2D_BLOCKS_PER_SM)
 add_sweep_2d_kernel(PolyView P, const double4 *__restrict__ pos, int64_t n_nodes, const int32_t *__restrict__ src,
                     const int32_t *__restrict__ dst, int64_t n_edges, const int32_t *__restrict__ parent,
                     const int64_t *__restrict__ tptr, const double *__restrict__ traj, const int32_t *__restrict__ ids,
@@ -155,7 +153,7 @@ add_sweep_2d_kernel(PolyView P, const double4 *__restrict__ pos, int64_t n_nodes
 
 // removeObstacle: ids[0] = the removed obstacle (still active while tested, :3228 vs :3267), ids[1..] = the others.
 template <int D>
-__global__ void __launch_bounds__(256, SWEEP2D_MINB)
+__global__ void __launch_bounds__(256, SWEEP2D_BLOCKS_PER_SM)
 remove_sweep_2d_kernel(PolyView P, const double4 *__restrict__ pos, const int32_t *__restrict__ src,
                        const int32_t *__restrict__ dst, int64_t n_edges, const uint8_t *__restrict__ edge_dist_inf,
                        const int64_t *__restrict__ tptr, const double *__restrict__ traj, const int32_t *__restrict__ ids,
@@ -317,7 +315,7 @@ void obstacle_add_sweep_2d(rrtqx_edges *E, const rrtqx_polygons *Pg, const int32
       post_launch(ctx);
       cand = R->cand2d.p;
       n_cand = R->cand2d_n.p;
-      blocks = (unsigned)std::min<int64_t>(blocks, (int64_t)ctx->sm_count * SWEEP2D_MINB);
+      blocks = (unsigned)std::min<int64_t>(blocks, (int64_t)ctx->sm_count * SWEEP2D_BLOCKS_PER_SM);
     }
 #define RQ_ADD2D(D_)                                                                                                   \
   add_sweep_2d_kernel<D_><<<blocks, 256, 0, st>>>(Pg->view(), t->pos.p, E->n_nodes, E->src.p, E->dst.p, E->n_edges, par, \
@@ -369,7 +367,7 @@ void obstacle_remove_sweep_2d(rrtqx_edges *E, const rrtqx_polygons *Pg, int32_t 
       post_launch(ctx);
       cand = R->cand2d.p;
       n_cand = R->cand2d_n.p;
-      blocks = (unsigned)std::min<int64_t>(blocks, (int64_t)ctx->sm_count * SWEEP2D_MINB);
+      blocks = (unsigned)std::min<int64_t>(blocks, (int64_t)ctx->sm_count * SWEEP2D_BLOCKS_PER_SM);
     }
 #define RQ_REM2D(D_)                                                                                                  \
   remove_sweep_2d_kernel<D_><<<blocks, 256, 0, st>>>(Pg->view(), t->pos.p, E->src.p, E->dst.p, E->n_edges, dinf,     \

@@ -275,9 +275,6 @@ __global__ void cell_scatter_kernel(const int32_t *__restrict__ cell_id, int64_t
 // whole ROW of cells is then sorted by x: the neighbours of a query in a row are one nearly contiguous run of slots
 // (fewer 128-byte lines per 32 gathered exact records in the range kernel's flush).  No kernel relies on the order
 // inside a cell for its result.
-#ifndef RRTQX_CELL_ORDER_X
-#define RRTQX_CELL_ORDER_X 1
-#endif
 __global__ void cell_sort_kernel(const int32_t *__restrict__ cell_start, int ncell, const double4 *__restrict__ pos,
                                  int32_t *__restrict__ sperm) {
   int c = blockIdx.x * blockDim.x + threadIdx.x;
@@ -286,11 +283,11 @@ __global__ void cell_sort_kernel(const int32_t *__restrict__ cell_start, int nce
   if (b - a > 256) return;  // degenerate pile-up: order left as scattered (result sets unaffected)
   for (int i = a + 1; i < b; ++i) {
     const int v = sperm[i];
-    const double xv = RRTQX_CELL_ORDER_X ? pos[v].x : 0.0;
+    const double xv = pos[v].x;
     int j = i - 1;
     while (j >= a) {
       const int u = sperm[j];
-      const double xu = RRTQX_CELL_ORDER_X ? pos[u].x : 0.0;
+      const double xu = pos[u].x;
       if (!(xu > xv || (xu == xv && u > v))) break;   // NaN x: compares false, keeps its place
       sperm[j + 1] = u;
       --j;
