@@ -10,7 +10,10 @@
 // invariants recomputed from the endpoints) and marks the edge -- every lane busy, high occupancy.  The result
 // is an OR over pairs, so order and duplicates do not matter.  Edges the scheme does not fit -- degenerate ones
 // (no reject possible: the reference collides them with every active obstacle) and edges with more than
-// PQ_KEEP surviving candidates -- are listed as items and decided by pq_slow_kernel with early exit.
+// PQ_KEEP surviving candidates -- are listed as items and decided by pq_slow_kernel with early exit.  Below the
+// measured break-even the same pq_slow_kernel runs over every item instead (whole-range mode, one thread per item),
+// so the thread-per-edge check and the two-stage one share the per-item walk of the binned table.  bin_obstacles
+// bins an obstacle table for both forms and builds the cover lists.
 //
 // Cover lists: edges whose half length is at most G.cov_cap (half a cover cell) do not walk the coarse rows;
 // they read the list of the one cover cell that holds their midpoint.  Obstacle o is on the list of cell c iff
@@ -39,7 +42,7 @@ struct SphCoverBufs {
   DevBuf<uint2> pairs;                  // (item, obstacle) pairs that survived the reject
   DevBuf<unsigned> slow;                // items decided by the slow kernels (list A, then list B)
   DevBuf<unsigned long long> n_pairs;   // [0] pairs, [1] slow list A, [2] slow list B
-  uint64_t build_id = 0;                // renewed by every build_sphere_cover: who built the lists last
+  uint64_t build_id = 0;                // renewed by every cover build (bin_obstacles): who built the lists last
 };
 
 // One warp per binned obstacle: append it to every cover cell it belongs to (fixed-capacity lists, so one pass,
@@ -91,29 +94,43 @@ cover_register_kernel(const double4 *__restrict__ rec2, const double2 *__restric
 
 constexpr int COV_MAX_OBSTACLES = 65536;  // obstacle numbers are packed into 16 bits of the list entries
 
-// After sphere_grid_kernel(..., cover = 1) on the same stream.  n_upper: upper bound of the table size
-// (<= COV_MAX_OBSTACLES, else the caller asks sphere_grid_kernel for cover = 0 and skips this).
-static inline void build_sphere_cover(rrtqx_ctx *ctx, SphCoverBufs &B, const double4 *rec2, const double2 *thr2,
-                                      const float4 *frec2, const int32_t *cstart, SphGrid *dG, int n_upper) {
-  cudaStream_t st = ctx->stream;
-  B.build_id = next_content_stamp();
-  B.cnt.ensure(COV_CELLS + 1, st);
-  B.list_f.ensure((size_t)COV_CELLS * COV_CAPC, st);
-  RQ_CUDA(cudaMemsetAsync(B.cnt.p, 0, (COV_CELLS + 1) * sizeof(int32_t), st));
-  const unsigned blocks = (unsigned)div_up((int64_t)n_upper * 32, (int64_t)256);
-  cover_register_kernel<<<blocks, 256, 0, st>>>(rec2, thr2, frec2, cstart, dG, n_upper, B.cnt.p, B.list_f.p);
-  post_launch(ctx, 1);
-}
-
 inline char g_cover_tag = 0;  // one key for all translation units (C++17 inline variable)
 static inline SphCoverBufs &cover_bufs(rrtqx_ctx *ctx) {  // owned by the context, freed in rrtqx_ctx_destroy
   return ctx->scratch.get<SphCoverBufs>(&g_cover_tag);
 }
 
-// Batches below the threshold keep the thread-per-edge kernels: the cover build and the extra launches cost
+// Bins an obstacle table (rec, thr and the optional payload ext; *n_live entries if n_live is not NULL, else n_upper)
+// into B on the context's stream; cover: also (re)build the context's cover lists (n_upper <= COV_MAX_OBSTACLES).
+static inline BinnedObstacles bin_obstacles(rrtqx_ctx *ctx, BinnedObstacleBufs &B, const double4 *rec, const double2 *thr,
+                                            const double2 *ext, const int32_t *n_live, int n_upper, bool cover) {
+  cudaStream_t st = ctx->stream;
+  B.rec.ensure((size_t)n_upper + 1, st);
+  B.thr.ensure((size_t)n_upper + 1, st);
+  if (ext) B.ext.ensure((size_t)n_upper + 1, st);
+  B.frec.ensure((size_t)n_upper + 1, st);
+  B.cstart.ensure(SG_MAX_CELLS + 4, st);
+  B.grid.ensure(sizeof(SphGrid) + 16, st);
+  SphGrid *dG = (SphGrid *)B.grid.p;
+  sphere_grid_kernel<<<1, 1024, 0, st>>>(rec, thr, ext, n_live, n_upper, B.rec.p, B.thr.p, ext ? B.ext.p : nullptr, B.cstart.p, dG,
+                                         B.frec.p, cover ? 1 : 0);
+  post_launch(ctx);
+  if (cover) {
+    SphCoverBufs &C = cover_bufs(ctx);
+    C.build_id = next_content_stamp();
+    C.cnt.ensure(COV_CELLS + 1, st);
+    C.list_f.ensure((size_t)COV_CELLS * COV_CAPC, st);
+    RQ_CUDA(cudaMemsetAsync(C.cnt.p, 0, (COV_CELLS + 1) * sizeof(int32_t), st));
+    const unsigned blocks = (unsigned)div_up((int64_t)n_upper * 32, (int64_t)256);
+    cover_register_kernel<<<blocks, 256, 0, st>>>(B.rec.p, B.thr.p, B.frec.p, B.cstart.p, dG, n_upper, C.cnt.p, C.list_f.p);
+    post_launch(ctx);
+  }
+  return B.view();
+}
+
+// Batches below the threshold take the thread-per-item kernel (pq_item_launch): the cover build and the extra launches cost
 // ~40 us, the two-stage path saves ~19 ns per 1000 edges in the batch check (break-even ~2e6 edges) and ~44 ns
 // per 1000 items in the add sweep (break-even ~1e6).  The context's tuning (environment read at rrtqx_ctx_create /
-// rrtqx_ctx_reload_tuning) can switch paths: RRTQX_EDGE_NO_QUEUE=1 forces the thread-per-edge kernels,
+// rrtqx_ctx_reload_tuning) can switch paths: RRTQX_EDGE_NO_QUEUE=1 forces the thread-per-item kernel,
 // RRTQX_COVER_MIN_ITEMS=n moves the threshold.
 constexpr int64_t PQ_MIN_ITEMS_BATCH = (int64_t)1 << 21, PQ_MIN_ITEMS_SWEEP = (int64_t)1 << 20;
 static inline int64_t cover_min_items(const rrtqx_ctx *ctx, int64_t dflt) {
@@ -186,7 +203,7 @@ constexpr unsigned PQ_NONE = 0xffffffffu;  // filler pair (skipped by the test k
 //                                                                    the exact end points from the item's own record
 //   float4 frec(int64_t i)                                           (RESIDENT) FP32 record of item i
 //   bool endpoints(int64_t i, double a[3], double b[3], int &v)   false: item has no edge (node without parent)
-//   void clear(int64_t i)                                           before any test of item i
+//   void clear(int64_t i)                                           item i is not hit (two-stage: before any test of it)
 //   bool accept(int o, const double4 &rec, const double a[3], int v)  extra condition on a colliding pair
 //   void mark(int64_t i)                                            some accepted obstacle collides with item i
 //
@@ -342,79 +359,90 @@ pq_test_kernel(Src S, const double4 *__restrict__ rec, const double2 *__restrict
   }
 }
 
-// Slow items, every candidate decided in place, the item ends at the first hit.  WARP = false: one thread per
-// item (list A: short edges with many surviving candidates).  WARP = true: one warp per item, the candidates of
-// a row spread over the lanes (list B: degenerate and long edges, which may meet most of the table).
-template <bool FMA_DOT, bool WARP, class Src>
-__global__ void __launch_bounds__(128)
-pq_slow_kernel(Src S, const double4 *__restrict__ rec, const double2 *__restrict__ thr, const float4 *__restrict__ frec,
-               const int32_t *__restrict__ cstart, const SphGrid *__restrict__ Gp, const unsigned *__restrict__ slow,
-               const unsigned long long *__restrict__ count) {
+// Items decided in place, every candidate of the item's rows, the item ends at its first hit.  ALL = false: the items
+// of a slow list (*count of them), WARP = false: one thread per item (list A: short edges with many surviving
+// candidates), WARP = true: one warp per item, the candidates of a row spread over the lanes (list B: degenerate and
+// long edges, which may meet most of the table).  ALL = true (WARP = false): every item, one thread each, the p-th
+// thread deciding item p (n_all of them) -- the thread-per-edge path of batches below the two-stage break-even; each
+// item is marked or cleared, an item without an edge is skipped and never marked.  A separate instantiation, so that the
+// list loop does not raise its register count.
+template <bool FMA_DOT, bool WARP, class Src, bool ALL = false>
+__global__ void __launch_bounds__(ALL ? 256 : 128)
+pq_slow_kernel(Src S, BinnedObstacles T, const unsigned *__restrict__ slow, const unsigned long long *__restrict__ count,
+               int64_t n_all) {
+  static_assert(!(ALL && WARP), "whole-range mode is one thread per item");
   __shared__ SphGrid G;
-  if (threadIdx.x == 0) G = *Gp;
+  if (threadIdx.x == 0) G = *T.G;
   __syncthreads();
   const int lane = WARP ? (threadIdx.x & 31) : 0, step = WARP ? 32 : 1;
-  const unsigned long long n = *count;
-  const unsigned long long tid = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
-  const unsigned long long nthr = (unsigned long long)gridDim.x * blockDim.x;
-  for (unsigned long long p = WARP ? tid >> 5 : tid; p < n; p += WARP ? nthr >> 5 : nthr) {
-    const int64_t i = (int64_t)slow[p];
-    double a[3], b[3];
-    int v;
-    S.endpoints(i, a, b, v);
+  auto collides = [&](const double a[3], const double b[3], int v) {
     const SegPre pre = seg_prepare(a[0], a[1], a[2], b[0], b[1], b[2]);
     const SegF32 sf = seg_f32(pre, G.cmax);
-    bool hit = false;  // warp-uniform when WARP
-    auto run = [&](int lo, int hi) {
-      for (int o0 = lo; o0 < hi && !hit; o0 += step) {
+    return sg_walk(G, T.cstart, pre, [&](int lo, int hi) {
+      bool h = false;  // warp-uniform when WARP
+      for (int o0 = lo; o0 < hi && !h; o0 += step) {
         const int o = o0 + lane;
-        bool h = false;
-        if (o < hi && !seg_reject_f32(sf, frec[o])) {  // never rejects a degenerate edge (sf.ok false)
-          const double4 r = rec[o];
-          h = seg_sphere_collide_exact<FMA_DOT>(pre, r.x, r.y, r.z, thr[o].y) && S.accept(o, r, a, v);
+        bool ho = false;
+        if (o < hi && !seg_reject_f32(sf, __ldg(&T.frec[o]))) {  // never rejects a degenerate edge (sf.ok false)
+          const double2 cxy = __ldg(reinterpret_cast<const double2 *>(&T.rec[o]));  // (radius unused)
+          const double4 r = make_double4(cxy.x, cxy.y, __ldg(&T.rec[o].z), 0.0);
+          ho = seg_sphere_collide_exact<FMA_DOT>(pre, r.x, r.y, r.z, __ldg(&T.thr[o].y)) && S.accept(o, r, a, v);
         }
-        hit = WARP ? __any_sync(FULL, h) : h;
+        h = WARP ? __any_sync(FULL, ho) : ho;
       }
-    };
-    const int ncell = G.nx * G.ny * G.nz;
-    if (!pre.cullable) {
-      run(0, G.n_total);
-    } else {
-      const double R = (pre.half + G.thr_max) * (1.0 + 1e-9) + 1e-300;
-      const int x0 = sg_cell(pre.mx - R, G.lo[0], G.inv[0], G.nx), x1 = sg_cell(pre.mx + R, G.lo[0], G.inv[0], G.nx);
-      const int y0 = sg_cell(pre.my - R, G.lo[1], G.inv[1], G.ny), y1 = sg_cell(pre.my + R, G.lo[1], G.inv[1], G.ny);
-      const int z0 = sg_cell(pre.mz - R, G.lo[2], G.inv[2], G.nz), z1 = sg_cell(pre.mz + R, G.lo[2], G.inv[2], G.nz);
-      for (int z = z0; z <= z1 && !hit; ++z)
-        for (int y = y0; y <= y1 && !hit; ++y) {
-          const int cb = (z * G.ny + y) * G.nx;
-          run(cstart[cb + x0], cstart[cb + x1 + 1]);
-        }
-      if (!hit) run(cstart[ncell], cstart[ncell + 1]);
+      return h;
+    });
+  };
+  double a[3], b[3];
+  int v;
+  if constexpr (ALL) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_all) return;
+    if (!S.endpoints(i, a, b, v)) return;  // invalid end point index: counted and cleared by the source
+    if constexpr (Src::RESIDENT)
+      if (S.frec(i).w < 0.f) return;     // no edge (node without parent): its exact record is all zeros
+    if (collides(a, b, v)) S.mark(i);
+    else S.clear(i);
+  } else {
+    const unsigned long long n = *count;
+    const unsigned long long tid = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const unsigned long long nthr = (unsigned long long)gridDim.x * blockDim.x;
+    for (unsigned long long p = WARP ? tid >> 5 : tid; p < n; p += WARP ? nthr >> 5 : nthr) {
+      const int64_t i = (int64_t)slow[p];
+      S.endpoints(i, a, b, v);
+      if (collides(a, b, v) && lane == 0) S.mark(i);
     }
-    if (hit && lane == 0) S.mark(i);
   }
 }
 
-// The four kernels on the context's stream.  Requires n_items < 2^32 (32-bit item numbers in the lists).
+// The four kernels of the two-stage form on the context's stream.  Requires n_items < 2^32 (32-bit item numbers in
+// the lists) and the cover lists of T's table, if its header has them switched on.
 template <bool FMA_DOT, class Src>
-static inline void pq_launch(rrtqx_ctx *ctx, SphCoverBufs &B, const Src &S, int64_t n_items, const double4 *rec,
-                             const double2 *thr, const float4 *frec, const int32_t *cstart, const SphGrid *dG) {
+static inline void pq_launch(rrtqx_ctx *ctx, const Src &S, int64_t n_items, const BinnedObstacles &T) {
   cudaStream_t st = ctx->stream;
+  SphCoverBufs &B = cover_bufs(ctx);
   const unsigned long long cap = 2ull * (unsigned long long)n_items + 1024;
   B.pairs.ensure((size_t)cap, st);
   B.slow.ensure(2 * (size_t)n_items + 2, st);
   B.n_pairs.ensure(4, st);
   unsigned *slow_a = B.slow.p, *slow_b = B.slow.p + n_items + 1;
   RQ_CUDA(cudaMemsetAsync(B.n_pairs.p, 0, 4 * sizeof(unsigned long long), st));
-  pq_collect_kernel<Src><<<(unsigned)div_up(n_items, (int64_t)PQ_THREADS), PQ_THREADS, 0, st>>>(S, n_items, frec, cstart, B.cnt.p,
-                                                                                                  B.list_f.p, dG, B.pairs.p, cap, slow_a, slow_b, B.n_pairs.p);
+  pq_collect_kernel<Src><<<(unsigned)div_up(n_items, (int64_t)PQ_THREADS), PQ_THREADS, 0, st>>>(S, n_items, T.frec, T.cstart, B.cnt.p,
+                                                                                                  B.list_f.p, T.G, B.pairs.p, cap, slow_a, slow_b, B.n_pairs.p);
   const unsigned tblocks = (unsigned)std::min<int64_t>(div_up((int64_t)cap, (int64_t)256), (int64_t)ctx->sm_count * 8);
-  pq_test_kernel<FMA_DOT, Src><<<tblocks, 256, 0, st>>>(S, rec, thr, B.pairs.p, cap, B.n_pairs.p);
+  pq_test_kernel<FMA_DOT, Src><<<tblocks, 256, 0, st>>>(S, T.rec, T.thr, B.pairs.p, cap, B.n_pairs.p);
   const unsigned ablocks = (unsigned)std::min<int64_t>(div_up(n_items, (int64_t)128), (int64_t)ctx->sm_count * 4);
-  pq_slow_kernel<FMA_DOT, false, Src><<<ablocks, 128, 0, st>>>(S, rec, thr, frec, cstart, dG, slow_a, B.n_pairs.p + 1);
+  pq_slow_kernel<FMA_DOT, false, Src><<<ablocks, 128, 0, st>>>(S, T, slow_a, B.n_pairs.p + 1, 0);
   const unsigned bblocks = (unsigned)std::min<int64_t>(div_up(n_items, (int64_t)4), (int64_t)ctx->sm_count * 8);
-  pq_slow_kernel<FMA_DOT, true, Src><<<bblocks, 128, 0, st>>>(S, rec, thr, frec, cstart, dG, slow_b, B.n_pairs.p + 2);
+  pq_slow_kernel<FMA_DOT, true, Src><<<bblocks, 128, 0, st>>>(S, T, slow_b, B.n_pairs.p + 2, 0);
   post_launch(ctx, 4);
+}
+
+// Thread-per-item form (batches below the two-stage break-even): pq_slow_kernel over every item.
+template <bool FMA_DOT, class Src>
+static inline void pq_item_launch(rrtqx_ctx *ctx, const Src &S, int64_t n_items, const BinnedObstacles &T) {
+  pq_slow_kernel<FMA_DOT, false, Src, true><<<(unsigned)div_up(n_items, (int64_t)256), 256, 0, ctx->stream>>>(S, T, nullptr, nullptr, n_items);
+  post_launch(ctx);
 }
 
 #endif  // __CUDACC__

@@ -13,14 +13,12 @@ namespace rrtqx {
 struct SphereTable {
   const double4 *rec;   // (cx,cy,cz,R)
   const double2 *thr;   // (thr, thr_le)
-  const int32_t *id;    // original obstacle index
   int n;
 };
 
 __global__ void sphere_table_kernel(const double4 *__restrict__ rec, const uint8_t *__restrict__ active, int n,
                                     int ignore_active, double robot_radius, double4 *__restrict__ out_rec,
-                                    double2 *__restrict__ out_thr, int32_t *__restrict__ out_id,
-                                    int32_t *__restrict__ out_n) {
+                                    double2 *__restrict__ out_thr, int32_t *__restrict__ out_n) {
   __shared__ int warp_cnt[32];
   __shared__ int base_s;
   if (threadIdx.x == 0) base_s = 0;
@@ -40,7 +38,6 @@ __global__ void sphere_table_kernel(const double4 *__restrict__ rec, const uint8
       double thr = __dadd_rn(robot_radius, r.w);  // robotRadius + thisObstacle.radius (DRRT_Q.jl:1790)
       out_rec[o] = r;
       out_thr[o] = make_double2(thr, sqrt_thresh_le(thr));
-      out_id[o] = i;
     }
     __syncthreads();
     if (threadIdx.x == 0) {
@@ -54,14 +51,11 @@ __global__ void sphere_table_kernel(const double4 *__restrict__ rec, const uint8
 }
 
 struct SphereTableBufs {
-  DevBuf<double4> rec, rec2;
-  DevBuf<double2> thr, thr2;
-  DevBuf<float4> frec2;
-  DevBuf<int32_t> id;
+  DevBuf<double4> rec;
+  DevBuf<double2> thr;
   DevBuf<int32_t> n;
-  DevBuf<int32_t> cstart;
   DevBuf<int32_t> bad;         // device counter of out-of-range edge endpoints
-  DevBuf<unsigned char> grid;  // SphGrid header
+  BinnedObstacleBufs binned;   // the table binned for the large-batch kernels
   // what the buffers currently hold: the table of obstacle set `key_version` for (robot radius, ignore flag);
   // grid_level 0: table only, 1: + obstacle grid, 2: + cover lists (build `cover_id` of the context's cover
   // buffers).  An unchanged obstacle set is not re-binned on every call (the planner checks thousands of edge
@@ -84,80 +78,37 @@ SphereTable build_sphere_table(rrtqx_ctx *ctx, const rrtqx_spheres *s, double ro
   size_t n = (size_t)s->n;
   b.rec.ensure(n + 1, st);
   b.thr.ensure(n + 1, st);
-  b.id.ensure(n + 1, st);
   b.n.ensure(4, st);
   const int ignore = (flags & RRTQX_CHECK_IGNORE_ACTIVE) ? 1 : 0;
   uint64_t rho_bits;
   memcpy(&rho_bits, &robot_radius, sizeof(rho_bits));
   if (!(s->version != 0 && b.key_version == s->version && b.key_rho == rho_bits && b.key_ignore == ignore)) {
-    sphere_table_kernel<<<1, 1024, 0, st>>>(s->rec.p, s->active.p, (int)n, ignore, robot_radius, b.rec.p, b.thr.p, b.id.p, b.n.p);
+    sphere_table_kernel<<<1, 1024, 0, st>>>(s->rec.p, s->active.p, (int)n, ignore, robot_radius, b.rec.p, b.thr.p, b.n.p);
     post_launch(ctx);
     b.key_version = s->version; b.key_rho = rho_bits; b.key_ignore = ignore; b.grid_level = 0;
   }
   SphereTable t;
   t.rec = b.rec.p;
   t.thr = b.thr.p;
-  t.id = b.id.p;
   t.n = (int)n;
   *n_dev_out = b.n.p;
   return t;
 }
 
-// One thread per edge against the binned obstacle table.
-template <bool FMA_DOT, bool SRC_TREE>
-__global__ void __launch_bounds__(256)
-edge_check_grid_kernel(const double4 *__restrict__ pos, const int32_t *__restrict__ src, const int32_t *__restrict__ dst,
-                       const double *__restrict__ starts, const double *__restrict__ ends, int64_t n_edges,
-                       const double4 *__restrict__ rec, const double2 *__restrict__ thr, const float4 *__restrict__ frec,
-                       const int32_t *__restrict__ cstart, const SphGrid *__restrict__ Gp, uint8_t *__restrict__ out,
-                       int n_nodes, int32_t *__restrict__ bad) {
-  __shared__ SphGrid G;
-  if (threadIdx.x == 0) G = *Gp;
-  __syncthreads();
-  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (e >= n_edges) return;
-  SegPre pre;
-  if (SRC_TREE) {
-    const int ia = src[e], ib = dst[e];
-    if ((unsigned)ia >= (unsigned)n_nodes || (unsigned)ib >= (unsigned)n_nodes) {  // reported as RRTQX_ERR_INVALID
-      atomicAdd(bad, 1);
-      out[e] = 0;
-      return;
-    }
-    const double4 a = pos[ia], b = pos[ib];
-    pre = seg_prepare(a.x, a.y, a.z, b.x, b.y, b.z);
-  } else {
-    const double *a = starts + 3 * e, *b = ends + 3 * e;
-    pre = seg_prepare(a[0], a[1], a[2], b[0], b[1], b[2]);
+// The table binned for the large-batch kernels, with the cover lists if want_cover; re-binned only when the table or
+// the cover lists changed (SphereTableBufs::grid_level).
+static BinnedObstacles binned_table(rrtqx_ctx *ctx, const SphereTable &tab, const int32_t *n_live, bool want_cover) {
+  SphereTableBufs &b = table_bufs(ctx);
+  const int want_level = want_cover ? 2 : 1;
+  if (!(b.grid_level == want_level && (!want_cover || cover_bufs(ctx).build_id == b.cover_id))) {
+    bin_obstacles(ctx, b.binned, tab.rec, tab.thr, nullptr, n_live, tab.n, want_cover);
+    b.grid_level = want_level;
+    if (want_cover) b.cover_id = cover_bufs(ctx).build_id;
   }
-  const int ncell = G.nx * G.ny * G.nz;
-  const SegF32 sf = seg_f32(pre, G.cmax);
-  bool hit = false;
-  auto run = [&](int a, int b) {
-    for (int o = a; o < b && !hit; ++o) {
-      if (seg_reject_f32(sf, frec[o])) continue;   // FP32 conservative reject: one 16-byte record
-      const double4 r = rec[o];
-      hit = seg_sphere_collide_exact<FMA_DOT>(pre, r.x, r.y, r.z, thr[o].y);
-    }
-  };
-  if (!pre.cullable) {
-    run(0, G.n_total);  // degenerate edge: the reference collides it with every active obstacle
-  } else {
-    const double R = (pre.half + G.thr_max) * (1.0 + 1e-9) + 1e-300;
-    const int x0 = sg_cell(pre.mx - R, G.lo[0], G.inv[0], G.nx), x1 = sg_cell(pre.mx + R, G.lo[0], G.inv[0], G.nx);
-    const int y0 = sg_cell(pre.my - R, G.lo[1], G.inv[1], G.ny), y1 = sg_cell(pre.my + R, G.lo[1], G.inv[1], G.ny);
-    const int z0 = sg_cell(pre.mz - R, G.lo[2], G.inv[2], G.nz), z1 = sg_cell(pre.mz + R, G.lo[2], G.inv[2], G.nz);
-    for (int z = z0; z <= z1 && !hit; ++z)
-      for (int y = y0; y <= y1 && !hit; ++y) {
-        const int base = (z * G.ny + y) * G.nx;
-        run(cstart[base + x0], cstart[base + x1 + 1]);
-      }
-    if (!hit) run(cstart[ncell], cstart[ncell + 1]);  // non-finite obstacles
-  }
-  out[e] = hit ? 1 : 0;
+  return b.binned.view();
 }
 
-// Item source of the two-stage form of the same check (collide_queue.cuh).
+// Item source of the binned-table kernels of the per-call check (collide_queue.cuh).
 template <bool SRC_TREE>
 struct BatchEdgeSrc {
   static constexpr bool RESIDENT = false;   // end points are gathered per call (no prepared item records)
@@ -311,48 +262,16 @@ void edge_check_launch(rrtqx_ctx *ctx, const rrtqx_tree *tree, const rrtqx_spher
     const unsigned blocks = (unsigned)div_up(n_edges, TB);
     const double4 *pos = from_tree ? tree->pos.p : nullptr;
     const bool fma = flags & RRTQX_CHECK_FMA_DOT;
-    if (n_edges >= 4096 && spheres->n >= 16 && !ctx->tune.edge_no_grid) {
+    if (n_edges >= 4096 && spheres->n >= 16) {
       // large batch: bin the obstacles once, then each edge meets only the obstacles around it
-      SphereTableBufs &b = table_bufs(ctx);
-      b.rec2.ensure((size_t)spheres->n + 1, st);
-      b.thr2.ensure((size_t)spheres->n + 1, st);
-      b.frec2.ensure((size_t)spheres->n + 1, st);
-      b.cstart.ensure(SG_MAX_CELLS + 4, st);
-      b.grid.ensure(sizeof(SphGrid) + 16, st);
-      SphGrid *dG = (SphGrid *)b.grid.p;
       const bool use_queue = n_edges >= cover_min_items(ctx, PQ_MIN_ITEMS_BATCH) && n_edges < ((int64_t)1 << 32);
-      const bool want_cover = use_queue && spheres->n <= COV_MAX_OBSTACLES;
-      const int want_level = want_cover ? 2 : 1;
-      const bool cached = b.grid_level == want_level && (!want_cover || cover_bufs(ctx).build_id == b.cover_id);
-      if (!cached) {
-        sphere_grid_kernel<<<1, 1024, 0, st>>>(tab.rec, tab.thr, nullptr, n_live, 0, b.rec2.p, b.thr2.p, nullptr, b.cstart.p, dG, b.frec2.p, want_cover ? 1 : 0);
-        post_launch(ctx);
-        b.grid_level = want_level;
-      }
-      if (use_queue) {
-        SphCoverBufs &cv = cover_bufs(ctx);
-        if (want_cover && !cached) {
-          build_sphere_cover(ctx, cv, b.rec2.p, b.thr2.p, b.frec2.p, b.cstart.p, dG, (int)spheres->n);
-          b.cover_id = cv.build_id;
-        }
-        if (from_tree) {
-          BatchEdgeSrc<true> S{pos, dsrc, ddst, nullptr, nullptr, dout, n_nodes, dbad};
-          if (fma) pq_launch<true>(ctx, cv, S, n_edges, b.rec2.p, b.thr2.p, b.frec2.p, b.cstart.p, dG);
-          else     pq_launch<false>(ctx, cv, S, n_edges, b.rec2.p, b.thr2.p, b.frec2.p, b.cstart.p, dG);
-        } else {
-          BatchEdgeSrc<false> S{nullptr, nullptr, nullptr, dstarts, dends, dout, 0, dbad};
-          if (fma) pq_launch<true>(ctx, cv, S, n_edges, b.rec2.p, b.thr2.p, b.frec2.p, b.cstart.p, dG);
-          else     pq_launch<false>(ctx, cv, S, n_edges, b.rec2.p, b.thr2.p, b.frec2.p, b.cstart.p, dG);
-        }
-      } else
-      if (from_tree) {
-        if (fma) edge_check_grid_kernel<true, true><<<blocks, TB, 0, st>>>(pos, dsrc, ddst, nullptr, nullptr, n_edges, b.rec2.p, b.thr2.p, b.frec2.p, b.cstart.p, dG, dout, n_nodes, dbad);
-        else     edge_check_grid_kernel<false, true><<<blocks, TB, 0, st>>>(pos, dsrc, ddst, nullptr, nullptr, n_edges, b.rec2.p, b.thr2.p, b.frec2.p, b.cstart.p, dG, dout, n_nodes, dbad);
-      } else {
-        if (fma) edge_check_grid_kernel<true, false><<<blocks, TB, 0, st>>>(pos, nullptr, nullptr, dstarts, dends, n_edges, b.rec2.p, b.thr2.p, b.frec2.p, b.cstart.p, dG, dout, n_nodes, dbad);
-        else     edge_check_grid_kernel<false, false><<<blocks, TB, 0, st>>>(pos, nullptr, nullptr, dstarts, dends, n_edges, b.rec2.p, b.thr2.p, b.frec2.p, b.cstart.p, dG, dout, n_nodes, dbad);
-      }
-      post_launch(ctx, use_queue ? 0 : 1);  // pq_launch counts its own kernels
+      const BinnedObstacles T = binned_table(ctx, tab, n_live, use_queue && spheres->n <= COV_MAX_OBSTACLES);
+      auto run = [&](const auto &S) {
+        if (use_queue) { if (fma) pq_launch<true>(ctx, S, n_edges, T); else pq_launch<false>(ctx, S, n_edges, T); }
+        else           { if (fma) pq_item_launch<true>(ctx, S, n_edges, T); else pq_item_launch<false>(ctx, S, n_edges, T); }
+      };
+      if (from_tree) run(BatchEdgeSrc<true>{pos, dsrc, ddst, nullptr, nullptr, dout, n_nodes, dbad});
+      else           run(BatchEdgeSrc<false>{nullptr, nullptr, nullptr, dstarts, dends, dout, 0, dbad});
     } else if (from_tree) {
       if (fma) edge_check_kernel<true, true><<<blocks, TB, 0, st>>>(pos, dsrc, ddst, nullptr, nullptr, n_edges, tab, n_live, dout, n_nodes, dbad);
       else     edge_check_kernel<false, true><<<blocks, TB, 0, st>>>(pos, dsrc, ddst, nullptr, nullptr, n_edges, tab, n_live, dout, n_nodes, dbad);
@@ -398,16 +317,6 @@ void edges_check(rrtqx_edges *E, const rrtqx_spheres *spheres, double robot_radi
     PhaseScope ph(ctx, "edges_check");
     const int32_t *n_live = nullptr;
     SphereTable tab = build_sphere_table(ctx, spheres, robot_radius, flags, &n_live);
-    SphereTableBufs &b = table_bufs(ctx);
-    b.rec2.ensure((size_t)spheres->n + 1, st);
-    b.thr2.ensure((size_t)spheres->n + 1, st);
-    b.frec2.ensure((size_t)spheres->n + 1, st);
-    b.cstart.ensure(SG_MAX_CELLS + 4, st);
-    b.grid.ensure(sizeof(SphGrid) + 16, st);
-    SphGrid *dG = (SphGrid *)b.grid.p;
-    const bool want_cover = spheres->n <= COV_MAX_OBSTACLES;
-    const int want_level = want_cover ? 2 : 1;
-    bool grid_done = false;
     if (E->igrid.valid && !ctx->tune.no_item_grid) {
       // obstacle-centric: only the cells of the item grid an active obstacle can reach are read
       RQ_CUDA(cudaMemsetAsync(dout, 0, (size_t)n, st));
@@ -426,25 +335,13 @@ void edges_check(rrtqx_edges *E, const rrtqx_spheres *spheres, double robot_radi
       RQ_CUDA(cudaMemcpyAsync(&M.h->aux[0], ovf_dev, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
       if (!out_dev) from_device(ctx, collide_out, dout, (size_t)n);
       RQ_CUDA(cudaStreamSynchronize(st));
-      grid_done = *(volatile int32_t *)&M.h->aux[0] == 0;
-      if (grid_done) return;   // the PhaseScope destructor records the end event
+      if (*(volatile int32_t *)&M.h->aux[0] == 0) return;   // the PhaseScope destructor records the end event
     }
-    SphCoverBufs &cv = cover_bufs(ctx);
-    const bool cached = b.grid_level == want_level && (!want_cover || cv.build_id == b.cover_id);
-    if (!grid_done && !cached) {
-      sphere_grid_kernel<<<1, 1024, 0, st>>>(tab.rec, tab.thr, nullptr, n_live, 0, b.rec2.p, b.thr2.p, nullptr, b.cstart.p, dG, b.frec2.p, want_cover ? 1 : 0);
-      post_launch(ctx);
-      b.grid_level = want_level;
-      if (want_cover) {
-        build_sphere_cover(ctx, cv, b.rec2.p, b.thr2.p, b.frec2.p, b.cstart.p, dG, (int)spheres->n);
-        b.cover_id = cv.build_id;
-      }
-    }
-    ResidentEdgeSrc S{ItemRecords{E->item_frec.p, E->item_exact.p}, dout};
-    if (grid_done) {
-    } else
-    if (flags & RRTQX_CHECK_FMA_DOT) pq_launch<true>(ctx, cv, S, n, b.rec2.p, b.thr2.p, b.frec2.p, b.cstart.p, dG);
-    else                             pq_launch<false>(ctx, cv, S, n, b.rec2.p, b.thr2.p, b.frec2.p, b.cstart.p, dG);
+    // no item grid, or it overflowed: the edge-centric two-stage kernels
+    const BinnedObstacles T = binned_table(ctx, tab, n_live, spheres->n <= COV_MAX_OBSTACLES);
+    const ResidentEdgeSrc S{ItemRecords{E->item_frec.p, E->item_exact.p}, dout};
+    if (flags & RRTQX_CHECK_FMA_DOT) pq_launch<true>(ctx, S, n, T);
+    else                             pq_launch<false>(ctx, S, n, T);
   }
   if (!out_dev) from_device(ctx, collide_out, dout, (size_t)n);
   RQ_CUDA(cudaStreamSynchronize(st));

@@ -109,7 +109,7 @@ inline bool is_device_ptr(const void *p) {
 // iteration.  None of the switches selects a CPU path.
 namespace rrtqx {
 struct Tuning {
-  bool edge_no_grid = false, edge_no_queue = false, range_two_pass = false, nearest_warp = false, no_item_grid = false;
+  bool edge_no_queue = false, range_two_pass = false, nearest_warp = false, no_item_grid = false;
   int64_t cover_min_items = -1;  // < 0: the measured break-even defaults
   int fused_variant = -1;        // < 0: chosen from the expected neighbour count
   int qsort_s = 2, qsort_f = 1;  // supercells of 2^3 cells with the 2:1 grid aspect (scripts/tune_v5.sh)
@@ -122,7 +122,6 @@ struct Tuning {
     auto on = [](const char *n) { return getenv(n) != nullptr; };
     auto geti = [](const char *n, long long d) { const char *e = getenv(n); return e ? atoll(e) : d; };
     auto getd = [](const char *n) { const char *e = getenv(n); return e ? atof(e) : 0.0; };
-    edge_no_grid = on("RRTQX_EDGE_NO_GRID");
     edge_no_queue = on("RRTQX_EDGE_NO_QUEUE");
     range_two_pass = on("RRTQX_RANGE_TWO_PASS");
     nearest_warp = on("RRTQX_NEAREST_WARP");

@@ -67,16 +67,13 @@ struct rrtqx_sweep_result {
   int64_t n_edge_hits = 0, n_node_hits = 0, n_candidates = 0, n_pair_tests = 0;
   rrtqx::DevBuf<uint8_t> edge_flag, node_flag;   // byte flags of the call in flight; zero again after sweep_finish
   bool flags_clean = false;                      // flag arrays and statistics are all-zero (left so by sweep_finish)
-  rrtqx::DevBuf<int32_t> edge_scan, node_scan, edge_list, node_list, scan_tmp;
+  rrtqx::DevBuf<int32_t> edge_list, node_list;
   rrtqx::DevBuf<unsigned long long> stats;
   // obstacle table of the sweep
   rrtqx::DevBuf<double4> ob_rec;
   rrtqx::DevBuf<double4> ob_par;  // (thr, thr_le, search_T_lt, search_range)
-  rrtqx::DevBuf<double2> ob_thr, ob_ext, ob_thr2, ob_ext2;  // (thr, thr_le) / (T_lt(searchRange), searchRange)
-  rrtqx::DevBuf<double4> ob_rec2;
-  rrtqx::DevBuf<float4> ob_frec2;  // FP32 reject records of the binned obstacles
-  rrtqx::DevBuf<int32_t> cstart;
-  rrtqx::DevBuf<unsigned char> grid;
+  rrtqx::DevBuf<double2> ob_thr, ob_ext;  // (thr, thr_le) / (T_lt(searchRange), searchRange)
+  rrtqx::BinnedObstacleBufs binned;        // the table binned for the edge-centric sweep
   rrtqx::DevBuf<int32_t> ids_stage, ids_stage2;
   rrtqx::DevBuf<uint8_t> inf_stage;
   rrtqx::DevBuf<unsigned char> filt2d;  // start-node filters of the Otte / Dubins sweeps (sweep2d.cu)

@@ -290,9 +290,7 @@ add_sweep_kernel(const double4 *__restrict__ pos, int n_nodes, const int32_t *__
           const double4 pr = s_par[o];
           const double q[3] = {c.x, c.y, c.z};
           const double s = sqdist<3>(q, p.x, p.y, p.z, 0.0);  // euclid(ob.position, node.position)
-          bool cand = s < pr.z;                                 // < searchRange
-          if (!cand && v == 0) cand = __dsqrt_rn(s) <= pr.w;    // root admitted with <= (kdTree_general.jl:896)
-          if (cand) {
+          if (start_node_in_range(s, pr.z, pr.w, v == 0)) {
             ncand += 1;
             ntests += (unsigned long long)deg;
             if (deg > 0) {
@@ -345,72 +343,10 @@ add_sweep_kernel(const double4 *__restrict__ pos, int n_nodes, const int32_t *__
   if (threadIdx.x < 2) atomicAdd(&stats[threadIdx.x], s_stats[threadIdx.x]);
 }
 
-// addNewObstacle, edge-centric form (no statistics): one thread per out-edge and per parent edge, the
-// sweep's obstacles binned into the obstacle grid.  Blocked <=> some obstacle o collides with the edge
-// AND the edge's START node passes o's start-node filter dist(c_o, v) < searchRange_o (root: <=), the
-// reference's candidate rule (findPointsInConflictWithObstacle).  The filter is evaluated only for the
-// few obstacles that actually collide; for edges shorter than delta it is implied by the collision.
-template <bool FMA_DOT>
-__global__ void __launch_bounds__(256)
-add_sweep_edge_kernel(const double4 *__restrict__ pos, int64_t n_nodes, const int32_t *__restrict__ src,
-                      const int32_t *__restrict__ dst, int64_t n_edges, const int32_t *__restrict__ parent,
-                      const double4 *__restrict__ rec, const double2 *__restrict__ thr, const double2 *__restrict__ ext,
-                      const float4 *__restrict__ frec, const int32_t *__restrict__ cstart, const SphGrid *__restrict__ Gp,
-                      uint8_t *__restrict__ edge_flag, uint8_t *__restrict__ node_flag) {
-  __shared__ SphGrid G;
-  if (threadIdx.x == 0) G = *Gp;
-  __syncthreads();
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n_edges + n_nodes) return;
-  const bool is_parent = i >= n_edges;
-  int v, w;
-  if (is_parent) {
-    v = (int)(i - n_edges);
-    w = parent ? parent[v] : -1;
-    if (w < 0) return;
-  } else {
-    v = src[i];
-    w = dst[i];
-  }
-  const double4 a = pos[v], b = pos[w];
-  const SegPre pre = seg_prepare(a.x, a.y, a.z, b.x, b.y, b.z);
-  const SegF32 sf = seg_f32(pre, G.cmax);
-  bool hit = false;
-  auto run = [&](int lo, int hi) {
-    for (int o = lo; o < hi && !hit; ++o) {
-      if (seg_reject_f32(sf, frec[o])) continue;   // FP32 conservative reject: one 16-byte record
-      const double4 r = rec[o];
-      if (seg_sphere_collide_exact<FMA_DOT>(pre, r.x, r.y, r.z, thr[o].y)) {
-        const double q[3] = {r.x, r.y, r.z};
-        const double s = sqdist<3>(q, a.x, a.y, a.z, 0.0);  // euclid(ob.position, startNode.position)
-        const double2 e = ext[o];
-        hit = (s < e.x) || (v == 0 && __dsqrt_rn(s) <= e.y);
-      }
-    }
-  };
-  const int ncell = G.nx * G.ny * G.nz;
-  if (!pre.cullable) {
-    run(0, G.n_total);
-  } else {
-    const double R = (pre.half + G.thr_max) * (1.0 + 1e-9) + 1e-300;
-    const int x0 = sg_cell(pre.mx - R, G.lo[0], G.inv[0], G.nx), x1 = sg_cell(pre.mx + R, G.lo[0], G.inv[0], G.nx);
-    const int y0 = sg_cell(pre.my - R, G.lo[1], G.inv[1], G.ny), y1 = sg_cell(pre.my + R, G.lo[1], G.inv[1], G.ny);
-    const int z0 = sg_cell(pre.mz - R, G.lo[2], G.inv[2], G.nz), z1 = sg_cell(pre.mz + R, G.lo[2], G.inv[2], G.nz);
-    for (int z = z0; z <= z1 && !hit; ++z)
-      for (int y = y0; y <= y1 && !hit; ++y) {
-        const int base = (z * G.ny + y) * G.nx;
-        run(cstart[base + x0], cstart[base + x1 + 1]);
-      }
-    if (!hit) run(cstart[ncell], cstart[ncell + 1]);
-  }
-  if (hit) {
-    if (is_parent) node_flag[v] = 1; else edge_flag[i] = 1;
-  }
-}
-
-// The same sweep in two-stage form (collide_queue.cuh): items are the out-edges followed by one parent edge
-// per node; a colliding (edge, obstacle) pair counts only if the edge's start node passes the obstacle's
-// start-node filter.
+// addNewObstacle, edge-centric form (no statistics; collide_queue.cuh), the sweep's obstacles binned into the
+// obstacle grid: items are the out-edges followed by one parent edge per node; a colliding (edge, obstacle) pair
+// counts only if the edge's START node passes the obstacle's start-node filter, the reference's candidate rule.  The
+// filter is evaluated only for the few obstacles that actually collide.
 struct SweepEdgeSrc {
   static constexpr bool RESIDENT = true;   // item records built with the edge set (collide_queue.cuh: ItemRecords)
   ItemRecords rec;
@@ -431,7 +367,7 @@ struct SweepEdgeSrc {
     const double q[3] = {r.x, r.y, r.z};
     const double s = sqdist<3>(q, a[0], a[1], a[2], 0.0);  // euclid(ob.position, startNode.position)
     const double2 e = ext[o];
-    return (s < e.x) || (v == 0 && __dsqrt_rn(s) <= e.y);
+    return start_node_in_range(s, e.x, e.y, [&] { return v == 0; });
   }
   __device__ __forceinline__ void mark(int64_t i) const {
     if (i >= n_edges) node_flag[i - n_edges] = 1; else edge_flag[i] = 1;
@@ -450,9 +386,7 @@ struct SweepGridSink {
   __device__ __forceinline__ bool accept(const IgObstacle &o, const double a[3], int it) const {
     const double q[3] = {o.cx, o.cy, o.cz};
     const double s = sqdist<3>(q, a[0], a[1], a[2], 0.0);  // euclid(ob.position, startNode.position)
-    if (s < o.ext_t) return true;
-    const int v = it >= n_edges ? (int)(it - n_edges) : src[it];
-    return v == 0 && __dsqrt_rn(s) <= o.ext_r;
+    return start_node_in_range(s, o.ext_t, o.ext_r, [&] { return (it >= n_edges ? (int)(it - n_edges) : src[it]) == 0; });
   }
   __device__ __forceinline__ void mark(int it) const {
     if (it >= n_edges) node_flag[it - n_edges] = 1; else edge_flag[it] = 1;
@@ -487,9 +421,7 @@ remove_sweep_kernel(const double4 *__restrict__ pos, const int32_t *__restrict__
     const double4 p = pos[v];
     const double q[3] = {c0.x, c0.y, c0.z};
     const double s = sqdist<3>(q, p.x, p.y, p.z, 0.0);
-    bool cand = s < p0.z;
-    if (!cand && v == 0) cand = __dsqrt_rn(s) <= p0.w;
-    if (cand) {
+    if (start_node_in_range(s, p0.z, p0.w, v == 0)) {
       atomicAdd(&s_cnt, 1u);  // (edge, obstacle) pairs that pass the start-node filter
       if (edge_dist_inf[e] && !removed_inactive) {  // DRRT_Q.jl:3319 (QX: obstacle already unused -> false)
         const double4 w = pos[dst[e]];
@@ -725,70 +657,22 @@ void obstacle_add_sweep(rrtqx_edges *E, const rrtqx_spheres *S, const int32_t *o
   if (E->dirty || E->tree->n != E->n_nodes) edges_rebuild(E);  // appended edges / parents / new nodes
   PhaseScope ph(ctx, "add_sweep");
   sweep_prepare_result(E, R);
-  bool no_stats = false;
-  if (n_obs > 0 && E->n_nodes > 0) {
-    R->ob_rec.ensure((size_t)n_obs, st);
-    R->ob_par.ensure((size_t)n_obs, st);
-    R->ob_thr.ensure((size_t)n_obs, st);
-    R->ob_ext.ensure((size_t)n_obs, st);
-    const int TB = 256;
-    sweep_table_kernel<<<div_up(n_obs, TB), TB, 0, st>>>(S->rec.p, dids, (int)n_obs, robot_radius, delta, R->ob_rec.p, R->ob_par.p, R->ob_thr.p, R->ob_ext.p);
-    bool grid_done = false;
-    if (!(flags & RRTQX_SWEEP_STATS) && E->igrid.valid && !ctx->tune.no_item_grid) {
-      // obstacle-centric sweep over the items sorted by midpoint cell: only the cells an obstacle can reach are read
-      const int32_t *par = E->has_parent ? E->parent.p : nullptr;
-      SweepGridSink K{E->n_edges, E->src.p, R->edge_flag.p, R->node_flag.p, delta >= 0.0};
-      const int32_t *ovf_dev;
-      if (flags & RRTQX_CHECK_FMA_DOT)
-        ovf_dev = item_grid_run<true>(ctx, E->igrid, &E->igrid1, R->ob_rec.p, R->ob_thr.p, R->ob_ext.p, nullptr, (int)n_obs, K,
-                                      E->tree->pos.p, E->n_nodes, E->src.p, E->dst.p, E->n_edges, par);
-      else
-        ovf_dev = item_grid_run<false>(ctx, E->igrid, &E->igrid1, R->ob_rec.p, R->ob_thr.p, R->ob_ext.p, nullptr, (int)n_obs, K,
-                                       E->tree->pos.p, E->n_nodes, E->src.p, E->dst.p, E->n_edges, par);
-      // the overflow flag (more work units than the list holds: huge obstacles) is read together with the counts;
-      // on overflow nothing was marked and the edge-centric kernels repeat the sweep (below)
-      int32_t ovf = 0;
-      sweep_finish(ctx, R, ovf_dev, &ovf);
-      grid_done = ovf == 0;
-      no_stats = true;
-      if (grid_done) { R->n_candidates = -1; R->n_pair_tests = -1; return; }
-      sweep_prepare_result(E, R);
-    }
-    if (grid_done) {
-    } else if (!(flags & RRTQX_SWEEP_STATS)) {
-      // edge-centric sweep over the obstacle grid (no candidate / pair statistics)
-      R->ob_rec2.ensure((size_t)n_obs + 1, st);
-      R->ob_thr2.ensure((size_t)n_obs + 1, st);
-      R->ob_ext2.ensure((size_t)n_obs + 1, st);
-      R->cstart.ensure(SG_MAX_CELLS + 4, st);
-      R->grid.ensure(sizeof(SphGrid) + 16, st);
-      SphGrid *dG = (SphGrid *)R->grid.p;
-      R->ob_frec2.ensure((size_t)n_obs + 1, st);
-      const int64_t work = E->n_edges + E->n_nodes;
-      const bool use_queue = work >= cover_min_items(ctx, PQ_MIN_ITEMS_SWEEP) && work < ((int64_t)1 << 32);
-      sphere_grid_kernel<<<1, 1024, 0, st>>>(R->ob_rec.p, R->ob_thr.p, R->ob_ext.p, nullptr, (int)n_obs, R->ob_rec2.p,
-                                             R->ob_thr2.p, R->ob_ext2.p, R->cstart.p, dG, R->ob_frec2.p, (use_queue && n_obs <= COV_MAX_OBSTACLES) ? 1 : 0);
-      const int32_t *par = E->has_parent ? E->parent.p : nullptr;
-      if (use_queue) {
-        SphCoverBufs &cv = cover_bufs(ctx);
-        if (n_obs <= COV_MAX_OBSTACLES) build_sphere_cover(ctx, cv, R->ob_rec2.p, R->ob_thr2.p, R->ob_frec2.p, R->cstart.p, dG, (int)n_obs);
-        SweepEdgeSrc Q{ItemRecords{E->item_frec.p, E->item_exact.p}, E->n_edges, E->src.p, R->ob_ext2.p, R->edge_flag.p, R->node_flag.p};
-        if (flags & RRTQX_CHECK_FMA_DOT) pq_launch<true>(ctx, cv, Q, work, R->ob_rec2.p, R->ob_thr2.p, R->ob_frec2.p, R->cstart.p, dG);
-        else                             pq_launch<false>(ctx, cv, Q, work, R->ob_rec2.p, R->ob_thr2.p, R->ob_frec2.p, R->cstart.p, dG);
-      } else if (flags & RRTQX_CHECK_FMA_DOT)
-        add_sweep_edge_kernel<true><<<div_up(work, TB), TB, 0, st>>>(E->tree->pos.p, E->n_nodes, E->src.p, E->dst.p, E->n_edges, par,
-                                                                     R->ob_rec2.p, R->ob_thr2.p, R->ob_ext2.p, R->ob_frec2.p, R->cstart.p, dG,
-                                                                     R->edge_flag.p, R->node_flag.p);
-      else
-        add_sweep_edge_kernel<false><<<div_up(work, TB), TB, 0, st>>>(E->tree->pos.p, E->n_nodes, E->src.p, E->dst.p, E->n_edges, par,
-                                                                      R->ob_rec2.p, R->ob_thr2.p, R->ob_ext2.p, R->ob_frec2.p, R->cstart.p, dG,
-                                                                      R->edge_flag.p, R->node_flag.p);
-      post_launch(ctx, 3);
-      no_stats = true;
-    } else {
+  if (n_obs == 0 || E->n_nodes == 0) {
+    sweep_finish(ctx, R);
+    return;
+  }
+  R->ob_rec.ensure((size_t)n_obs, st);
+  R->ob_par.ensure((size_t)n_obs, st);
+  R->ob_thr.ensure((size_t)n_obs, st);
+  R->ob_ext.ensure((size_t)n_obs, st);
+  const int TB = 256;
+  sweep_table_kernel<<<div_up(n_obs, TB), TB, 0, st>>>(S->rec.p, dids, (int)n_obs, robot_radius, delta, R->ob_rec.p, R->ob_par.p, R->ob_thr.p, R->ob_ext.p);
+  post_launch(ctx);
+  const bool fma = flags & RRTQX_CHECK_FMA_DOT;
+  const int32_t *par = E->has_parent ? E->parent.p : nullptr;
+  if (flags & RRTQX_SWEEP_STATS) {  // node-centric, the only form with candidate / pair statistics
     const int blocks = std::max(1, std::min(div_up(E->n_nodes * 32, TB), ctx->sm_count * 8));
-    const int32_t *par = E->has_parent ? E->parent.p : nullptr;
-    if (flags & RRTQX_CHECK_FMA_DOT)
+    if (fma)
       add_sweep_kernel<true><<<blocks, TB, 0, st>>>(E->tree->pos.p, (int)E->n_nodes, E->row_ptr.p, E->csr_dst.p, E->csr_eid.p, par,
                                                     E->lmax.p, E->degenerate.p, R->ob_rec.p, R->ob_par.p, (int)n_obs,
                                                     R->edge_flag.p, R->node_flag.p, R->stats.p);
@@ -796,11 +680,38 @@ void obstacle_add_sweep(rrtqx_edges *E, const rrtqx_spheres *S, const int32_t *o
       add_sweep_kernel<false><<<blocks, TB, 0, st>>>(E->tree->pos.p, (int)E->n_nodes, E->row_ptr.p, E->csr_dst.p, E->csr_eid.p, par,
                                                      E->lmax.p, E->degenerate.p, R->ob_rec.p, R->ob_par.p, (int)n_obs,
                                                      R->edge_flag.p, R->node_flag.p, R->stats.p);
-    post_launch(ctx, 2);
-    }
+    post_launch(ctx);
+    sweep_finish(ctx, R);
+    return;
   }
+  if (E->igrid.valid && !ctx->tune.no_item_grid) {
+    // obstacle-centric sweep over the items sorted by midpoint cell: only the cells an obstacle can reach are read
+    SweepGridSink K{E->n_edges, E->src.p, R->edge_flag.p, R->node_flag.p, delta >= 0.0};
+    const int32_t *ovf_dev;
+    if (fma)
+      ovf_dev = item_grid_run<true>(ctx, E->igrid, &E->igrid1, R->ob_rec.p, R->ob_thr.p, R->ob_ext.p, nullptr, (int)n_obs, K,
+                                    E->tree->pos.p, E->n_nodes, E->src.p, E->dst.p, E->n_edges, par);
+    else
+      ovf_dev = item_grid_run<false>(ctx, E->igrid, &E->igrid1, R->ob_rec.p, R->ob_thr.p, R->ob_ext.p, nullptr, (int)n_obs, K,
+                                     E->tree->pos.p, E->n_nodes, E->src.p, E->dst.p, E->n_edges, par);
+    // the overflow flag (more work units than the list holds: huge obstacles) is read together with the counts;
+    // on overflow nothing was marked and the edge-centric kernels repeat the sweep (below)
+    int32_t ovf = 0;
+    sweep_finish(ctx, R, ovf_dev, &ovf);
+    R->n_candidates = R->n_pair_tests = -1;
+    if (ovf == 0) return;
+    sweep_prepare_result(E, R);
+  }
+  // edge-centric sweep over the binned obstacles
+  const int64_t work = E->n_edges + E->n_nodes;
+  const bool use_queue = work >= cover_min_items(ctx, PQ_MIN_ITEMS_SWEEP) && work < ((int64_t)1 << 32);
+  const BinnedObstacles T = bin_obstacles(ctx, R->binned, R->ob_rec.p, R->ob_thr.p, R->ob_ext.p, nullptr, (int)n_obs,
+                                          use_queue && n_obs <= COV_MAX_OBSTACLES);
+  const SweepEdgeSrc Q{ItemRecords{E->item_frec.p, E->item_exact.p}, E->n_edges, E->src.p, T.ext, R->edge_flag.p, R->node_flag.p};
+  if (use_queue) { if (fma) pq_launch<true>(ctx, Q, work, T); else pq_launch<false>(ctx, Q, work, T); }
+  else           { if (fma) pq_item_launch<true>(ctx, Q, work, T); else pq_item_launch<false>(ctx, Q, work, T); }
   sweep_finish(ctx, R);
-  if (no_stats) { R->n_candidates = -1; R->n_pair_tests = -1; }
+  R->n_candidates = R->n_pair_tests = -1;
 }
 
 void obstacle_remove_sweep(rrtqx_edges *E, const rrtqx_spheres *S, int32_t ob_id, const int32_t *other_ids,

@@ -366,8 +366,8 @@ def test_edge_check_cover_lists_short_edges(ctx):
 
 
 def test_two_stage_and_thread_per_edge_paths_agree(ctx):
-    """The same edge batch and add sweep through the library's own choice (thread-per-edge grid kernels at this
-    size; the two-stage kernels take over above ~1e6 items), the thread-per-edge kernels forced
+    """The same edge batch and add sweep through the library's own choice (the thread-per-item kernel over the obstacle grid at
+    this size; the two-stage kernels take over above ~1e6 items), the thread-per-edge kernels forced
     (RRTQX_EDGE_NO_QUEUE=1) and the two-stage kernels forced (RRTQX_COVER_MIN_ITEMS=1): identical flags / id lists, and equal to the oracle."""
     import os
     pts, _, _ = W.c2_workload(12000, 1)
@@ -378,7 +378,7 @@ def test_two_stage_and_thread_per_edge_paths_agree(ctx):
     E = EdgeSet(t)
     E.upload(src, dst, parent)
     ids = np.arange(len(radii), dtype=np.int32)
-    small = slice(0, 6000)                      # 4096 <= n < 16384: thread-per-edge grid kernel by default
+    small = slice(0, 6000)                      # 4096 <= n < 16384: thread-per-item kernel over the obstacle grid by default
     want = _orc_edges(sph, ns, pts, src, dst, W.ROBOT_RADIUS)
     results = {}
     # the add sweep over a resident edge set takes the obstacle-centric item grid by default; RRTQX_NO_ITEM_GRID=1 gives
@@ -418,7 +418,7 @@ def test_bad_edge_endpoints_fail_the_call_host_and_device_arrays(ctx, building2)
     dst = src[::-1].copy()
     good = edge_check_batch(t, S, src, dst, W.ROBOT_RADIUS)
     for bad_value in (-1, 6000, 2 ** 31 - 1):
-        for n_e in (100, 5000):           # tiled kernel / obstacle-grid kernel
+        for n_e in (100, 5000):           # tiled kernel / thread-per-item kernel over the obstacle grid
             s2, d2 = src[:n_e].copy(), dst[:n_e].copy()
             d2[n_e // 2] = bad_value
             with pytest.raises(A.RRTQXError) as ei:
