@@ -304,6 +304,38 @@ RRTQX_API rrtqx_status rrtqx_extend_query(
     double *point_cert, int32_t *n_neighbors, int32_t *nbr_idx,
     double *nbr_dist, uint8_t *fwd_collide, uint8_t *rev_collide);
 
+/* rrtqx_extend_query for n independent planning instances in ONE launch and
+ * one host wait (multirrtqx's agents, rrtqx.jl:331,915, run in lock-step).
+ * Instance i: tree trees[i], obstacle set spheres[i] (the same handle may
+ * serve several instances), sample points[i*d .. i*d+d), radius ranges[i]
+ * (points and ranges: host arrays).  Per-instance outputs at index i;
+ * neighbour arrays have stride `capacity` (instance i's list starts at
+ * i*capacity).  Every per-instance value equals what rrtqx_extend_query
+ * returns for the same arguments.  n_instances == 0 does nothing.  Refused
+ * before anything is launched or written (RRTQX_ERR_INVALID): a NULL handle,
+ * handles of different contexts, trees of different d, the same tree twice,
+ * capacity < 0, device pointers for points / ranges.  A wrap-around tree, an
+ * empty tree or more than 768 active obstacles fail the whole call with the
+ * status of rrtqx_extend_query; the message names the instance.  The
+ * active-obstacle table of each tree is shared with rrtqx_extend_query; the
+ * mapped result buffers belong to the context, so single and multi calls may
+ * be interleaved freely. */
+RRTQX_API rrtqx_status rrtqx_extend_query_multi(
+    rrtqx_tree *const *trees, const rrtqx_spheres *const *spheres,
+    int32_t n_instances, const double *points, const double *ranges,
+    double robot_radius, uint32_t flags, int32_t capacity,
+    int32_t *nearest_idx, double *nearest_dist, uint8_t *point_collides,
+    double *point_cert, int32_t *n_neighbors, int32_t *nbr_idx,
+    double *nbr_dist, uint8_t *fwd_collide, uint8_t *rev_collide);
+/* rrtqx_tree_insert of positions[i*d ..] (host, n x d) into trees[i] for
+ * every i, in ONE asynchronous launch; index_out[i] (NULL allowed) receives
+ * the node's index.  The trees must be distinct, of one context and one d
+ * (refused as in rrtqx_extend_query_multi); n == 0 does nothing. */
+RRTQX_API rrtqx_status rrtqx_tree_insert_multi(rrtqx_tree *const *trees,
+                                               int32_t n,
+                                               const double *positions,
+                                               int32_t *index_out);
+
 /* The DubinsEdge counterpart (config C4: a 4-D tree [x y t theta] whose
  * dimension 3 wraps with period 2 pi = 6.283185307179586; every other layout
  * fails with RRTQX_ERR_UNSUPPORTED) for the new sample `point` (4 doubles,

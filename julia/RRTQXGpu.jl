@@ -44,7 +44,7 @@ export Context, GpuKDTree, GpuObstacles, GpuPolygons, GpuEdges, GpuWorld, attach
        explicitEdgeCheck, explicitEdgeCheckBatch, explicitPointCheck, explicitPointCheck3D,
        explicitNodeCheck, explicitNodeCheck3D,
        findPointsInConflictWithObstacle, addNewObstacle, removeObstacle, syncObstacles!, syncPolygons!, syncEdges!,
-       extendQuery, pinnedVector
+       extendQuery, extendQueryMulti, kdInsertMulti, pinnedVector
 
 const LIB = get(ENV, "RRTQX_B200_LIB", joinpath(@__DIR__, "..", "rrtqx_3d_b200", "librrtqx_b200.so"))
 
@@ -157,6 +157,32 @@ function kdInsert(tree::GpuKDTree{T}, node::T) where {T}
   end
   tree.treeSize += 1
   refreshKdFields!(tree, Int(idx[]), 1)
+  return
+end
+
+# kdInsert(trees[i], nodes[i]) for every i in ONE launch (multirrtqx's agents in lock-step): the trees are distinct
+# and of one context; each keeps nodes / index / root / treeSize and the kd fields exactly as kdInsert does
+function kdInsertMulti(trees::Vector, nodes::Vector)
+  keep = [i for i = 1:length(trees) if !nodes[i].kdInTree]
+  isempty(keep) && return
+  ts = trees[keep]; ns = nodes[keep]
+  handles = Ptr{Cvoid}[t.h for t in ts]
+  pos = Matrix{Float64}(undef, ts[1].d, length(ns))      # column-major d x n == row-major n x d for C
+  for (k, n) in enumerate(ns); pos[:, k] = vec(n.position); end
+  idx = Vector{Int32}(undef, length(ns))
+  GC.@preserve handles pos idx check(ts[1].ctx, ccall((:rrtqx_tree_insert_multi, LIB), Int32,
+      (Ptr{Ptr{Cvoid}}, Int32, Ptr{Float64}, Ptr{Int32}), handles, length(ns), pos, idx))
+  for k = 1:length(ns)
+    t = ts[k]; n = ns[k]
+    n.kdInTree = true
+    push!(t.nodes, n)
+    t.index[n] = idx[k]
+    if t.treeSize == 0
+      t.root = n
+    end
+    t.treeSize += 1
+    refreshKdFields!(t, Int(idx[k]), 1)
+  end
   return
 end
 
@@ -671,6 +697,50 @@ function extendQuery(S, tree::GpuKDTree, point::Array{Float64}, range::Float64; 
   warm = S.inWarmupTime                     # obstacles are ignored during warm-up (DRRT_Q.jl:1805-1807, 1523-1525)
   return (tree.nodes[nearestIdx[] + 1], nearestDist[], warm ? false : collides[] != 0, warm ? Inf : cert[],
           view(idx, 1:k), view(dist, 1:k), warm ? falses(k) : view(fwd, 1:k) .!= 0, warm ? falses(k) : view(rev, 1:k) .!= 0)
+end
+
+# extendQuery for many planners in lock-step (multirrtqx's agents, rrtqx.jl:331,915): agent i is (Ss[i], trees[i],
+# points[i], ranges[i]), each with its own CSpace and tree.  One launch and one host wait serve the whole round; each
+# agent gets the tuple extendQuery returns, warm-up handling included.  The views stay valid until the next
+# extendQueryMulti on the same first CSpace.  An agent whose ball holds more than `capacity` nodes is repeated alone
+# with extendQuery (rare).  The agents share one robot radius (the C call takes one).
+function extendQueryMulti(Ss::Vector, trees::Vector, points::Vector, ranges::Vector{Float64}; capacity::Int = 8192)
+  n = length(trees)
+  n == 0 && return Any[]
+  rho = Ss[1].robotRadius
+  all(S -> S.robotRadius == rho, Ss) || error("extendQueryMulti: the agents' robot radii differ")
+  sets = Ptr{Cvoid}[syncObstacles!(world(S).spheres, S).h for S in Ss]
+  handles = Ptr{Cvoid}[t.h for t in trees]
+  P = Matrix{Float64}(undef, trees[1].d, n)               # column-major d x n == row-major n x d for C
+  for i = 1:n; P[:, i] = vec(points[i]); end
+  W = world(Ss[1])
+  if !haskey(W.pinned, :mIdx) || length(W.pinned[:mIdx]) < n * capacity
+    W.pinned[:mIdx] = pinnedVector(W.ctx, Int32, n * capacity); W.pinned[:mDist] = pinnedVector(W.ctx, Float64, n * capacity)
+    W.pinned[:mFwd] = pinnedVector(W.ctx, UInt8, n * capacity); W.pinned[:mRev] = pinnedVector(W.ctx, UInt8, n * capacity)
+  end
+  idx = W.pinned[:mIdx]::Vector{Int32}; dist = W.pinned[:mDist]::Vector{Float64}
+  fwd = W.pinned[:mFwd]::Vector{UInt8}; rev = W.pinned[:mRev]::Vector{UInt8}
+  nearestIdx = Vector{Int32}(undef, n); nearestDist = Vector{Float64}(undef, n)
+  collides = Vector{UInt8}(undef, n); cert = Vector{Float64}(undef, n); cnt = Vector{Int32}(undef, n)
+  GC.@preserve sets handles P ranges idx dist fwd rev nearestIdx nearestDist collides cert cnt check(trees[1].ctx,
+      ccall((:rrtqx_extend_query_multi, LIB), Int32,
+            (Ptr{Ptr{Cvoid}}, Ptr{Ptr{Cvoid}}, Int32, Ptr{Float64}, Ptr{Float64}, Float64, UInt32, Int32, Ptr{Int32},
+             Ptr{Float64}, Ptr{UInt8}, Ptr{Float64}, Ptr{Int32}, Ptr{Int32}, Ptr{Float64}, Ptr{UInt8}, Ptr{UInt8}),
+            handles, sets, n, P, ranges, rho, CHECK_QUICK_PASS, Int32(capacity), nearestIdx, nearestDist, collides,
+            cert, cnt, idx, dist, fwd, rev))
+  out = Vector{Any}(undef, n)
+  for i = 1:n
+    S = Ss[i]; c = Int(cnt[i])
+    if c > capacity                          # overflow: this agent alone, with room for its whole ball
+      out[i] = extendQuery(S, trees[i], points[i], ranges[i]; capacity = 2 * c)
+      continue
+    end
+    r = (i - 1) * capacity + 1 : (i - 1) * capacity + c
+    warm = S.inWarmupTime                    # obstacles are ignored during warm-up (DRRT_Q.jl:1805-1807, 1523-1525)
+    out[i] = (trees[i].nodes[nearestIdx[i] + 1], nearestDist[i], warm ? false : collides[i] != 0, warm ? Inf : cert[i],
+              view(idx, r), view(dist, r), warm ? falses(c) : view(fwd, r) .!= 0, warm ? falses(c) : view(rev, r) .!= 0)
+  end
+  return out
 end
 
 # ------------------------------------------------------------------ Dubins edges (2-D polygon world)

@@ -478,6 +478,48 @@ rrtqx_status rrtqx_extend_query(rrtqx_tree *tree, const rrtqx_spheres *spheres, 
   });
 }
 
+namespace {
+// The context of a multi-instance call: that of its first non-NULL tree (the call refuses NULL handles itself, with
+// the instance named in the context's message); NULL when there is none.
+rrtqx_ctx *first_ctx(rrtqx_tree *const *trees, int32_t n) {
+  for (int32_t i = 0; trees && i < n; ++i)
+    if (trees[i]) return trees[i]->ctx;
+  return nullptr;
+}
+}  // namespace
+
+rrtqx_status rrtqx_extend_query_multi(rrtqx_tree *const *trees, const rrtqx_spheres *const *spheres, int32_t n_instances,
+                                      const double *points, const double *ranges, double robot_radius, uint32_t flags,
+                                      int32_t capacity, int32_t *nearest_idx, double *nearest_dist,
+                                      uint8_t *point_collides, double *point_cert, int32_t *n_neighbors,
+                                      int32_t *nbr_idx, double *nbr_dist, uint8_t *fwd_collide, uint8_t *rev_collide) {
+  if (n_instances == 0) return RRTQX_OK;
+  rrtqx_ctx *ctx = first_ctx(trees, n_instances);
+  if (!ctx) {
+    g_last_error = "no tree handle";
+    return RRTQX_ERR_INVALID;
+  }
+  return guarded(ctx, [&] {
+    bind_device(ctx);
+    extend_query_multi(trees, spheres, n_instances, points, ranges, robot_radius, flags, capacity, nearest_idx,
+                       nearest_dist, point_collides, point_cert, n_neighbors, nbr_idx, nbr_dist, fwd_collide,
+                       rev_collide);
+  });
+}
+
+rrtqx_status rrtqx_tree_insert_multi(rrtqx_tree *const *trees, int32_t n, const double *positions, int32_t *index_out) {
+  if (n == 0) return RRTQX_OK;
+  rrtqx_ctx *ctx = first_ctx(trees, n);
+  if (!ctx) {
+    g_last_error = "no tree handle";
+    return RRTQX_ERR_INVALID;
+  }
+  return guarded(ctx, [&] {
+    bind_device(ctx);
+    tree_insert_multi(trees, n, positions, index_out);
+  });
+}
+
 rrtqx_status rrtqx_extend_query_dubins(rrtqx_tree *tree, const rrtqx_polygons *polygons, double *point, double delta,
                                        double range, double robot_radius, double min_turn_radius, uint32_t flags,
                                        int32_t capacity, int32_t *nearest_idx, double *nearest_dist,

@@ -225,6 +225,21 @@ inline void post_launch(rrtqx_ctx *ctx, int n = 1) {
     throw Error(RRTQX_ERR_CUDA, std::string("kernel launch failed: ") + cudaGetErrorString(e));
 }
 
+// Spin until the device has published call number `want` into the mapped pinned *word; a stream query every few
+// thousand spins turns a faulted launch into an error instead of a hang.
+inline void wait_published(const unsigned long long *word, unsigned long long want, cudaStream_t st) {
+  const volatile unsigned long long *seqp = word;
+  for (unsigned spins = 0; *seqp != want; ++spins) {
+    if ((spins & 0xfff) == 0xfff) {
+      cudaError_t qe = cudaStreamQuery(st);
+      if (qe == cudaSuccess) break;
+      if (qe != cudaErrorNotReady) RQ_CUDA(qe);
+    }
+  }
+  std::atomic_thread_fence(std::memory_order_acquire);
+  if (*seqp != want) RQ_CUDA(cudaStreamSynchronize(st));
+}
+
 // Small results of a call (counts, flags) travel through one block of mapped pinned memory per context: the call's
 // last kernel stores them and then a call number, and the host spins on that word -- no copy operations, no stream
 // synchronisation (each of those costs 10-15 us on a call whose kernels take 40).  D2H copies of single words that
@@ -240,20 +255,7 @@ struct HostMail {
     RQ_CUDA(cudaHostGetDevicePointer((void **)&d, h, 0));
     memset(h, 0, sizeof(Block));
   }
-  // spin until the device has published call `want`; a stream query every few thousand spins turns a faulted launch
-  // into an error instead of a hang
-  void wait(cudaStream_t st, unsigned long long want) {
-    volatile unsigned long long *seqp = &h->seq;
-    for (unsigned spins = 0; *seqp != want; ++spins) {
-      if ((spins & 0xfff) == 0xfff) {
-        cudaError_t qe = cudaStreamQuery(st);
-        if (qe == cudaSuccess) break;
-        if (qe != cudaErrorNotReady) RQ_CUDA(qe);
-      }
-    }
-    std::atomic_thread_fence(std::memory_order_acquire);
-    if (*seqp != want) RQ_CUDA(cudaStreamSynchronize(st));
-  }
+  void wait(cudaStream_t st, unsigned long long want) { wait_published(&h->seq, want, st); }
 };
 inline HostMail &host_mail(rrtqx_ctx *ctx) {
   static const char tag = 0;

@@ -76,16 +76,21 @@ struct ExtendParams {
   unsigned long long seq;  // call number, echoed into the header when every result is visible to the host
 };
 
+// The whole query of one instance, run by one block of EXT_WARPS warps: obstacle table in shared memory, range search,
+// nearest, node check, edge checks; the header and the entries are stored, but no completion word is published.
 template <int D, bool FMA_DOT>
-__global__ void __launch_bounds__(EXT_WARPS * 32, 1)
-extend_query_kernel(GridView g, const ExtendParams prm, const double4 *__restrict__ sph_rec,
-                    const uint8_t *__restrict__ sph_active, int n_sph, ExtendHeader *__restrict__ hdr,
-                    ExtendEntry *__restrict__ ent /* device scratch */, ExtendEntry *__restrict__ ent_out /* mapped host */) {
+__device__ __forceinline__ void extend_block(const GridView &g, const ExtendParams &prm, const double4 *__restrict__ sph_rec,
+                                             const uint8_t *__restrict__ sph_active, int n_sph, ExtendHeader *__restrict__ hdr,
+                                             ExtendEntry *__restrict__ ent /* device scratch */,
+                                             ExtendEntry *__restrict__ ent_out /* mapped host */) {
   __shared__ double4 s_rec[EXT_MAX_SPHERES];
   __shared__ double2 s_thr[EXT_MAX_SPHERES];
   __shared__ int s_nsph, s_count;
   __shared__ double s_best_s[EXT_WARPS];
   __shared__ int s_best_n[EXT_WARPS];
+  // both kernels run blocks of EXT_WARPS warps (their launch bounds); an inlined device function does not inherit
+  // that range of threadIdx.x, and the index arithmetic is tighter with it
+  __builtin_assume(threadIdx.x < EXT_WARPS * 32);
   const int lane = lane_id(), warp = threadIdx.x >> 5, tid = threadIdx.x;
   const unsigned lt = lanemask_lt();
   if (tid == 0) { s_nsph = 0; s_count = 0; }
@@ -266,12 +271,58 @@ extend_query_kernel(GridView g, const ExtendParams prm, const double4 *__restric
       ent_out[k] = e;
     }
   }
+}
+
+template <int D, bool FMA_DOT>
+__global__ void __launch_bounds__(EXT_WARPS * 32, 1)
+extend_query_kernel(GridView g, const ExtendParams prm, const double4 *__restrict__ sph_rec,
+                    const uint8_t *__restrict__ sph_active, int n_sph, ExtendHeader *__restrict__ hdr,
+                    ExtendEntry *__restrict__ ent /* device scratch */, ExtendEntry *__restrict__ ent_out /* mapped host */) {
+  extend_block<D, FMA_DOT>(g, prm, sph_rec, sph_active, n_sph, hdr, ent, ent_out);
   // completion: every thread's stores to the mapped host buffers are fenced to system scope, then one thread
   // publishes the call number; the host spins on that word instead of paying a stream synchronisation
   __threadfence_system();
   __syncthreads();
-  if (tid == 0) {
+  if (threadIdx.x == 0) {
     *(volatile unsigned long long *)&hdr->seq = prm.seq;
+    __threadfence_system();
+  }
+}
+
+// One instance of rrtqx_extend_query_multi: its tree, its compacted active-obstacle table, its query and its slices of
+// the context's result buffers.
+struct ExtendInstance {
+  GridView g;
+  ExtendParams prm;
+  const double4 *table;   // active obstacles (the tree's ExtendState cache)
+  int32_t n_table;
+  ExtendHeader *hdr;      // mapped host
+  ExtendEntry *ent;       // device scratch, capacity entries
+  ExtendEntry *ent_out;   // mapped host, capacity entries
+};
+
+// n independent extend queries in one launch, one block per instance.  The descriptor is staged in shared memory, so
+// the query reads it like the single kernel reads its parameters.  The last block to finish (device ticket, reset
+// for the next call) publishes the call number once every block's results are visible to the host.
+template <int D, bool FMA_DOT>
+__global__ void __launch_bounds__(EXT_WARPS * 32, 1)
+extend_query_multi_kernel(const ExtendInstance *__restrict__ inst, unsigned *__restrict__ ticket,
+                          unsigned long long *done, unsigned long long seq) {
+  __shared__ ExtendInstance s_inst;
+  static_assert(sizeof(ExtendInstance) % sizeof(unsigned long long) == 0, "descriptor copied as 8-byte words");
+  constexpr int WORDS = sizeof(ExtendInstance) / sizeof(unsigned long long);
+  if (threadIdx.x < WORDS)
+    reinterpret_cast<unsigned long long *>(&s_inst)[threadIdx.x] =
+        reinterpret_cast<const unsigned long long *>(inst + blockIdx.x)[threadIdx.x];
+  __syncthreads();
+  extend_block<D, FMA_DOT>(s_inst.g, s_inst.prm, s_inst.table, nullptr, s_inst.n_table, s_inst.hdr, s_inst.ent,
+                           s_inst.ent_out);
+  __threadfence_system();
+  __syncthreads();
+  if (threadIdx.x == 0 && atomicAdd(ticket, 1u) == gridDim.x - 1) {
+    *ticket = 0;
+    __threadfence_system();
+    *(volatile unsigned long long *)done = seq;
     __threadfence_system();
   }
 }
@@ -380,20 +431,7 @@ void extend_query(rrtqx_tree *t, const rrtqx_spheres *S, const double *point, do
 #undef RQ_EXT
     post_launch(ctx);
   }
-  // wait for the kernel's completion word (mapped pinned memory); a stream query every few thousand spins
-  // turns a faulted launch into an error instead of a hang
-  {
-    volatile unsigned long long *seqp = &es->h_hdr->seq;
-    for (unsigned spins = 0; *seqp != prm.seq; ++spins) {
-      if ((spins & 0xfff) == 0xfff) {
-        cudaError_t qe = cudaStreamQuery(st);
-        if (qe == cudaSuccess) break;  // kernel finished: the word is visible on the next read
-        if (qe != cudaErrorNotReady) RQ_CUDA(qe);
-      }
-    }
-    std::atomic_thread_fence(std::memory_order_acquire);
-    if (*seqp != prm.seq) RQ_CUDA(cudaStreamSynchronize(st));
-  }
+  wait_published(&es->h_hdr->seq, prm.seq, st);   // the kernel's completion word (mapped pinned memory)
   const ExtendHeader h = *es->h_hdr;
   if (nearest_idx) *nearest_idx = h.nearest_idx;
   if (nearest_dist) *nearest_dist = h.nearest_dist;
@@ -407,5 +445,182 @@ void extend_query(rrtqx_tree *t, const rrtqx_spheres *S, const double *point, do
     if (nbr_dist) nbr_dist[k] = e.dist;
     if (fwd_collide) fwd_collide[k] = e.fwd;
     if (rev_collide) rev_collide[k] = e.rev;
+  }
+}
+
+template <typename T>
+static void mapped_alloc(T *&h, T *&d, size_t n) {
+  RQ_CUDA(cudaHostAlloc((void **)&h, sizeof(T) * n, cudaHostAllocMapped));
+  RQ_CUDA(cudaHostGetDevicePointer((void **)&d, h, 0));
+}
+
+struct ExtendMultiState {   // per context: descriptors and mapped result buffers of rrtqx_extend_query_multi
+  ExtendInstance *h_inst = nullptr;                    // pinned staging of the descriptors
+  DevBuf<ExtendInstance> inst;
+  ExtendHeader *h_hdr = nullptr, *d_hdr = nullptr;     // mapped pinned, one per instance
+  ExtendEntry *h_ent = nullptr, *d_ent_out = nullptr;  // mapped pinned, `capacity` per instance
+  DevBuf<ExtendEntry> scratch;
+  int32_t *h_counts = nullptr;                         // pinned: compacted obstacle counts, read back together
+  unsigned long long *h_done = nullptr, *d_done = nullptr;  // mapped pinned completion word
+  DevBuf<unsigned> ticket;                             // blocks finished; the last one resets it
+  int n_inst = 0;
+  size_t n_ent = 0;
+  unsigned long long seq = 0;  // calls issued
+  void free_instances() {
+    for (void *p : {(void *)h_inst, (void *)h_hdr, (void *)h_counts})
+      if (p) cudaFreeHost(p);
+    h_inst = nullptr; h_hdr = nullptr; h_counts = nullptr;
+  }
+  ~ExtendMultiState() {
+    free_instances();
+    if (h_ent) cudaFreeHost(h_ent);
+    if (h_done) cudaFreeHost(h_done);
+  }
+  // grow-only; every call waits for its own completion, so the buffers are idle between calls
+  void ensure(int n, size_t entries, cudaStream_t st) {
+    if (!h_done) {
+      mapped_alloc(h_done, d_done, 1);
+      *h_done = 0;
+      ticket.ensure(1, st);
+      RQ_CUDA(cudaMemsetAsync(ticket.p, 0, sizeof(unsigned), st));
+    }
+    if (n > n_inst) {
+      if (h_inst) { RQ_CUDA(cudaStreamSynchronize(st)); free_instances(); }
+      const int nc = std::max(n, 2 * n_inst);
+      RQ_CUDA(cudaHostAlloc((void **)&h_inst, sizeof(ExtendInstance) * (size_t)nc, cudaHostAllocDefault));
+      RQ_CUDA(cudaHostAlloc((void **)&h_counts, sizeof(int32_t) * (size_t)nc, cudaHostAllocDefault));
+      mapped_alloc(h_hdr, d_hdr, (size_t)nc);
+      inst.ensure((size_t)nc, st);
+      n_inst = nc;
+    }
+    if (entries > n_ent) {
+      if (h_ent) { RQ_CUDA(cudaStreamSynchronize(st)); cudaFreeHost(h_ent); h_ent = nullptr; }
+      const size_t nc = std::max(entries, 2 * n_ent);
+      mapped_alloc(h_ent, d_ent_out, nc);
+      scratch.ensure(nc, st);
+      n_ent = nc;
+    }
+  }
+};
+
+static ExtendMultiState &extend_multi_state(rrtqx_ctx *ctx) {  // owned by the context, freed in rrtqx_ctx_destroy
+  static const char tag = 0;
+  return ctx->scratch.get<ExtendMultiState>(&tag);
+}
+
+static std::string instance_msg(int i, const char *what) { return "instance " + std::to_string(i) + ": " + what; }
+
+void extend_query_multi(rrtqx_tree *const *trees, const rrtqx_spheres *const *spheres, int n, const double *points,
+                        const double *ranges, double robot_radius, uint32_t flags, int32_t capacity,
+                        int32_t *nearest_idx, double *nearest_dist, uint8_t *point_collides, double *point_cert,
+                        int32_t *n_neighbors, int32_t *nbr_idx, double *nbr_dist, uint8_t *fwd_collide,
+                        uint8_t *rev_collide) {
+  RQ_REQUIRE(n >= 0, "n_instances is negative");
+  if (n == 0) return;
+  RQ_REQUIRE(trees != nullptr && spheres != nullptr, "trees / spheres is NULL");
+  RQ_REQUIRE(capacity >= 0, "capacity is negative");
+  RQ_REQUIRE(points != nullptr && !is_device_ptr(points), "points must be a host array");
+  RQ_REQUIRE(ranges != nullptr && !is_device_ptr(ranges), "ranges must be a host array");
+  rrtqx_ctx *ctx = trees[0] ? trees[0]->ctx : nullptr;
+  std::set<const rrtqx_tree *> seen;
+  for (int i = 0; i < n; ++i) {
+    const rrtqx_tree *t = trees[i];
+    if (!t || !spheres[i]) throw Error(RRTQX_ERR_INVALID, instance_msg(i, "NULL tree or obstacle set"));
+    if (t->ctx != ctx || spheres[i]->ctx != ctx) throw Error(RRTQX_ERR_INVALID, instance_msg(i, "handle of another context"));
+    if (t->d != trees[0]->d) throw Error(RRTQX_ERR_INVALID, instance_msg(i, "trees of different dimension d"));
+    if (!seen.insert(t).second) throw Error(RRTQX_ERR_INVALID, instance_msg(i, "the same tree appears twice"));
+    if (t->wrap.num_wraps > 0)
+      throw Error(RRTQX_ERR_UNSUPPORTED, instance_msg(i, "extend query on a wrap-around tree (use the batched nearest / range calls)"));
+    if (t->n == 0) throw Error(RRTQX_ERR_EMPTY_TREE, instance_msg(i, "extend query on an empty tree"));
+  }
+  const int d = trees[0]->d;
+  cudaStream_t st = ctx->stream;
+  const size_t stride = (size_t)std::max(capacity, 1);
+  ExtendMultiState &ms = extend_multi_state(ctx);
+  ms.ensure(n, stride * (size_t)n, st);
+  for (int i = 0; i < n; ++i) tree_prepare_query(trees[i]);
+
+  // active-obstacle tables: each tree's ExtendState cache, shared with the single call; every stale table is
+  // compacted first, then all their counts come back with one synchronise
+  const int ignore_active = (flags & RRTQX_CHECK_IGNORE_ACTIVE) ? 1 : 0;
+  std::vector<int> stale;
+  for (int i = 0; i < n; ++i) {
+    ExtendState *es = &extend_state(trees[i]);
+    const rrtqx_spheres *S = spheres[i];
+    if (es->act_version == S->version && es->act_ignore == ignore_active) continue;
+    es->act_rec.ensure((size_t)S->n + 1, st);
+    es->act_n.ensure(4, st);
+    RQ_CUDA(cudaMemsetAsync(es->act_n.p, 0, sizeof(int32_t), st));
+    if (S->n > 0) {
+      extend_compact_kernel<<<div_up(S->n, 256), 256, 0, st>>>(S->rec.p, S->active.p, (int)S->n, ignore_active,
+                                                               es->act_rec.p, es->act_n.p);
+      post_launch(ctx);
+    }
+    RQ_CUDA(cudaMemcpyAsync(&ms.h_counts[stale.size()], es->act_n.p, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    stale.push_back(i);
+  }
+  if (!stale.empty()) {
+    RQ_CUDA(cudaStreamSynchronize(st));
+    for (size_t k = 0; k < stale.size(); ++k) {
+      ExtendState *es = &extend_state(trees[stale[k]]);
+      es->n_act = ms.h_counts[k];
+      es->act_version = spheres[stale[k]]->version;
+      es->act_ignore = ignore_active;
+    }
+  }
+  for (int i = 0; i < n; ++i)
+    if (extend_state(trees[i]).n_act > EXT_MAX_SPHERES)
+      throw Error(RRTQX_ERR_INVALID, instance_msg(i, "extend_query supports at most 768 ACTIVE obstacles; use the batched calls"));
+
+  const unsigned long long seq = ++ms.seq;
+  for (int i = 0; i < n; ++i) {
+    const ExtendState &es = extend_state(trees[i]);
+    ExtendInstance &I = ms.h_inst[i];
+    I.g = trees[i]->view();
+    ExtendParams &prm = I.prm;
+    for (int c = 0; c < 4; ++c) prm.p[c] = c < d ? points[(size_t)i * d + c] : 0.0;
+    prm.r = ranges[i];
+    prm.T = host_sqrt_thresh_lt(ranges[i]);
+    prm.rho = robot_radius;
+    prm.capacity = capacity;
+    prm.quick_pass = (flags & RRTQX_CHECK_QUICK_PASS) ? 1 : 0;
+    prm.ignore_active = 1;  // the table holds the active obstacles only
+    prm.fma_dot = (flags & RRTQX_CHECK_FMA_DOT) ? 1 : 0;
+    prm.seq = seq;
+    I.table = es.act_rec.p;
+    I.n_table = es.n_act;
+    I.hdr = ms.d_hdr + i;
+    I.ent = ms.scratch.p + stride * i;
+    I.ent_out = ms.d_ent_out + stride * i;
+  }
+  RQ_CUDA(cudaMemcpyAsync(ms.inst.p, ms.h_inst, sizeof(ExtendInstance) * (size_t)n, cudaMemcpyHostToDevice, st));
+#define RQ_EXTM(D_, F_) extend_query_multi_kernel<D_, F_><<<n, EXT_WARPS * 32, 0, st>>>(ms.inst.p, ms.ticket.p, ms.d_done, seq)
+  const bool fma = (flags & RRTQX_CHECK_FMA_DOT) != 0;
+  switch (d) {
+    case 2: if (fma) RQ_EXTM(2, true); else RQ_EXTM(2, false); break;
+    case 3: if (fma) RQ_EXTM(3, true); else RQ_EXTM(3, false); break;
+    case 4: if (fma) RQ_EXTM(4, true); else RQ_EXTM(4, false); break;
+    default: throw Error(RRTQX_ERR_UNSUPPORTED, "d must be 2, 3 or 4");
+  }
+#undef RQ_EXTM
+  post_launch(ctx);
+  wait_published(ms.h_done, seq, st);
+
+  for (int i = 0; i < n; ++i) {
+    const ExtendHeader h = ms.h_hdr[i];
+    if (nearest_idx) nearest_idx[i] = h.nearest_idx;
+    if (nearest_dist) nearest_dist[i] = h.nearest_dist;
+    if (point_collides) point_collides[i] = (uint8_t)h.point_collides;
+    if (point_cert) point_cert[i] = h.cert;
+    if (n_neighbors) n_neighbors[i] = h.count;
+    const int m = std::min(h.count, capacity);
+    const ExtendEntry *src = ms.h_ent + stride * i;
+    const size_t o = (size_t)capacity * i;
+    for (int k = 0; k < m; ++k) {
+      if (nbr_idx) nbr_idx[o + k] = src[k].node;
+      if (nbr_dist) nbr_dist[o + k] = src[k].dist;
+      if (fwd_collide) fwd_collide[o + k] = src[k].fwd;
+      if (rev_collide) rev_collide[o + k] = src[k].rev;
+    }
   }
 }

@@ -275,12 +275,6 @@ extend_dubins_check_kernel(GridView g, PolyView P, int ignore_active, const Exte
   }
 }
 
-template <typename T>
-static void mapped_alloc(T *&h, T *&d, size_t n) {
-  RQ_CUDA(cudaHostAlloc((void **)&h, sizeof(T) * n, cudaHostAllocMapped));
-  RQ_CUDA(cudaHostGetDevicePointer((void **)&d, h, 0));
-}
-
 struct ExtendDubinsState {   // per tree: mapped pinned result buffers + device scratch
   ExtendDubinsHeader *h_hdr = nullptr, *d_hdr = nullptr;
   int32_t *h_idx = nullptr, *d_idx = nullptr;

@@ -90,6 +90,11 @@ void extend_query(rrtqx_tree *t, const rrtqx_spheres *S, const double *point, do
                   uint32_t flags, int32_t capacity, int32_t *nearest_idx, double *nearest_dist,
                   uint8_t *point_collides, double *point_cert, int32_t *n_neighbors, int32_t *nbr_idx,
                   double *nbr_dist, uint8_t *fwd_collide, uint8_t *rev_collide);
+void extend_query_multi(rrtqx_tree *const *trees, const rrtqx_spheres *const *spheres, int n, const double *points,
+                        const double *ranges, double robot_radius, uint32_t flags, int32_t capacity,
+                        int32_t *nearest_idx, double *nearest_dist, uint8_t *point_collides, double *point_cert,
+                        int32_t *n_neighbors, int32_t *nbr_idx, double *nbr_dist, uint8_t *fwd_collide,
+                        uint8_t *rev_collide);
 void extend_query_dubins(rrtqx_tree *t, const rrtqx_polygons *P, double *point, double delta, double range,
                          double robot_radius, double min_turn_radius, uint32_t flags, int32_t capacity,
                          int32_t *nearest_idx, double *nearest_dist, int32_t *n_neighbors, int32_t *nbr_idx,

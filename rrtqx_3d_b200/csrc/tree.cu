@@ -3,6 +3,8 @@
 // index (cell-sorted SoA).
 #include <algorithm>
 #include <cmath>
+#include <set>
+#include <string>
 
 #include "scan.cuh"
 #include "tree.cuh"
@@ -121,12 +123,10 @@ __global__ void kd_insert_one_kernel(const double4 *__restrict__ pos, unsigned *
   }
 }
 
-// The planner's per-iteration insert in ONE launch: the position travels as a kernel argument (no staging
-// copy, nothing to wait for), the thread initialises the node's records and walks down to its slot.
-__global__ void kd_insert_point_kernel(double4 p, double4 *__restrict__ pos, unsigned *__restrict__ child,
-                                       int32_t *__restrict__ parent, int8_t *__restrict__ split, int32_t *__restrict__ cur,
-                                       int64_t i, int d) {
-  if (threadIdx.x != 0 || blockIdx.x != 0) return;
+// One thread initialises node i's records and walks down to its slot (sequential kdInsert).
+__device__ __forceinline__ void kd_insert_point(double4 p, double4 *__restrict__ pos, unsigned *__restrict__ child,
+                                                int32_t *__restrict__ parent, int8_t *__restrict__ split,
+                                                int32_t *__restrict__ cur, int64_t i, int d) {
   pos[i] = p;
   child[2 * i] = KD_EMPTY;
   child[2 * i + 1] = KD_EMPTY;
@@ -146,6 +146,108 @@ __global__ void kd_insert_point_kernel(double4 p, double4 *__restrict__ pos, uns
       return;
     }
     q = (int32_t)c;
+  }
+}
+
+// The planner's per-iteration insert in ONE launch: the position travels as a kernel argument (no staging
+// copy, nothing to wait for).
+__global__ void kd_insert_point_kernel(double4 p, double4 *__restrict__ pos, unsigned *__restrict__ child,
+                                       int32_t *__restrict__ parent, int8_t *__restrict__ split, int32_t *__restrict__ cur,
+                                       int64_t i, int d) {
+  if (threadIdx.x != 0 || blockIdx.x != 0) return;
+  kd_insert_point(p, pos, child, parent, split, cur, i, d);
+}
+
+struct InsertInstance {   // one tree's insert of rrtqx_tree_insert_multi
+  double4 p;
+  double4 *pos;
+  unsigned *child;
+  int32_t *parent;
+  int8_t *split;
+  int32_t *cur;
+  int64_t i;
+  int32_t d, pad;
+};
+
+// One insert into each of n distinct trees, one thread per tree.
+__global__ void kd_insert_point_multi_kernel(const InsertInstance *__restrict__ ins, int n) {
+  const int k = blockIdx.x * blockDim.x + threadIdx.x;
+  if (k >= n) return;
+  const InsertInstance I = ins[k];
+  kd_insert_point(I.p, I.pos, I.child, I.parent, I.split, I.cur, I.i, I.d);
+}
+
+// Descriptors of rrtqx_tree_insert_multi, per context.  The call does not wait for the device, so the pinned staging
+// array is refilled only after the previous call's copy out of it has completed (an event, normally long done).
+struct InsertMultiState {
+  InsertInstance *h = nullptr;
+  DevBuf<InsertInstance> d;
+  int cap = 0;
+  cudaEvent_t copied = nullptr;
+  bool pending = false;
+  ~InsertMultiState() {
+    if (pending) cudaEventSynchronize(copied);
+    if (h) cudaFreeHost(h);
+    if (copied) cudaEventDestroy(copied);
+  }
+};
+
+void tree_insert_multi(rrtqx_tree *const *trees, int n, const double *positions, int32_t *index_out) {
+  RQ_REQUIRE(n >= 0, "n is negative");
+  if (n == 0) return;
+  RQ_REQUIRE(trees != nullptr, "trees is NULL");
+  RQ_REQUIRE(positions != nullptr && !is_device_ptr(positions), "positions must be a host array");
+  rrtqx_ctx *ctx = trees[0] ? trees[0]->ctx : nullptr;
+  std::set<const rrtqx_tree *> seen;
+  for (int i = 0; i < n; ++i) {
+    const rrtqx_tree *t = trees[i];
+    const std::string at = "tree " + std::to_string(i) + ": ";
+    if (!t) throw Error(RRTQX_ERR_INVALID, at + "NULL handle");
+    if (t->ctx != ctx) throw Error(RRTQX_ERR_INVALID, at + "handle of another context");
+    if (t->d != trees[0]->d) throw Error(RRTQX_ERR_INVALID, at + "trees of different dimension d");
+    if (!seen.insert(t).second) throw Error(RRTQX_ERR_INVALID, at + "the same tree appears twice");
+    if (t->n + 1 >= (int64_t)0x7fffffff) throw Error(RRTQX_ERR_INVALID, at + "tree too large for int32 node indices");
+  }
+  cudaStream_t st = ctx->stream;
+  static const char tag = 0;
+  InsertMultiState &ms = ctx->scratch.get<InsertMultiState>(&tag);
+  if (!ms.copied) RQ_CUDA(cudaEventCreateWithFlags(&ms.copied, cudaEventDisableTiming));
+  if (ms.pending) RQ_CUDA(cudaEventSynchronize(ms.copied));
+  ms.pending = false;
+  if (n > ms.cap) {
+    if (ms.h) cudaFreeHost(ms.h);
+    ms.h = nullptr;
+    const int nc = std::max(n, 2 * ms.cap);
+    RQ_CUDA(cudaHostAlloc((void **)&ms.h, sizeof(InsertInstance) * (size_t)nc, cudaHostAllocDefault));
+    ms.cap = nc;
+  }
+  ms.d.ensure((size_t)n, st);
+  const int d = trees[0]->d;
+  for (int i = 0; i < n; ++i) {
+    rrtqx_tree *t = trees[i];
+    const int64_t first = t->n;
+    const size_t need = (size_t)(first + 1);
+    t->pos.ensure(need, st, (size_t)first);
+    t->child.ensure(2 * need, st, 2 * (size_t)first);
+    t->parent.ensure(need, st, (size_t)first);
+    t->split.ensure(need, st, (size_t)first);
+    t->cur.ensure(need, st, (size_t)first);
+    const double *x = positions + (size_t)i * d;
+    InsertInstance &I = ms.h[i];
+    I.p = make_double4(x[0], x[1], d >= 3 ? x[2] : 0.0, d >= 4 ? x[3] : 0.0);
+    I.pos = t->pos.p; I.child = t->child.p; I.parent = t->parent.p; I.split = t->split.p; I.cur = t->cur.p;
+    I.i = first;
+    I.d = d;
+    I.pad = 0;
+  }
+  RQ_CUDA(cudaMemcpyAsync(ms.d.p, ms.h, sizeof(InsertInstance) * (size_t)n, cudaMemcpyHostToDevice, st));
+  RQ_CUDA(cudaEventRecord(ms.copied, st));
+  ms.pending = true;
+  kd_insert_point_multi_kernel<<<div_up(n, 128), 128, 0, st>>>(ms.d.p, n);
+  post_launch(ctx);
+  for (int i = 0; i < n; ++i) {
+    if (index_out) index_out[i] = (int32_t)trees[i]->n;
+    trees[i]->n += 1;
   }
 }
 

@@ -106,6 +106,8 @@ struct rrtqx_tree {
 namespace rrtqx {
 void tree_insert_batch(rrtqx_tree *t, const double *positions, int64_t n);
 void tree_insert_point(rrtqx_tree *t, const double *host_position);  // one node, one launch, asynchronous
+// one node into each of n distinct trees of one context (host positions, n x d), one launch, asynchronous
+void tree_insert_multi(rrtqx_tree *const *trees, int n, const double *positions, int32_t *index_out);
 void tree_reindex(rrtqx_tree *t);
 // re-index if the unsorted tail has outgrown its limit
 void tree_prepare_query(rrtqx_tree *t);

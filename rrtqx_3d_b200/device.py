@@ -480,6 +480,53 @@ def extend_query(tree: DeviceTree, spheres: SphereSet, point, r, robot_radius, f
     return out
 
 
+def extend_query_multi(trees, sphere_sets, points, ranges, robot_radius, flags=0, capacity=4096):
+    """extend_query for n independent instances (trees[i], sphere_sets[i], points[i], ranges[i]) in one launch and
+    one host wait; returns one ExtendResult per instance, equal to what extend_query returns for it."""
+    n = len(trees)
+    if n == 0:
+        return []
+    d = trees[0].d
+    pts = A.as_f64(points, d)
+    rr = A.as_f64(ranges).reshape(-1)
+    assert len(sphere_sets) == n and pts.shape[0] == n and rr.size == n
+    th = (A.vp * n)(*[None if t is None else t.h for t in trees])
+    sh = (A.vp * n)(*[None if s is None else s.h for s in sphere_sets])
+    ni, nd = np.empty(n, dtype=np.int32), np.empty(n, dtype=np.float64)
+    pc, ce, cnt = np.empty(n, dtype=np.uint8), np.empty(n, dtype=np.float64), np.empty(n, dtype=np.int32)
+    w = n * capacity
+    idx, dist = np.empty(max(w, 1), dtype=np.int32), np.empty(max(w, 1), dtype=np.float64)
+    fwd, rev = np.empty(max(w, 1), dtype=np.uint8), np.empty(max(w, 1), dtype=np.uint8)
+    L = trees[0].L
+    ctx_h = next((t.ctx.h for t in trees if t is not None), None)
+    A.check(L.rrtqx_extend_query_multi(th, sh, n, A.ptr(pts), A.ptr(rr), float(robot_radius), int(flags), int(capacity),
+                                       A.ptr(ni), A.ptr(nd), A.ptr(pc), A.ptr(ce), A.ptr(cnt), A.ptr(idx), A.ptr(dist),
+                                       A.ptr(fwd), A.ptr(rev)), ctx_h)
+    outs = []
+    for i in range(n):
+        out = ExtendResult()
+        out.nearest_idx, out.nearest_dist = int(ni[i]), float(nd[i])
+        out.point_collides, out.point_cert, out.count = bool(pc[i]), float(ce[i]), int(cnt[i])
+        a, b = i * capacity, i * capacity + min(out.count, capacity)
+        out.idx, out.dist, out.fwd, out.rev = idx[a:b], dist[a:b], fwd[a:b], rev[a:b]
+        outs.append(out)
+    return outs
+
+
+def insert_multi(trees, positions):
+    """rrtqx_tree_insert of positions[i] into trees[i] for every i in one asynchronous launch; returns the indices."""
+    n = len(trees)
+    if n == 0:
+        return np.empty(0, dtype=np.int32)
+    pos = A.as_f64(positions, trees[0].d)
+    assert pos.shape[0] == n
+    th = (A.vp * n)(*[None if t is None else t.h for t in trees])
+    out = np.empty(n, dtype=np.int32)
+    ctx_h = next((t.ctx.h for t in trees if t is not None), None)
+    A.check(trees[0].L.rrtqx_tree_insert_multi(th, n, A.ptr(pos), A.ptr(out)), ctx_h)
+    return out
+
+
 class PolygonSet:
     """rrtqx_polygons: the 2-D obstacle list of the Otte generation (kinds 1 = ball, 3 = polygon)."""
 
