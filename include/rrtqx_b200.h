@@ -370,6 +370,38 @@ RRTQX_API rrtqx_status rrtqx_extend_query_dubins(
     double *nbr_dist, double *edge_dist, int32_t *edge_type,
     uint8_t *edge_collide, rrtqx_dubins_result **trajectories);
 
+/* rrtqx_extend_query_dubins for n independent Dubins planning instances in
+ * the same three launches and one host wait (the city-block instances of
+ * config C5 run in lock-step).  Instance i: tree trees[i], polygon set
+ * polygons[i] (the same handle may serve several instances), sample
+ * points[i*4 .. i*4+4) (host, in/out: saturated in place with
+ * RRTQX_EXTEND_SATURATE), radius ranges[i] (host); delta, robot_radius and
+ * min_turn_radius are one value per call.  Per-instance outputs at index i;
+ * instance i's neighbour arrays start at i*capacity and its edge arrays at
+ * i*2*capacity, with the single call's edge numbering (edge 2k = new -> nbr k,
+ * 2k+1 = nbr k -> new).  Every per-instance value, trajectory rows included,
+ * equals what rrtqx_extend_query_dubins returns for the same arguments.  Any
+ * output pointer may be NULL.  With trajectories != NULL one
+ * rrtqx_dubins_result (created when *trajectories is NULL) holds the rows of
+ * every instance, packed in instance order: instance i's edges follow the
+ * 2*min(n_neighbors[j], capacity) edges of every instance j < i.
+ * n_instances == 0 does nothing.  Refused before anything is launched or
+ * written (RRTQX_ERR_INVALID): a NULL handle, handles of different contexts,
+ * the same tree twice, capacity < 0, device pointers for points / ranges.  A
+ * tree of another layout (RRTQX_ERR_UNSUPPORTED) or an empty tree
+ * (RRTQX_ERR_EMPTY_TREE) fails the whole call with the status of
+ * rrtqx_extend_query_dubins; the message names the instance.  The scratch and
+ * mapped result buffers belong to the context, so single and multi calls may
+ * be interleaved freely. */
+RRTQX_API rrtqx_status rrtqx_extend_query_dubins_multi(
+    rrtqx_tree *const *trees, const rrtqx_polygons *const *polygons,
+    int32_t n_instances, double *points, const double *ranges, double delta,
+    double robot_radius, double min_turn_radius, uint32_t flags,
+    int32_t capacity, int32_t *nearest_idx, double *nearest_dist,
+    int32_t *n_neighbors, int32_t *nbr_idx, double *nbr_dist,
+    double *edge_dist, int32_t *edge_type, uint8_t *edge_collide,
+    rrtqx_dubins_result **trajectories);
+
 /* ------------------------------------------------- resident edge set + sweeps */
 /* Device mirror of the planner's out-edge lists: for node v the reference
  * iterates InitialNeighborListOut then rrtNeighborsOut

@@ -44,7 +44,7 @@ export Context, GpuKDTree, GpuObstacles, GpuPolygons, GpuEdges, GpuWorld, attach
        explicitEdgeCheck, explicitEdgeCheckBatch, explicitPointCheck, explicitPointCheck3D,
        explicitNodeCheck, explicitNodeCheck3D,
        findPointsInConflictWithObstacle, addNewObstacle, removeObstacle, syncObstacles!, syncPolygons!, syncEdges!,
-       extendQuery, extendQueryMulti, kdInsertMulti, pinnedVector
+       extendQuery, extendQueryMulti, kdInsertMulti, extendQueryDubinsMulti, dubinsEdgesFromQueryMulti!, pinnedVector
 
 const LIB = get(ENV, "RRTQX_B200_LIB", joinpath(@__DIR__, "..", "rrtqx_3d_b200", "librrtqx_b200.so"))
 
@@ -831,6 +831,102 @@ function dubinsEdgesFromQuery!(S, edges::Vector)
       (Ptr{Cvoid}, Ptr{Float64}, Ptr{Int32}, Ptr{Int64}, Ptr{Float64}), res[], dist, typ, ptr, xy))
   for (i, e) in enumerate(edges)
     e === nothing || setDubinsTrajectory!(e, dist[i], typ[i], xy, ptr[i], ptr[i+1])
+  end
+  return edges
+end
+
+# extendQueryDubins for many Dubins planners in lock-step (the city-block instances of config C5): agent i is
+# (Ss[i], trees[i], points[i], ranges[i]), each with its own CSpace and tree.  One call and one host wait serve the
+# whole round; each agent gets the tuple extendQueryDubins returns, warm-up handling included.  The views and the
+# device solve stay valid until the next extendQueryDubinsMulti on the same first CSpace; dubinsEdgesFromQueryMulti!
+# puts an agent's solved edges onto its DubinsEdge objects.  An agent whose ball holds more than `capacity` nodes is
+# repeated alone with extendQueryDubins (rare; Dubins balls hold about 16 nodes), and its edges then come from
+# dubinsEdgesFromQuery! on its CSpace.  The agents share one robot radius, turning radius and delta (the C call takes
+# one of each).
+function extendQueryDubinsMulti(Ss::Vector, trees::Vector, points::Vector, ranges::Vector{Float64};
+                                saturate::Bool = false, capacity::Int = 1024)
+  n = length(trees)
+  n == 0 && return Any[]
+  S1 = Ss[1]
+  all(S -> S.robotRadius == S1.robotRadius, Ss) || error("extendQueryDubinsMulti: the agents' robot radii differ")
+  all(S -> S.minTurningRadius == S1.minTurningRadius, Ss) ||
+    error("extendQueryDubinsMulti: the agents' turning radii differ")
+  all(S -> S.delta == S1.delta, Ss) || error("extendQueryDubinsMulti: the agents' delta differ")
+  sets = Ptr{Cvoid}[syncPolygons!(world(S).polygons, S).h for S in Ss]
+  handles = Ptr{Cvoid}[t.h for t in trees]
+  P = Matrix{Float64}(undef, 4, n)                        # column-major 4 x n == row-major n x 4 for C
+  for i = 1:n; P[:, i] = vec(points[i])[1:4]; end
+  W = world(S1)
+  if !haskey(W.pinned, :mdIdx) || length(W.pinned[:mdIdx]) < n * capacity
+    W.pinned[:mdIdx] = pinnedVector(W.ctx, Int32, n * capacity); W.pinned[:mdDist] = pinnedVector(W.ctx, Float64, n * capacity)
+    W.pinned[:mdEdist] = pinnedVector(W.ctx, Float64, 2 * n * capacity)
+    W.pinned[:mdEtype] = pinnedVector(W.ctx, Int32, 2 * n * capacity)
+    W.pinned[:mdEcol] = pinnedVector(W.ctx, UInt8, 2 * n * capacity)
+  end
+  if !haskey(W.pinned, :mdRes)
+    r = Ref{Ptr{Cvoid}}(C_NULL)
+    W.pinned[:mdRes] = r
+    finalizer(x -> x[] != C_NULL && ccall((:rrtqx_dubins_result_destroy, LIB), Int32, (Ptr{Cvoid},), x[]), r)
+  end
+  idx = W.pinned[:mdIdx]::Vector{Int32}; dist = W.pinned[:mdDist]::Vector{Float64}
+  edist = W.pinned[:mdEdist]::Vector{Float64}; etype = W.pinned[:mdEtype]::Vector{Int32}
+  ecol = W.pinned[:mdEcol]::Vector{UInt8}; res = W.pinned[:mdRes]::Base.RefValue{Ptr{Cvoid}}
+  nearestIdx = Vector{Int32}(undef, n); nearestDist = Vector{Float64}(undef, n); cnt = Vector{Int32}(undef, n)
+  flags = saturate ? EXTEND_SATURATE : UInt32(0)
+  GC.@preserve sets handles P ranges idx dist edist etype ecol nearestIdx nearestDist cnt check(trees[1].ctx,
+      ccall((:rrtqx_extend_query_dubins_multi, LIB), Int32,
+            (Ptr{Ptr{Cvoid}}, Ptr{Ptr{Cvoid}}, Int32, Ptr{Float64}, Ptr{Float64}, Float64, Float64, Float64, UInt32,
+             Int32, Ptr{Int32}, Ptr{Float64}, Ptr{Int32}, Ptr{Int32}, Ptr{Float64}, Ptr{Float64}, Ptr{Int32},
+             Ptr{UInt8}, Ref{Ptr{Cvoid}}),
+            handles, sets, n, P, ranges, S1.delta, S1.robotRadius, S1.minTurningRadius, flags, Int32(capacity),
+            nearestIdx, nearestDist, cnt, idx, dist, edist, etype, ecol, res))
+  first = Vector{Int}(undef, n)                           # agent i's first edge (0-based) in the packed solve
+  alone = falses(n)
+  out = Vector{Any}(undef, n)
+  f = 0
+  for i = 1:n
+    S = Ss[i]; c = Int(cnt[i])
+    first[i] = f
+    f += 2 * min(c, capacity)
+    if c > capacity                          # overflow: this agent alone, with room for its whole ball
+      out[i] = extendQueryDubins(S, trees[i], points[i], ranges[i]; saturate = saturate, capacity = 2 * c)
+      alone[i] = true
+      continue
+    end
+    r = (i - 1) * capacity + 1 : (i - 1) * capacity + c
+    re = 2 * (i - 1) * capacity + 1 : 2 * (i - 1) * capacity + 2 * c
+    warm = S.inWarmupTime                    # obstacles are ignored during warm-up (DRRT.jl:1660-1678)
+    out[i] = (trees[i].nodes[nearestIdx[i] + 1], nearestDist[i], P[:, i], view(idx, r), view(dist, r), view(edist, re),
+              view(etype, re), warm ? falses(2 * c) : view(ecol, re) .!= 0)
+  end
+  W.pinned[:mdFirst] = first; W.pinned[:mdAlone] = alone; W.pinned[:mdFetched] = nothing
+  return out
+end
+
+# Puts agent i's device solve of the last extendQueryDubinsMulti whose first CSpace was S onto DubinsEdge objects:
+# edges[e] receives the agent's edge e (edges[2k-1] = new -> n_k, edges[2k] = n_k -> new; `nothing` entries are
+# skipped).  The packed solve is fetched once per call and shared by the agents.
+function dubinsEdgesFromQueryMulti!(S, i::Int, edges::Vector)
+  W = world(S)
+  (W.pinned[:mdAlone]::BitVector)[i] &&
+    error("agent $i was repeated alone by extendQueryDubinsMulti: its edges come from dubinsEdgesFromQuery!")
+  if W.pinned[:mdFetched] === nothing
+    res = W.pinned[:mdRes]::Base.RefValue{Ptr{Cvoid}}
+    ne = Ref{Int64}(0); nr = Ref{Int64}(0)
+    check(W.ctx, ccall((:rrtqx_dubins_result_sizes, LIB), Int32, (Ptr{Cvoid}, Ref{Int64}, Ref{Int64}), res[], ne, nr))
+    dist = Vector{Float64}(undef, ne[]); typ = Vector{Int32}(undef, ne[]); ptr = Vector{Int64}(undef, ne[] + 1)
+    xy = Matrix{Float64}(undef, 2, nr[])
+    GC.@preserve dist typ ptr xy check(W.ctx, ccall((:rrtqx_dubins_result_fetch, LIB), Int32,
+        (Ptr{Cvoid}, Ptr{Float64}, Ptr{Int32}, Ptr{Int64}, Ptr{Float64}), res[], dist, typ, ptr, xy))
+    W.pinned[:mdFetched] = (dist, typ, ptr, xy)
+  end
+  dist, typ, ptr, xy = W.pinned[:mdFetched]
+  first = (W.pinned[:mdFirst]::Vector{Int})[i]
+  last = i < length(W.pinned[:mdFirst]) ? W.pinned[:mdFirst][i + 1] : length(dist)
+  length(edges) <= last - first || error("agent $i has $(last - first) edges in the last call, not $(length(edges))")
+  for (k, e) in enumerate(edges)
+    j = first + k                            # 1-based index of the packed edge
+    e === nothing || setDubinsTrajectory!(e, dist[j], typ[j], xy, ptr[j], ptr[j+1])
   end
   return edges
 end

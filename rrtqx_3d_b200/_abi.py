@@ -63,6 +63,8 @@ SIGNATURES = {
     "rrtqx_tree_insert_multi": (i32, [vp, i32, vp, vp]),
     "rrtqx_extend_query_dubins": (i32, [vp, vp, vp, f64, f64, f64, f64, u32, i32, C.POINTER(i32), C.POINTER(f64),
                                         C.POINTER(i32), vp, vp, vp, vp, vp, C.POINTER(vp)]),
+    "rrtqx_extend_query_dubins_multi": (i32, [vp, vp, i32, vp, vp, f64, f64, f64, u32, i32, vp, vp, vp, vp, vp, vp, vp,
+                                              vp, C.POINTER(vp)]),
     "rrtqx_spheres_create": (i32, [vp, C.POINTER(vp)]),
     "rrtqx_spheres_destroy": (i32, [vp]),
     "rrtqx_spheres_upload": (i32, [vp, vp, vp, vp, i64]),

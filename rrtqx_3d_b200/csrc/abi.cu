@@ -536,6 +536,27 @@ rrtqx_status rrtqx_extend_query_dubins(rrtqx_tree *tree, const rrtqx_polygons *p
   });
 }
 
+rrtqx_status rrtqx_extend_query_dubins_multi(rrtqx_tree *const *trees, const rrtqx_polygons *const *polygons,
+                                             int32_t n_instances, double *points, const double *ranges, double delta,
+                                             double robot_radius, double min_turn_radius, uint32_t flags,
+                                             int32_t capacity, int32_t *nearest_idx, double *nearest_dist,
+                                             int32_t *n_neighbors, int32_t *nbr_idx, double *nbr_dist,
+                                             double *edge_dist, int32_t *edge_type, uint8_t *edge_collide,
+                                             rrtqx_dubins_result **trajectories) {
+  if (n_instances == 0) return RRTQX_OK;
+  rrtqx_ctx *ctx = first_ctx(trees, n_instances);
+  if (!ctx) {
+    g_last_error = "no tree handle";
+    return RRTQX_ERR_INVALID;
+  }
+  return guarded(ctx, [&] {
+    bind_device(ctx);
+    extend_query_dubins_multi(trees, polygons, n_instances, points, ranges, delta, robot_radius, min_turn_radius, flags,
+                              capacity, nearest_idx, nearest_dist, n_neighbors, nbr_idx, nbr_dist, edge_dist,
+                              edge_type, edge_collide, trajectories);
+  });
+}
+
 // ---------------------------------------------------------------- spheres
 rrtqx_status rrtqx_spheres_create(rrtqx_ctx *ctx, rrtqx_spheres **out) {
   if (!ctx) return RRTQX_ERR_INVALID;

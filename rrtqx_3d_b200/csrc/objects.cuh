@@ -100,6 +100,11 @@ void extend_query_dubins(rrtqx_tree *t, const rrtqx_polygons *P, double *point, 
                          int32_t *nearest_idx, double *nearest_dist, int32_t *n_neighbors, int32_t *nbr_idx,
                          double *nbr_dist, double *edge_dist, int32_t *edge_type, uint8_t *edge_collide,
                          rrtqx_dubins_result **trajectories);
+void extend_query_dubins_multi(rrtqx_tree *const *trees, const rrtqx_polygons *const *polygons, int n, double *points,
+                               const double *ranges, double delta, double robot_radius, double min_turn_radius,
+                               uint32_t flags, int32_t capacity, int32_t *nearest_idx, double *nearest_dist,
+                               int32_t *n_neighbors, int32_t *nbr_idx, double *nbr_dist, double *edge_dist,
+                               int32_t *edge_type, uint8_t *edge_collide, rrtqx_dubins_result **trajectories);
 // collision.cu
 void edge_check(rrtqx_ctx *ctx, const rrtqx_tree *tree, const rrtqx_spheres *spheres, const int32_t *src,
                 const int32_t *dst, const double *starts, const double *ends, int64_t n_edges, double robot_radius,

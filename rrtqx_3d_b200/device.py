@@ -674,7 +674,7 @@ def dubins_saturate_batch(ctx: Context, new_points, closest, delta):
 class ExtendDubinsResult:
     """Outputs of one rrtqx_extend_query_dubins call.  Edge 2i runs new -> idx[i], edge 2i+1 idx[i] -> new."""
     __slots__ = ("point", "nearest_idx", "nearest_dist", "count", "idx", "dist", "edge_dist", "edge_type",
-                 "edge_collide", "trajectories")
+                 "edge_collide", "trajectories", "first_edge")
 
 
 def extend_query_dubins(tree: DeviceTree, polys: PolygonSet, point, r, robot_radius, min_turn_radius, delta=0.0,
@@ -701,8 +701,47 @@ def extend_query_dubins(tree: DeviceTree, polys: PolygonSet, point, r, robot_rad
     m = min(out.count, capacity)
     out.idx, out.dist = idx[:m], dist[:m]
     out.edge_dist, out.edge_type, out.edge_collide = edist[:2 * m], etype[:2 * m], ecol[:2 * m]
-    out.trajectories = trajectories
+    out.trajectories, out.first_edge = trajectories, 0
     return out
+
+
+def extend_query_dubins_multi(trees, poly_sets, points, ranges, robot_radius, min_turn_radius, delta=0.0, flags=0,
+                              capacity=1024, trajectories: DubinsResult | bool | None = None):
+    """extend_query_dubins for n independent instances (trees[i], poly_sets[i], points[i], ranges[i]) in one call;
+    returns one ExtendDubinsResult per instance, equal to what extend_query_dubins returns for it.  The instances
+    share one trajectory result: instance i's edges start at its first_edge in the packed edge order."""
+    n = len(trees)
+    if n == 0:
+        return []
+    pts = np.array(A.as_f64(points, 4), copy=True)
+    rr = A.as_f64(ranges).reshape(-1)
+    assert len(poly_sets) == n and pts.shape[0] == n and rr.size == n
+    th = (A.vp * n)(*[None if t is None else t.h for t in trees])
+    ph = (A.vp * n)(*[None if p is None else p.h for p in poly_sets])
+    ni, nd, cnt = np.empty(n, dtype=np.int32), np.empty(n), np.empty(n, dtype=np.int32)
+    w = max(n * capacity, 1)
+    idx, dist = np.empty(w, dtype=np.int32), np.empty(w)
+    edist, etype, ecol = np.empty(2 * w), np.empty(2 * w, dtype=np.int32), np.empty(2 * w, dtype=np.uint8)
+    ctx = next((t.ctx for t in trees if t is not None), None)
+    if trajectories is True:
+        trajectories = DubinsResult(ctx)
+    L = ctx.L if ctx is not None else A.lib()
+    A.check(L.rrtqx_extend_query_dubins_multi(
+        th, ph, n, A.ptr(pts), A.ptr(rr), float(delta), float(robot_radius), float(min_turn_radius), int(flags),
+        int(capacity), A.ptr(ni), A.ptr(nd), A.ptr(cnt), A.ptr(idx), A.ptr(dist), A.ptr(edist), A.ptr(etype),
+        A.ptr(ecol), C.byref(trajectories.h) if trajectories is not None else None), ctx.h if ctx else None)
+    outs, first = [], 0
+    for i in range(n):
+        out = ExtendDubinsResult()
+        out.point, out.nearest_idx, out.nearest_dist, out.count = pts[i], int(ni[i]), float(nd[i]), int(cnt[i])
+        m = min(out.count, capacity)
+        a, e = i * capacity, 2 * i * capacity
+        out.idx, out.dist = idx[a:a + m], dist[a:a + m]
+        out.edge_dist, out.edge_type, out.edge_collide = edist[e:e + 2 * m], etype[e:e + 2 * m], ecol[e:e + 2 * m]
+        out.trajectories, out.first_edge = trajectories, first
+        first += 2 * m
+        outs.append(out)
+    return outs
 
 
 def extend_query_dubins_composed(tree: DeviceTree, polys: PolygonSet, point, r, robot_radius, min_turn_radius,
